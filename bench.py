@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- eBWT positions/s of the ebwt2clust + clust2snp hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload C2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload C2] [--dump-outputs DIR]
 
 One "step" = one full pass of the hot path (cluster scan -> merge -> statistics -> per-cluster
 SNP calling) over the shard(s) resident in HBM.  `value` is device-resident throughput (CUDA
@@ -529,6 +529,46 @@ def bench_c4_streamed(args, torch, dist, api, sharding, rank, world, local, dev)
         dist.destroy_process_group()
 
 
+DUMP_CLUSTER_SAMPLE = 1 << 20   # cluster records kept by --dump-outputs (20 B each as float64 index / start + float32 length)
+DUMP_EVENT_BYTES = 40 << 20     # budget of the events' arrays
+
+
+def dump_outputs(out_dir, counts, start, ln, events, event_type, seed=0):
+    """--dump-outputs: what one step of the timed path hands its caller, as float .npy files in out_dir (under 63 MB).
+    counts: {name: int} of the step's result; start / ln: the .clusters records; events: event_type (api.Event) list in
+    .snp order.
+    Larger outputs are cut to a sample that depends only on their size (seeded), so two builds of the project that compute
+    the same outputs dump the same files."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"counts": np.array([counts[k] for k in sorted(counts)], dtype=np.float64)}  # in the order of the names
+    m = len(ln)
+    idx = np.arange(m, dtype=np.int64)
+    if m > DUMP_CLUSTER_SAMPLE:
+        idx = np.sort(np.random.default_rng(seed).choice(m, size=DUMP_CLUSTER_SAMPLE, replace=False))
+    arrays["cluster_index"] = idx.astype(np.float64)
+    arrays["cluster_start"] = np.asarray(start, dtype=np.uint64)[idx].astype(np.float64)
+    arrays["cluster_len"] = np.asarray(ln)[idx].astype(np.float32)
+    n_ev = len(events)
+    ev = {f: np.array([getattr(e, f) for e in events], dtype=np.int64) for f in
+          ("cluster_start", "D", "gap", "supp0", "supp1", "right_len", "keep")}
+    raw = np.frombuffer(b"".join(bytes(e) for e in events), dtype=np.uint8).reshape(n_ev, C.sizeof(event_type))
+    ctx = {f: raw[:, getattr(event_type, f).offset:getattr(event_type, f).offset + getattr(event_type, f).size]
+           for f in ("left0", "left1", "right")}
+    width = max(int(np.flatnonzero(c.any(axis=0)).max()) + 1 if c.any() else 0 for c in ctx.values())  # the rest is 0
+    keep = np.arange(n_ev)
+    per_event = 2 * 8 + 6 * 4 + 3 * 4 * width
+    if n_ev * per_event > DUMP_EVENT_BYTES:
+        keep = np.sort(np.random.default_rng(seed + 1).choice(n_ev, size=DUMP_EVENT_BYTES // per_event, replace=False))
+    arrays["event_index"] = keep.astype(np.float64)
+    arrays["event_cluster_start"] = ev["cluster_start"][keep].astype(np.float64)
+    arrays["event_fields"] = np.stack([ev[f][keep] for f in ("D", "gap", "supp0", "supp1", "right_len", "keep")], axis=1).astype(np.float32).reshape(-1, 6)
+    for f, c in ctx.items():
+        arrays[f"event_{f}"] = c[keep, :width].astype(np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return arrays
+
+
 def synth_positions(name):
     from ebwt2snp_b200 import synth
     c = synth.CONFIGS[name]
@@ -568,7 +608,15 @@ def main():
     ap.add_argument("--tiles", type=int, default=1,
                     help="resident-only study: tile the workload T times on the GPU (read ids shifted; every tile starts with "
                          "lcp = 0), e.g. --tiles 8 = 4.46e9 positions, C3/C4-sized shards; implies --no-e2e --no-cpu-baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (result counts, a seeded sample of the "
+                         ".clusters records, the events) as DIR/<name>.npy, float32 / float64, under 63 MB: the same arguments "
+                         "give the same inputs, so two builds can be compared output for output.  With N > 1 the counts are "
+                         "global, the records and events rank 0's shard only.  The resident path only: not with --workload C4 "
+                         "(streamed) or --impl reference")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "C4"):
+        raise SystemExit("--dump-outputs covers the resident B200 path (--impl b200, workloads C1 - C3)")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -739,12 +787,25 @@ def main():
         ktimes = {kid: ctx.kernel_time(kid) for kid in KERNELS}
         launches = ctx.launches - launches0
         ctx.timing(False)
+        if args.dump_outputs and rank == 0:
+            if world == 1:
+                counts = {"n_written": out.n_written, "n_clust_out": out.n_clust_out, "max_clust_length": out.max_clust_length}
+                snp = out.snp
+            else:
+                counts = {"n_written": out[0].total_written, "n_clust_out": out[0].n_clust_out, "max_clust_length": out[1].max_clust_length}
+                snp = out[2]
+            counts.update({f: getattr(snp, f) for f, _ in api.SnpCounts._fields_})
+            dumped = (counts, *sh.cluster_fetch(), sh.events())  # fetched here, written once the clocks are sampled
         n_soak = 1000 if T == 1 else 150  # a fixed count: every rank must run the same number of (collective) steps
         for _ in range(n_soak):
             step()
         sync_all()
         clocks = sampler.stop()
         clocks["window"] = f"timed region + {n_soak} more of the same steps, untimed"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *dumped, api.Event, seed=args.seed)
+        del dumped
+        log(f"[dump] outputs of the last timed step written to {args.dump_outputs}")
 
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device=dev)

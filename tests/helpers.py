@@ -99,6 +99,40 @@ def assemble(summaries, shard_records):
     return np.array(S, dtype=np.uint64), np.array(L, dtype=np.uint16), mg
 
 
+def reference_outputs(fa, eg, reads, nreads1):
+    """What the unmodified reference's ebwt2clust + clust2snp (defaults, -x 4 -y 4 -z 4) make of the dataset `fa` (written by
+    synth.write_dataset from the index `eg` and `reads`): (.clusters bytes, .snp bytes or None where clust2snp fails, the
+    n_clust_out it prints, {"returncode", "allowed", "n_candidates", and with the binaries "stdout" of clust2snp}).
+    The binaries themselves (oracle/_ref) where they are built, then the files they wrote are removed.  Elsewhere the oracle's
+    restatement of them (oracle/oracle.c): the committed outputs of the binaries under tests/golden pin it byte for byte on
+    their read sets (micro fixtures, equal-length fuzz, field widths), but not on the caller's inputs, so there the caller
+    compares with the restatement and not with the binaries."""
+    from oracle import oracle as O
+    snp_path = os.path.join(os.path.dirname(fa), os.path.basename(fa).rsplit(".fast", 1)[0] + ".snp")
+    if O.ref_available():
+        r1, ncl = O.ref_ebwt2clust(fa)
+        assert r1.returncode == 0, r1.stderr
+        r2, info = O.ref_clust2snp(fa, nreads1)
+        info["stdout"] = r2.stdout
+        cl = open(fa + ".clusters", "rb").read()
+        os.remove(fa + ".clusters")
+        snp = open(snp_path, "rb").read() if info["returncode"] == 0 else None
+        if os.path.exists(snp_path):
+            os.remove(snp_path)
+        return cl, snp, ncl, info
+    lcp, text, suff, bwt = (np.asarray(eg[k]) for k in ("lcp", "text", "suff", "bwt"))
+    s, l, ncl, _ = O.cluster_lm(lcp, bwt, 16, 2)
+    cl = O.clusters_to_bytes(s, l)
+    if len(l) == 0:  # the reference divides by zero in its statistics
+        return cl, None, ncl, {"returncode": 1}
+    p = O.default_params(nreads1)
+    st = O.statistics(s, l, p.mcov_out, p.pval)
+    snp, res = O.find_events(lcp, text, suff, bwt, s, l, p, st.max_clust_length, reads, O.uniform_read_offsets(*reads.shape),
+                             strict=False)
+    return cl, snp, ncl, {"returncode": 0 if snp is not None else 1, "allowed": (2 * p.mcov_out, st.max_clust_length),
+                          "n_candidates": int(res.n_candidates)}
+
+
 _DS_CACHE = {}
 
 

@@ -9,6 +9,7 @@ import pytest
 from ebwt2snp_b200 import synth
 from oracle import oracle as O
 from tests import golden_util as GU
+from tests import helpers as H
 
 pytestmark = pytest.mark.gpu
 
@@ -125,32 +126,34 @@ def test_cli_sharded_on_one_box(built, tmp_path):
         assert open(os.path.join(str(tmp_path), "micro_a.snp"), "rb").read() == g["variants"][0]["snp"], n_gpu
 
 
-@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built")
 def test_cli_live_vs_reference(built, tmp_path):
-    """a fresh seeded read set (not one of the fixtures): reference and B200 CLIs on the same files"""
+    """a fresh seeded read set (not one of the fixtures): reference (oracle/_ref where it is built, else the oracle's
+    restatement of it) and B200 CLIs on the same files"""
     rs = synth.make_read_set(G=30_000, reads_per_sample=6_000, L=100, n_snps=60, n_indels=10, rc=True, seed=321)
     e = synth.build_egsa(rs.reads)
     eg = {k: (v.numpy() if hasattr(v, "numpy") else v) for k, v in e.items()}
     ref_dir, our_dir = tmp_path / "ref", tmp_path / "b200"
     fa_ref = synth.write_dataset(str(ref_dir), rs, eg)
     fa_our = synth.write_dataset(str(our_dir), rs, eg)
-    r1, ncl = O.ref_ebwt2clust(fa_ref)
-    r2, info = O.ref_clust2snp(fa_ref, rs.nreads1)
-    assert r1.returncode == 0 and info["returncode"] == 0
+    ref_cl, ref_snp, ncl, info = H.reference_outputs(fa_ref, eg, rs.reads, rs.nreads1)
+    assert info["returncode"] == 0
     o1 = run("ebwt2clust", "-i", fa_our, "-x", 4, "-y", 4, "-z", 4)
     o2 = run("clust2snp", "-i", fa_our, "-n", rs.nreads1, "-x", 4, "-y", 4, "-z", 4)
     assert o1.returncode == 0 and o2.returncode == 0, (o1.stderr, o2.stderr)
-    assert open(fa_our + ".clusters", "rb").read() == open(fa_ref + ".clusters", "rb").read()
-    assert open(os.path.join(str(our_dir), "ALL.snp"), "rb").read() == open(os.path.join(str(ref_dir), "ALL.snp"), "rb").read()
+    assert open(fa_our + ".clusters", "rb").read() == ref_cl
+    assert open(os.path.join(str(our_dir), "ALL.snp"), "rb").read() == ref_snp
     assert stdout_value(o1.stdout, "Done. ") == ncl
     assert stdout_value(o2.stdout, "Done. ") == info["n_candidates"]
+    assert f"Cluster sizes allowed: [{info['allowed'][0]},{info['allowed'][1]}]" in o2.stdout
+    if "stdout" not in info:  # the restatement prints nothing
+        return
     # the histogram block of statistics() is printed identically (ref:clust2snp.cpp:916-934)
     def hist_block(out):
         lines = out.splitlines()
         a = next(i for i, ln in enumerate(lines) if ln.startswith("cluster length"))
         b = next(i for i, ln in enumerate(lines) if ln.startswith("Cluster sizes allowed"))
         return lines[a:b + 1]
-    assert hist_block(o2.stdout) == hist_block(r2.stdout)
+    assert hist_block(o2.stdout) == hist_block(info["stdout"])
 
 
 def test_cli_multiline_fasta(built, tmp_path):

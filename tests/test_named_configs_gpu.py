@@ -1,5 +1,5 @@
-"""-m gpu: byte parity on the NAMED configs of BASELINE.json (SURVEY.md 8(d)), against the unmodified reference
-(oracle/_ref run here on the same files).
+"""-m gpu: byte parity on the NAMED configs of BASELINE.json (SURVEY.md 8(d)), against the unmodified reference run on
+the same files (oracle/_ref where it is built, else the oracle's restatement of it: tests/helpers.py:reference_outputs).
 
   C1  exactly as stated (1 Mbp genome, 2 x 50 k reads of 100 bp, 1 000 SNPs, no reverse complements): file against file.
   C2  the whole E. coli-size set (5.6e8 positions, ~2 min of the single-threaded reference): file against file.
@@ -21,8 +21,9 @@ import pytest
 
 from ebwt2snp_b200 import api, sharding, synth
 from oracle import oracle as O
+from tests import helpers as H
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built")]
+pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "ebwt2snp_b200", "bin")
@@ -40,15 +41,11 @@ def run_cli(tool, *args, env=None):
     return subprocess.run([os.path.join(BIN, tool), *[str(a) for a in args]], capture_output=True, text=True, env=e, timeout=3600)
 
 
-def both_tool_chains(fa, nreads1, out_dir):
+def both_tool_chains(fa, eg, reads, nreads1, out_dir):
     """reference, then this repository's CLIs, on the same input files -> ((clusters, snp) of each, stdout counts)"""
     snp = os.path.join(out_dir, "ALL.snp")
-    r1, ncl = O.ref_ebwt2clust(fa)
-    r2, info = O.ref_clust2snp(fa, nreads1)
-    assert r1.returncode == 0 and info["returncode"] == 0, (r1.stderr, r2.stderr)
-    ref_cl, ref_snp = open(fa + ".clusters", "rb").read(), open(snp, "rb").read()
-    os.remove(fa + ".clusters")
-    os.remove(snp)
+    ref_cl, ref_snp, ncl, info = H.reference_outputs(fa, eg, reads, nreads1)
+    assert info["returncode"] == 0
     o1 = run_cli("ebwt2clust", "-i", fa, "-x", 4, "-y", 4, "-z", 4)
     assert o1.returncode == 0, o1.stderr
     o2 = run_cli("clust2snp", "-i", fa, "-n", nreads1, "-x", 4, "-y", 4, "-z", 4)
@@ -79,7 +76,7 @@ def test_named_config_file_vs_file(built, name):
     d = scratch_dir(n * 15)
     try:
         fa = synth.write_dataset(d, rs, eg, fixed_headers=True)
-        ref, our = both_tool_chains(fa, rs.nreads1, d)
+        ref, our = both_tool_chains(fa, eg, rs.reads, rs.nreads1, d)
         assert our[0] == ref[0], f"{name}: .clusters differ"
         assert our[1] == ref[1], f"{name}: .snp differ"
         assert our[2] == ref[2] and our[3] == ref[3]
@@ -190,11 +187,7 @@ def test_c3_windows_vs_reference_and_full_run(c3):
             wdir = os.path.join(d, f"w{wi}")
             wrs = synth.ReadSet(reads=reads, nreads1=n1, genome1=None, genome2=None, snp_pos=None, indels=[])
             fa = synth.write_dataset(wdir, wrs, sub, fixed_headers=True)
-            r1, ncl = O.ref_ebwt2clust(fa)
-            r2, info = O.ref_clust2snp(fa, n1)
-            assert r1.returncode == 0, (why, r1.stderr)
-            ref_cl = open(fa + ".clusters", "rb").read()
-            ref_snp = open(os.path.join(wdir, "ALL.snp"), "rb").read() if info["returncode"] == 0 else None
+            ref_cl, ref_snp, ncl, info = H.reference_outputs(fa, sub, reads, n1)
             # ---- the CUDA path on the window's own files (C ABI, from the .gesa records) ----
             rec = np.fromfile(fa + ".gesa", dtype=np.uint8)
             wsh = wctx.shard(b - a)
@@ -220,11 +213,9 @@ def test_c3_windows_vs_reference_and_full_run(c3):
             else:
                 assert wres.snp.n_candidates == 0
             if wi in (0, 1, 2):  # and file against file through the CLIs
-                os.remove(fa + ".clusters")
                 assert run_cli("ebwt2clust", "-i", fa, "-x", 4, "-y", 4, "-z", 4).returncode == 0
                 assert open(fa + ".clusters", "rb").read() == ref_cl
                 if ref_snp is not None:
-                    os.remove(os.path.join(wdir, "ALL.snp"))
                     assert run_cli("clust2snp", "-i", fa, "-n", n1, "-x", 4, "-y", 4, "-z", 4).returncode == 0
                     assert open(os.path.join(wdir, "ALL.snp"), "rb").read() == ref_snp
             # ---- the full-size run agrees with the window in the window's interior ----

@@ -133,3 +133,27 @@ def test_reference_build_matches_the_goldens():
     mk = open(os.path.join(os.path.dirname(here), "oracle", "Makefile")).read()
     for f in flags.split("(")[0].split():
         assert f in mk, f
+
+
+def test_reference_outputs_with_the_binaries(tmp_path, monkeypatch):
+    """tests/helpers.py:reference_outputs where oracle/_ref is built: clust2snp reads the .clusters ebwt2clust wrote, its stdout
+    comes back with the outputs, and both output files are gone afterwards (stand-in tools with the reference's file contract)"""
+    ref = tmp_path / "_ref"
+    ref.mkdir()
+    tools = {
+        "ebwt2clust": 'printf "CLUSTERS" > "$2.clusters"; echo "Done. 7 clusters saved to file."',
+        "clust2snp": 'cat "$2.clusters" > /dev/null || exit 1; printf "SNP" > "${2%.fasta}.snp"; '
+                     'echo "Cluster sizes allowed: [10,42]"; echo "Done. 3 potential variants found."',
+    }
+    for name, body in tools.items():
+        (ref / name).write_text("#!/bin/sh\n" + body + "\n")
+        (ref / name).chmod(0o755)
+    monkeypatch.setattr(O, "REF_DIR", str(ref))
+    assert O.ref_available()
+    fa = str(tmp_path / "ALL.fasta")
+    open(fa, "w").write(">r0\nACGT\n")
+    cl, snp, ncl, info = H.reference_outputs(fa, None, None, 1)
+    assert (cl, snp, ncl) == (b"CLUSTERS", b"SNP", 7)
+    assert info["returncode"] == 0 and info["allowed"] == (10, 42) and info["n_candidates"] == 3
+    assert "Cluster sizes allowed: [10,42]" in info["stdout"]
+    assert not os.path.exists(fa + ".clusters") and not os.path.exists(str(tmp_path / "ALL.snp"))
