@@ -1864,15 +1864,20 @@ int e2s_cluster_finalize(e2s_shard* s, const e2s_cluster_merged* mg) {
     s->adopt_put = false;
     s->finalized = true;
     if (s->chunked && s->pf_mcov && mg->n_adopt) {  // their records are still on the device (the range's last chunk): to the payload
+        // only the lengths phase 2 analyses (2 mcov_out .. 150): any other adopted record is never read, and may be far longer
+        // than the payload reserves per record or start in a chunk that has left the device
         SurvEntry extra[4];
+        unsigned long long n = 0;
         for (uint32_t i = 0; i < mg->n_adopt && i < 4; ++i)
-            extra[i] = SurvEntry{mg->adopt_start[i], mg->adopt_start[i] - s->global_off, uint32_t(mg->adopt_len[i]), 0u};
-        const unsigned long long n = mg->n_adopt;
-        CU(c, cudaMemcpyAsync(s->d_pf_list, extra, n * sizeof(SurvEntry), cudaMemcpyHostToDevice, c->stream));
-        CU(c, cudaMemcpyAsync(&s->d_res->n_pf, &n, 8, cudaMemcpyHostToDevice, c->stream));
-        CU(c, cudaStreamSynchronize(c->stream));
-        int rc = capture_survivors(s, n);
-        if (rc) return rc;
+            if (mg->adopt_len[i] >= 2 * uint64_t(s->pf_mcov) && mg->adopt_len[i] <= uint64_t(E2S_MAX_C_LEN))
+                extra[n++] = SurvEntry{mg->adopt_start[i], mg->adopt_start[i] - s->global_off, uint32_t(mg->adopt_len[i]), 0u};
+        if (n) {
+            CU(c, cudaMemcpyAsync(s->d_pf_list, extra, n * sizeof(SurvEntry), cudaMemcpyHostToDevice, c->stream));
+            CU(c, cudaMemcpyAsync(&s->d_res->n_pf, &n, 8, cudaMemcpyHostToDevice, c->stream));
+            CU(c, cudaStreamSynchronize(c->stream));
+            int rc = capture_survivors(s, n);
+            if (rc) return rc;
+        }
         s->pf_has_adopted = true;
     }
     return E2S_OK;
@@ -2684,8 +2689,7 @@ static int pipeline_host_resident(e2s_ctx* c, const void* gesa, uint64_t n, int 
 // All chunks of a chunked shard's range from host records (`records` = the record of global position `first`; it must reach
 // from the range's left context to its right halo): load, scan, this chunk's records out (into rec10 from slot *off_rec on).
 static int stream_range(e2s_shard* s, const void* records, uint64_t first, int x, int y, int z, uint32_t k, int32_t min_len,
-                        int mcov_out, void* rec10, uint64_t cap_records, uint64_t* off_rec, e2s_pipeline_result* res,
-                        bool* unsupported_first) {
+                        int mcov_out, void* rec10, uint64_t cap_records, uint64_t* off_rec, e2s_pipeline_result* res) {
     e2s_ctx* c = s->ctx;
     const uint64_t n = s->n_global, end = s->range_lo + s->range_n;
     const int rs = x + y + z + 1;
@@ -2700,9 +2704,7 @@ static int stream_range(e2s_shard* s, const void* records, uint64_t first, int x
         if ((rc = e2s_shard_load_gesa(s, src + (a - first) * uint64_t(rs), a, b - a, x, y, z))) return rc;
         res->h2d_bytes += (b - a) * uint64_t(rs);
         uint64_t m = 0;
-        rc = e2s_chunk_scan(s, k, min_len, mcov_out, &m);
-        if (rc == E2S_ERR_UNSUPPORTED && lo == s->range_lo && unsupported_first) *unsupported_first = true;
-        if (rc) return rc;
+        if ((rc = e2s_chunk_scan(s, k, min_len, mcov_out, &m))) return rc;
         if (rec10) {
             if (*off_rec + m > cap_records) return fail(c, E2S_ERR_ARG, "record capacity too small");
             uint64_t got = 0;
@@ -2745,20 +2747,27 @@ int e2s_pipeline_host(e2s_ctx* c, const void* gesa, uint64_t n, int x, int y, in
     } else if ((rc = e2s_chunked_reset(s))) {
         return rc;
     }
-    uint64_t off_rec = 0;
-    bool unsupported_first = false;
-    rc = stream_range(s, gesa, 0, x, y, z, k, min_len, p->mcov_out, rec10, cap_records, &off_rec, res, &unsupported_first);
-    if (unsupported_first)  // e.g. -m > 33: the resident two-kernel path takes it
+    // An input the streamed path refuses, whichever chunk finds it -- an LCP value above 127 under -k > 127, a cluster of
+    // 65 536 positions or more whose wrapped length passes the filters and whose start has left the device -- goes through
+    // a resident shard from the first record on: the records and counts of the streamed attempt are dropped.
+    const uint64_t reads_h2d = res->h2d_bytes;
+    auto resident = [&]() {
+        memset(res, 0, sizeof *res);
+        res->h2d_bytes = reads_h2d;
         return pipeline_host_resident(c, gesa, n, x, y, z, k, min_len, p, rec10, cap_records, events, cap_events, res);
+    };
+    uint64_t off_rec = 0;
+    rc = stream_range(s, gesa, 0, x, y, z, k, min_len, p->mcov_out, rec10, cap_records, &off_rec, res);
+    if (rc == E2S_ERR_UNSUPPORTED) return resident();
     if (rc) return rc;
     e2s_cluster_summary sum;
-    if ((rc = e2s_chunked_finish(s, k, min_len, &sum))) return rc;
+    if ((rc = e2s_chunked_finish(s, k, min_len, &sum))) return rc == E2S_ERR_UNSUPPORTED ? resident() : rc;
     e2s_cluster_merged mg;
     if ((rc = e2s_cluster_merge(&sum, 1, 0, &mg))) {
         c->err = g_err;
         return rc;
     }
-    if ((rc = e2s_cluster_finalize(s, &mg))) return rc;
+    if ((rc = e2s_cluster_finalize(s, &mg))) return rc == E2S_ERR_UNSUPPORTED ? resident() : rc;
     if (rec10) {  // the records of the tail rule come last (ref:ebwt2clust.cpp:127-135)
         if (off_rec + mg.n_append > cap_records) return fail(c, E2S_ERR_ARG, "e2s_pipeline_host: record capacity too small");
         for (uint32_t i = 0; i < mg.n_append; ++i) {
@@ -2998,7 +3007,7 @@ int e2s_pipeline_host_sharded(e2s_ctx* c, e2s_comm* cm, const void* records, uin
     }
     uint8_t* out = static_cast<uint8_t*>(rec10);
     uint64_t off_rec = rec10 ? 1 : 0;  // slot 0 is kept for the shard's head record
-    if ((rc = stream_range(s, records, first, x, y, z, k, min_len, p->mcov_out, rec10, cap_records, &off_rec, res, nullptr))) return rc;
+    if ((rc = stream_range(s, records, first, x, y, z, k, min_len, p->mcov_out, rec10, cap_records, &off_rec, res))) return rc;
     if ((rc = e2s_chunked_exchange(s, cm, k, min_len, p->mcov_out, p->pval, merged, stats))) return rc;
     uint64_t slice_first = 1, m_slice = off_rec ? off_rec - 1 : 0;
     if (rec10) {

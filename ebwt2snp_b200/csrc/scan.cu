@@ -817,9 +817,14 @@ cudaError_t launch_scan(const Scan8Params& p0, uint64_t alloc_r, cudaStream_t st
     for (int b = 0; b < 7; ++b) p.km[b] = ((kk >> b) & 1u) ? 0xffffffffu : 0u;
     p.km[7] = kk >= 128u ? 0xffffffffu : 0u;
     // tiles [t_int_lo, t_int_hi) need none of the edge rules: not the first tile of the eBWT, wholly inside n_local, not
-    // the tile that holds position n_global - 1
+    // the tile that holds position n_global - 1 nor the one that holds n_global - 2 (an END there decides the post-EOF
+    // phantom value; it can be an earlier tile than n_global - 1's, or the last tile of a range that is not the last)
     p.t_int_lo = p.global_off == 0 ? 1u : 0u;
     p.t_int_hi = p.global_off + p.n_local == p.n_global ? (p.num_tiles ? p.num_tiles - 1 : 0) : uint32_t(p.n_local / SC_T);
+    if (p.n_global >= 2 && p.n_global - 2 >= p.global_off && p.n_global - 2 < p.global_off + p.n_local) {
+        const uint32_t t_nm2 = uint32_t((p.n_global - 2 - p.global_off) / SC_T);
+        if (t_nm2 < p.t_int_hi) p.t_int_hi = t_nm2;
+    }
     // the bit-sliced LCP as rows of 256 bytes = one run of 32 words (8 rows per block of LCPT_BLOCK positions); the boxes
     // the kernel takes from it are 2 words x 8 runs: the plane words of the group before / after a tile
     CUtensorMap tmap;

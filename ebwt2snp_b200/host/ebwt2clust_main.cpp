@@ -132,7 +132,7 @@ int main(int argc, char** argv) {
                 if (!r) r = e2s_shard_set_layout(sh[size_t(g)], idx.x, idx.y, idx.z, idx.bcr ? 1 : 0);
                 uint64_t m = 0;
                 if (!r) r = e2s_chunk_scan(sh[size_t(g)], uint32_t(k), min_len, 0, &m);
-                if (r == E2S_ERR_UNSUPPORTED && clo == lo) {  // not an input for the one-pass scan
+                if (r == E2S_ERR_UNSUPPORTED) {  // not an input for the one-pass scan, whichever chunk finds it
                     fall_back = true;
                     r = 0;
                     break;
