@@ -170,15 +170,18 @@ int oracle_statistics(const uint64_t *start, const uint16_t *len, uint64_t m, in
 
 /* ---- clust2snp: find_variants --------------------------------------------------------- */
 
+/* A candidate's reads: min(consensus_reads, ORACLE_MAX_C_LEN) per sample at most (an analysed cluster never has more records),
+ * so any -c is exact here (the reference keeps them in a vector).  They live in one pool: idx0[n0] pos0[n0] idx1[n1] pos1[n1]
+ * from pool[at]. */
 typedef struct {
-    uint64_t idx0[64], pos0[64]; int n0;   /* consensus_reads is capped at 64 in this restatement */
-    uint64_t idx1[64], pos1[64]; int n1;
+    size_t at; int n0, n1;
     uint64_t right_idx, right_pos;
 } candidate;
 
-typedef struct { candidate *v; size_t n, cap; } cand_vec;
+typedef struct { candidate *v; size_t n, cap; uint64_t *pool; size_t pn, pcap; } cand_vec;
 
-static int cand_push(cand_vec *cv, const candidate *c) {
+static int cand_push(cand_vec *cv, candidate *c, const uint64_t *idx0, const uint64_t *pos0, const uint64_t *idx1,
+                     const uint64_t *pos1) {
     if (cv->n == cv->cap) {
         size_t nc = cv->cap ? cv->cap * 2 : 256;
         candidate *nv = (candidate *)realloc(cv->v, nc * sizeof *nv);
@@ -186,6 +189,22 @@ static int cand_push(cand_vec *cv, const candidate *c) {
         cv->v = nv;
         cv->cap = nc;
     }
+    const size_t need = 2 * (size_t)(c->n0 + c->n1);
+    if (cv->pn + need > cv->pcap) {
+        size_t nc = cv->pcap ? cv->pcap * 2 : 4096;
+        while (nc < cv->pn + need) nc *= 2;
+        uint64_t *np = (uint64_t *)realloc(cv->pool, nc * sizeof *np);
+        if (!np) return -1;
+        cv->pool = np;
+        cv->pcap = nc;
+    }
+    uint64_t *d = cv->pool + cv->pn;
+    memcpy(d, idx0, sizeof *d * (size_t)c->n0);
+    memcpy(d + c->n0, pos0, sizeof *d * (size_t)c->n0);
+    memcpy(d + 2 * c->n0, idx1, sizeof *d * (size_t)c->n1);
+    memcpy(d + 2 * c->n0 + c->n1, pos1, sizeof *d * (size_t)c->n1);
+    c->at = cv->pn;
+    cv->pn += need;
     cv->v[cv->n++] = *c;
     return 0;
 }
@@ -224,6 +243,7 @@ static int find_variants(const t_gsa *cl, uint64_t len, const oracle_params *p, 
             unsigned char c0 = f0[a], c1 = f1[b];
             if (c0 == c1) continue;
             candidate cd;
+            uint64_t idx0[ORACLE_MAX_C_LEN], pos0[ORACLE_MAX_C_LEN], idx1[ORACLE_MAX_C_LEN], pos1[ORACLE_MAX_C_LEN];
             cd.n0 = cd.n1 = 0;
             for (uint64_t i = 0; i < len; ++i) {
                 int sample = cl[i].text < p->nr_reads1 ? 0 : 1;
@@ -232,21 +252,21 @@ static int find_variants(const t_gsa *cl, uint64_t len, const oracle_params *p, 
                 uint64_t l = cl[i].lcp;
                 if (prefix_len >= (uint64_t)(int64_t)p->k_left && ch == c0 && sample == 0 &&
                     l >= (uint64_t)(int64_t)p->k_right && cd.n0 < p->consensus_reads) {
-                    cd.idx0[cd.n0] = cl[i].text;
-                    cd.pos0[cd.n0] = cl[i].suff - (uint64_t)p->k_left;
+                    idx0[cd.n0] = cl[i].text;
+                    pos0[cd.n0] = cl[i].suff - (uint64_t)p->k_left;
                     cd.n0++;
                 }
                 if (prefix_len >= (uint64_t)(int64_t)p->k_left && ch == c1 && sample == 1 &&
                     l >= (uint64_t)(int64_t)p->k_right && cd.n1 < p->consensus_reads) {
-                    cd.idx1[cd.n1] = cl[i].text;
-                    cd.pos1[cd.n1] = cl[i].suff - (uint64_t)p->k_left;
+                    idx1[cd.n1] = cl[i].text;
+                    pos1[cd.n1] = cl[i].suff - (uint64_t)p->k_left;
                     cd.n1++;
                 }
             }
             if (cd.n0 > 0 && cd.n1 > 0) {
                 cd.right_idx = max_idx;
                 cd.right_pos = max_pos;
-                if (cand_push(out, &cd)) return -1;
+                if (cand_push(out, &cd, idx0, pos0, idx1, pos1)) return -1;
             }
         }
     }
@@ -400,8 +420,11 @@ int oracle_find_events_w(const uint32_t *lcp, const uint32_t *text, const uint32
     memset(res, 0, sizeof *res);
     *snp_text = NULL;
     *snp_len = 0;
-    if (n == 0 || p->consensus_reads > 64 || p->k_left > 256 || p->max_gap > p->k_left) return -1;
-    cand_vec cands = {0, 0, 0};
+    /* outside what this restatement supports (an empty index, -c < 1, -L > 256, -g > -L, clusters longer than the reference's
+     * MAX_C_LEN): refused, with no flag set */
+    if (n == 0 || p->consensus_reads < 1 || p->k_left > 256 || p->max_gap > p->k_left || max_clust_length > ORACLE_MAX_C_LEN)
+        return -1;
+    cand_vec cands = {0, 0, 0, 0, 0, 0};
     t_gsa *cl = (t_gsa *)malloc(65536 * sizeof *cl);
     if (!cl) return -1;
     const uint64_t slot = oracle_phantom_slot(lcp[n - 1], text[n - 1], suff[n - 1], bwt[n - 1], x, y, z, bcr);
@@ -441,10 +464,11 @@ int oracle_find_events_w(const uint32_t *lcp, const uint32_t *text, const uint32
     char l0[256], l1[256];
     for (size_t c = 0; c < cands.n && !rc; ++c) {
         const candidate *v = &cands.v[c];
+        const uint64_t *r0 = cands.pool + v->at, *r1 = r0 + 2 * v->n0;
         int supp0 = 0, supp1 = 0;
-        if (consensus_support(v->idx0, v->pos0, v->n0, p->k_left, p->max_err, read_bases, read_off, n_reads, l0,
+        if (consensus_support(r0, r0 + v->n0, v->n0, p->k_left, p->max_err, read_bases, read_off, n_reads, l0,
                               &supp0, &res->flags) ||
-            consensus_support(v->idx1, v->pos1, v->n1, p->k_left, p->max_err, read_bases, read_off, n_reads, l1,
+            consensus_support(r1, r1 + v->n1, v->n1, p->k_left, p->max_err, read_bases, read_off, n_reads, l1,
                               &supp1, &res->flags)) { rc = -1; break; }
         if (!(supp0 > 0 && supp1 > 0)) continue;     /* :595 */
         if (v->right_idx >= n_reads) { res->flags |= ORACLE_FLAG_BAD_READ_REF; rc = -1; break; }
@@ -463,6 +487,7 @@ int oracle_find_events_w(const uint32_t *lcp, const uint32_t *text, const uint32
         }
     }
     free(cands.v);
+    free(cands.pool);
     if (rc) { free(out.s); return -1; }
     *snp_text = out.s;
     *snp_len = out.n;

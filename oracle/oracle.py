@@ -15,6 +15,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "_build", "liboracle.so")
 REF_DIR = os.path.join(HERE, "_ref")
 MAX_C_LEN = 150
+FLAG_SAW_N = 1         # oracle.h ORACLE_FLAG_SAW_N
+FLAG_BAD_READ_REF = 2  # oracle.h ORACLE_FLAG_BAD_READ_REF
 
 
 class Params(C.Structure):
@@ -123,7 +125,10 @@ def find_events(lcp, text, suff, bwt, start, ln, params: Params, max_clust_lengt
     if rc:
         if not strict:  # the candidate count is printed by the reference before it crashes (ref:clust2snp.cpp:859)
             return None, res
-        raise ValueError(f"oracle_find_events: input the reference would crash on (flags={res.flags})")
+        if res.flags & FLAG_BAD_READ_REF:
+            raise ValueError(f"oracle_find_events: input the reference would crash on (flags={res.flags})")
+        raise ValueError("oracle_find_events: options outside what the restatement supports (consensus_reads < 1, k_left > 256, "
+                         "max_gap > k_left, max_clust_length > 150) or an empty index")
     data = C.string_at(out, out_len.value)
     lib().oracle_free(out)
     return data, res
