@@ -505,14 +505,23 @@ static void keep_range(const e2s_shard* s, uint64_t* lo, uint64_t* hi) {
     *hi = h < s->n_global ? h : s->n_global;
 }
 
+// the scan looks at positions [-2, n_local] (on the last shard lcp[n_local] is the phantom, which only feeds END(n-1),
+// left to the host tail rule): only those decide whether the byte copy is usable
+static int64_t checked_hi(const e2s_shard* s) { return int64_t(s->n_local) + (s->global_off + s->n_local == s->n_global ? 0 : 1); }
+
 // every load also writes the narrow resident copies of what it loaded (k_derive): byte LCP + base-code bit planes
 static cudaError_t derive_loaded(e2s_shard* s, int64_t l, uint64_t cnt, bool have_lcp, bool have_bwt) {
-    const bool last_shard = s->global_off + s->n_local == s->n_global;
-    // the scan looks at positions [-2, n_local] (on the last shard lcp[n_local] is the phantom, which only feeds END(n-1),
-    // left to the host tail rule): only those decide whether the byte copy is usable
     return launch_derive(s->lcp, have_bwt ? s->bwt : nullptr, have_lcp ? s->lcpt : nullptr, s->d_planes,
-                         l, l + int64_t(cnt), -2, int64_t(s->n_local) + (last_shard ? 0 : 1), s->d_seal_flag, s->ctx->stream,
-                         s->ctx->sm_count);
+                         l, l + int64_t(cnt), -2, checked_hi(s), s->d_seal_flag, s->ctx->stream, s->ctx->sm_count);
+}
+
+// Called once per LCP load with the global positions [a, b) the whole call writes, before its first piece: a load over all the
+// checked positions (left of global position 0 there is only the zero pad) replaces every value the last verdict came from, so
+// a reloaded shard forgets it.  A partial reload keeps it (conservative: the 4-byte stream, still exact).
+static cudaError_t forget_verdict_if_covered(e2s_shard* s, uint64_t a, uint64_t b) {
+    const int64_t chk_lo = s->global_off >= 2 ? -2 : -int64_t(s->global_off);
+    if (int64_t(a) - int64_t(s->global_off) > chk_lo || int64_t(b) - int64_t(s->global_off) < checked_hi(s)) return cudaSuccess;
+    return cudaMemsetAsync(s->d_seal_flag, 0, 4, s->ctx->stream);
 }
 
 int e2s_shard_load_gesa(e2s_shard* s, const void* records, uint64_t first, uint64_t count, int x, int y, int z) {
@@ -526,6 +535,7 @@ int e2s_shard_load_gesa(e2s_shard* s, const void* records, uint64_t first, uint6
     uint64_t a = first > lo ? first : lo, b = first + count < hi ? first + count : hi;
     if (a >= b) return E2S_OK;
     s->lay_x = x; s->lay_y = y; s->lay_z = z; s->lay_bcr = 0;
+    CU(c, forget_verdict_if_covered(s, a, b));
     const int rs = x + y + z + 1;
     const uint64_t chunk = uint64_t(1) << 22;  // records per H2D chunk (multiple of 16)
     const size_t need = size_t(chunk < (b - a) ? chunk : round_up(b - a, 16)) * rs + 64;
@@ -584,6 +594,7 @@ int e2s_shard_load_gesa_fd(e2s_shard* s, int fd, uint64_t first, uint64_t count,
     const uint64_t a = first > lo ? first : lo, b = first + count < hi ? first + count : hi;
     if (a >= b) return E2S_OK;
     s->lay_x = x; s->lay_y = y; s->lay_z = z; s->lay_bcr = 0;
+    CU(c, forget_verdict_if_covered(s, a, b));
     const int rs = x + y + z + 1;
     constexpr int R = 4;                          // pinned slots
     const uint64_t piece = uint64_t(1) << 20;     // records per piece (multiple of 16)
@@ -703,6 +714,7 @@ static int load_soa(e2s_shard* s, const uint32_t* lcp, const uint32_t* text, con
     if (a >= b) return E2S_OK;
     const int64_t l = int64_t(a) - int64_t(s->global_off);
     const uint64_t so = a - first, cnt = b - a;
+    if (lcp) CU(c, forget_verdict_if_covered(s, a, b));
     if (lcp) CU(c, cudaMemcpyAsync(s->lcp + l, lcp + so, cnt * 4, kind, c->stream));
     if (text) CU(c, cudaMemcpyAsync(s->text + l, text + so, cnt * 4, kind, c->stream));
     if (suff) CU(c, cudaMemcpyAsync(s->suff + l, suff + so, cnt * 4, kind, c->stream));
@@ -773,6 +785,7 @@ static int load_lcp_bwt(e2s_shard* s, const void* lcp, int x, const uint8_t* bwt
     const uint64_t a = first > lo ? first : lo, b = first + count < hi ? first + count : hi;
     if (a >= b) return E2S_OK;
     s->lay_x = x;
+    CU(c, forget_verdict_if_covered(s, a, b));
     const uint8_t* src = static_cast<const uint8_t*>(lcp);
     const int64_t l0 = int64_t(a) - int64_t(s->global_off);
     const cudaMemcpyKind kind = dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
