@@ -80,7 +80,7 @@ class PipelineResult(C.Structure):
 SYMBOLS = [
     "e2s_version", "e2s_ctx_create", "e2s_ctx_destroy", "e2s_last_error", "e2s_ctx_set_stream",
     "e2s_ctx_synchronize", "e2s_ctx_mem_info", "e2s_ctx_launch_count", "e2s_ctx_timing", "e2s_ctx_kernel_time", "e2s_shard_create", "e2s_shard_destroy", "e2s_shard_load_gesa", "e2s_shard_load_gesa_fd",
-    "e2s_shard_load_soa", "e2s_shard_load_soa_dev", "e2s_build_egsa_dev", "e2s_build_egsa", "e2s_build_egsa_ragged_dev", "e2s_build_egsa_ragged", "e2s_build_egsa_range_dev", "e2s_shard_set_layout", "e2s_shard_seal", "e2s_shard_lcp_bytes_resident", "e2s_reads_stage", "e2s_reads_stage_dev",
+    "e2s_shard_load_soa", "e2s_shard_load_soa_dev", "e2s_build_egsa_dev", "e2s_build_egsa", "e2s_build_egsa_ragged_dev", "e2s_build_egsa_ragged", "e2s_build_egsa_range_dev", "e2s_build_egsa_ragged_range_dev", "e2s_shard_set_layout", "e2s_shard_seal", "e2s_shard_lcp_bytes_resident", "e2s_reads_stage", "e2s_reads_stage_dev",
     "e2s_cluster_prefilter", "e2s_cluster_run", "e2s_cluster_merge", "e2s_cluster_finalize", "e2s_cluster_lm", "e2s_cluster_count",
     "e2s_cluster_fetch", "e2s_cluster_fetch_packed", "e2s_clusters_stage_packed", "e2s_clusters_stage",
     "e2s_statistics", "e2s_statistics_finish", "e2s_exchange_finish", "e2s_snp_default_params", "e2s_find_events", "e2s_events_fetch",
@@ -131,6 +131,8 @@ def load_library():
     lib.e2s_build_egsa_ragged.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64] + [C.c_void_p] * 4
     lib.e2s_build_egsa_range_dev.argtypes = ([C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32,
                                               C.c_uint64] + [C.c_void_p] * 4 + [C.POINTER(C.c_uint64)] * 2)
+    lib.e2s_build_egsa_ragged_range_dev.argtypes = ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32,
+                                                     C.c_uint32, C.c_uint64] + [C.c_void_p] * 4 + [C.POINTER(C.c_uint64)] * 2)
     lib.e2s_shard_lcp_bytes_resident.argtypes = [C.c_void_p]
     lib.e2s_shard_set_layout.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.e2s_reads_stage.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
@@ -397,6 +399,32 @@ class Context:
         self._ck(self.lib.e2s_build_egsa_ragged_dev(self.h, _ptr(bases_t), off.ctypes.data, R, _ptr(out["lcp"]), _ptr(out["text"]),
                                                     _ptr(out["suff"]), _ptr(out["bwt"])))
         out.update(n=n, R=R)
+        return out
+
+    def build_egsa_ragged_range(self, bases, off, key_lo, key_hi, before=None, capacity=None):
+        """One key range of the index of reads of any lengths (e2s_build_egsa_ragged_range_dev): `bases` / `off` as for
+        build_egsa_ragged, the range, `before` and `capacity` as for build_egsa_range.  Returns the dict of build_egsa_ragged cut to the
+        range + first = its index position."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        R = len(off) - 1
+        cap = int(off[R]) + R if capacity is None else int(capacity)
+        bases_t = (torch.from_numpy(np.ascontiguousarray(bases, dtype=np.uint8).reshape(-1)) if isinstance(bases, np.ndarray) else bases)
+        if bases_t.numel() == 0:
+            bases_t = torch.zeros(1, dtype=torch.uint8)
+        bases_t = bases_t.to(dev).contiguous()
+        out = {k: torch.empty(max(cap, 1), dtype=torch.int32, device=dev) for k in ("lcp", "text", "suff")}
+        out["bwt"] = torch.empty(max(cap, 1), dtype=torch.uint8, device=dev)
+        n_rec, first = C.c_uint64(0), C.c_uint64(0)
+        bt, bs = (0xFFFFFFFF, 0) if before is None else (int(before[0]), int(before[1]))
+        torch.cuda.synchronize(dev)
+        self._ck(self.lib.e2s_build_egsa_ragged_range_dev(self.h, _ptr(bases_t), off.ctypes.data, R, int(key_lo), int(key_hi), bt, bs, cap,
+                                                          _ptr(out["lcp"]), _ptr(out["text"]), _ptr(out["suff"]), _ptr(out["bwt"]),
+                                                          C.byref(n_rec), C.byref(first)))
+        m = int(n_rec.value)
+        out = {k: v[:m] for k, v in out.items()}
+        out.update(n=m, R=R, first=int(first.value))
         return out
 
     def shard(self, n_local, global_off=0, n_global=None, chunk_positions=None):

@@ -30,8 +30,9 @@
 //                  decoupled look-back per bin, four tiles at a time (one 64-bit tagged word per tile and bin: no clearing
 //                  between passes), keys and ids staged together in shared memory in output order and written in one sweep,
 //                  so every bin leaves as a coalesced run.  The last place of a word moves the ids only.
-//   key ranges     (equal lengths) k_range_select / k_scan_chunks pick the suffixes whose first key word lies in [lo, hi) -- a
-//                  contiguous range of the index -- and the same sort runs on those alone (build_egsa_range).
+//   key ranges     k_range_select / k_scan_chunks pick the suffixes whose first key word lies in [lo, hi) -- a contiguous range
+//                  of the index -- and the same sort runs on those alone (build_egsa_range).  Equal lengths: the selected ids are
+//                  already shortest first.  Ragged: they come in (read, offset) order and the length pass sorts them as above.
 //   k_egsa_finish  decode (r, p); text, suff, bwt; lcp with the previous record = min(len_a - p_a, len_b - p_b, first
 //                  differing symbol) by clz on XORed key words.
 // Ids are 32-bit when they fit (equal lengths: n < 2^32; ragged: R << shift <= 2^32), else 64-bit.
@@ -441,46 +442,119 @@ __global__ void k_egsa_finish(ReadsView v, const uint64_t* __restrict__ packed, 
     if (valid) lcp[i] = l;
 }
 
-// ---- one key range of the index (equal-length reads: the suffix ids are the iota, the length of suffix id i is i / R) ----------
+// ---- one key range of the index ---------------------------------------------------------------------------------------------
 // The suffixes whose first key word (32 symbols, zero padded) lies in [lo, hi) are a contiguous range of the index: a GPU that
-// cannot hold the scratch of the whole collection, or one GPU of several, sorts only those.  Two sweeps over all suffix ids: count
-// per chunk of 4096 ids (+ how many lie below the range, + the selected per length), then a stable compaction into both id buffers.
+// cannot hold the scratch of the whole collection, or one GPU of several, sorts only those.  Two sweeps over all suffix slots: count
+// per chunk of 4096 slots (+ how many lie below the range, + the selected per length), then a stable compaction of their ids.
+//   equal lengths: slot i = suffix id i (the iota, length i / R): the ids go to both id buffers, already shortest first.
+//   ragged:        slot i = suffix (r, p) with start_r + r + p = i, the (read, offset) order of k_init_ids_ragged.  A CTA finds the
+//                  reads its chunk touches (two binary searches over the device offsets), stages their slot starts in shared memory,
+//                  and every thread finds its first read there and walks forward.  The ids (r << shift) | p go to one buffer; the
+//                  length pass then brings them to shortest-first order as in the whole build.
 constexpr int SEL_THREADS = 256;
 constexpr int SEL_IPT = 16;
 constexpr int SEL_CHUNK = SEL_THREADS * SEL_IPT;
+constexpr uint32_t SEL_HIST_BINS = 2048;  // ragged: per-CTA length histogram in shared memory while L + 1 bins fit, else global atomics
 
 struct SelStats {
     unsigned long long n_below;   // suffixes whose first key word is below lo = index position of the range's first record
     unsigned long long n_sel;
 };
 
-template <typename IdT, bool WRITE>
+// ragged: the last read r with start_r + r <= i (the read that owns slot i)
+__device__ __forceinline__ uint64_t read_of_slot(const uint64_t* __restrict__ off, uint64_t R, uint64_t i) {
+    uint64_t a = 0, b = R;  // off[a] + a <= i < off[b] + b
+    while (b - a > 1) {
+        const uint64_t m = a + ((b - a) >> 1);
+        if (off[m] + m <= i) a = m;
+        else b = m;
+    }
+    return a;
+}
+
+template <typename IdT, bool WRITE, bool RAGGED>
 __global__ void __launch_bounds__(SEL_THREADS) k_range_select(ReadsView v, const uint64_t* __restrict__ packed, uint64_t n, uint64_t lo, uint64_t hi,
                                                               uint64_t* __restrict__ chunk_cnt, unsigned long long* __restrict__ len_hist,
                                                               SelStats* __restrict__ stats, IdT* __restrict__ out0, IdT* __restrict__ out1) {
     __shared__ uint32_t s_w[SEL_THREADS / 32];
     __shared__ uint32_t s_below, s_first_len_cnt;
+    // ragged: slot starts of the chunk's reads r0 + k relative to r0's (k <= SEL_CHUNK: every read after r0 owns a slot of the
+    // chunk), and the chunk's length histogram
+    __shared__ uint32_t s_start[RAGGED ? SEL_CHUNK + 1 : 1];
+    __shared__ uint32_t s_hist[RAGGED && !WRITE ? SEL_HIST_BINS : 1];
+    __shared__ uint64_t s_r[3];  // ragged: r0 = the read of the chunk's first slot, r1 = of its last, off[r0]
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint64_t base = uint64_t(blockIdx.x) * SEL_CHUNK + uint64_t(tid) * SEL_IPT;
-    const uint64_t first_len = uint64_t(blockIdx.x) * SEL_CHUNK / v.R;  // the length of the chunk's first suffix
+    const uint64_t chunk_base = uint64_t(blockIdx.x) * SEL_CHUNK;
+    const uint64_t base = chunk_base + uint64_t(tid) * SEL_IPT;
+    const uint64_t first_len = RAGGED ? 0 : chunk_base / v.R;  // equal lengths: the length of the chunk's first suffix
+    const bool shared_hist = RAGGED && !WRITE && v.L < SEL_HIST_BINS;
     if (tid == 0) { s_below = 0; s_first_len_cnt = 0; }
+    if (RAGGED) {
+        if (tid == 0) {
+            s_r[0] = read_of_slot(v.off, v.R, chunk_base);
+            s_r[2] = v.off[s_r[0]];
+        }
+        if (tid == 32) s_r[1] = read_of_slot(v.off, v.R, (chunk_base + SEL_CHUNK < n ? chunk_base + SEL_CHUNK : n) - 1);
+        if (shared_hist)
+            for (uint32_t b = tid; b <= v.L; b += SEL_THREADS) s_hist[b] = 0;
+        __syncthreads();
+        const uint64_t r0 = s_r[0], st0 = s_r[2] + r0;
+        const uint32_t nr = uint32_t(s_r[1] - r0) + 2;  // reads r0 .. r1 and the start of the one after
+        for (uint32_t k = tid; k < nr; k += SEL_THREADS) s_start[k] = uint32_t(v.off[r0 + k] + r0 + k - st0);
+    }
     __syncthreads();
+    // the thread's first slot: read r = r0 + k, offset p, length len, bases from st
+    uint64_t r = 0, st = 0;
+    uint32_t k = 0, p = 0, len = v.L;
+    const uint64_t r0 = RAGGED ? s_r[0] : 0;
+    if (RAGGED && base < n) {
+        const uint32_t b = uint32_t(base - (s_r[2] + r0));
+        uint32_t a = 0, z = uint32_t(s_r[1] - r0) + 1;  // s_start[a] <= b < s_start[z]
+        while (z - a > 1) {
+            const uint32_t m = (a + z) >> 1;
+            if (s_start[m] <= b) a = m;
+            else z = m;
+        }
+        k = a;
+        p = b - s_start[k];
+        len = s_start[k + 1] - s_start[k] - 1;
+        r = r0 + k;
+        st = s_r[2] + s_start[k] - k;
+    }
+    const uint32_t k_first = k, p_first = p;
     uint32_t sel = 0, below = 0, at_first_len = 0;
 #pragma unroll 4
     for (int j = 0; j < SEL_IPT; ++j) {
         const uint64_t i = base + j;
         if (i < n) {
-            uint64_t r;
-            uint32_t p;
-            v.decode(IdT(i), r, p);
-            const uint64_t key = suffix_word(packed + v.row(r, v.start(r)), v.L, p, 0);
+            uint32_t q;
+            if (RAGGED) {
+                if (p > len) {  // past read r's terminator: the next read (every read owns at least its terminator slot)
+                    ++k;
+                    p = 0;
+                    len = s_start[k + 1] - s_start[k] - 1;
+                    r = r0 + k;
+                    st += (s_start[k] - s_start[k - 1]) - 1;
+                }
+                q = p++;
+            } else {
+                v.decode(IdT(i), r, q);
+                st = v.start(r);
+            }
+            const uint64_t key = suffix_word(packed + v.row(r, st), len, q, 0);
             if (key < lo) ++below;
             else if (hi == 0 || key < hi) {
                 sel |= 1u << j;
                 if (!WRITE) {
-                    const uint64_t len = uint64_t(v.L - p);
-                    if (len == first_len) ++at_first_len;
-                    else atomicAdd(len_hist + len, 1ull);  // (a chunk seldom spans two lengths)
+                    const uint32_t sl = len - q;
+                    if (RAGGED) {
+                        if (shared_hist) atomicAdd(&s_hist[sl], 1u);
+                        else atomicAdd(len_hist + sl, 1ull);
+                    } else if (sl == first_len) {
+                        ++at_first_len;
+                    } else {
+                        atomicAdd(len_hist + sl, 1ull);  // (a chunk seldom spans two lengths)
+                    }
                 }
             }
         }
@@ -512,15 +586,33 @@ __global__ void __launch_bounds__(SEL_THREADS) k_range_select(ReadsView v, const
             if (total) atomicAdd(&stats->n_sel, (unsigned long long)total);
             if (s_first_len_cnt) atomicAdd(len_hist + first_len, (unsigned long long)s_first_len_cnt);
         }
+        if (shared_hist)
+            for (uint32_t b = tid; b <= v.L; b += SEL_THREADS)
+                if (s_hist[b]) atomicAdd(len_hist + b, (unsigned long long)s_hist[b]);
     } else {
         uint64_t at = chunk_cnt[blockIdx.x] + wbase + inc - cnt;
-#pragma unroll 4
-        for (int j = 0; j < SEL_IPT; ++j)
-            if (sel & (1u << j)) {
-                out0[at] = IdT(base + j);
-                out1[at] = IdT(base + j);
-                ++at;
+        if (RAGGED) {  // the same walk again, ids in (read, offset) order
+            k = k_first;
+            p = p_first;
+            len = s_start[k + 1] - s_start[k] - 1;
+            for (int j = 0; j < SEL_IPT && sel >> j; ++j) {
+                if (p > len) {
+                    ++k;
+                    p = 0;
+                    len = s_start[k + 1] - s_start[k] - 1;
+                }
+                if (sel & (1u << j)) out0[at++] = IdT(((r0 + k) << v.shift) | p);
+                ++p;
             }
+        } else {
+#pragma unroll 4
+            for (int j = 0; j < SEL_IPT; ++j)
+                if (sel & (1u << j)) {
+                    out0[at] = IdT(base + j);
+                    out1[at] = IdT(base + j);
+                    ++at;
+                }
+        }
     }
 }
 
@@ -605,15 +697,17 @@ cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const
     }
     const uint64_t n_chunks = (n_all + SEL_CHUNK - 1) / SEL_CHUNK;
     if (range) {  // first sweep: who is in the range
-        if (v.shift || n_chunks >= (uint64_t(1) << 31)) return done(cudaErrorInvalidConfiguration);
+        if (n_chunks >= (uint64_t(1) << 31)) return done(cudaErrorInvalidConfiguration);
         const size_t sel_bytes = (size_t(v.L) + 1) * 8 + sizeof(SelStats);
         if ((e = cudaMalloc(reinterpret_cast<void**>(&chunk_cnt), n_chunks * 8)) != cudaSuccess) return done(e);
         if ((e = cudaMalloc(reinterpret_cast<void**>(&sel_misc), sel_bytes)) != cudaSuccess) return done(e);
         if ((e = cudaMemsetAsync(sel_misc, 0, sel_bytes, stream)) != cudaSuccess) return done(e);
         unsigned long long* len_hist = reinterpret_cast<unsigned long long*>(sel_misc);
         SelStats* stats = reinterpret_cast<SelStats*>(sel_misc + v.L + 1);
-        k_range_select<IdT, false><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n_all, range->lo, range->hi, chunk_cnt, len_hist, stats,
-                                                                                   nullptr, nullptr);
+        if (v.shift) k_range_select<IdT, false, true><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n_all, range->lo, range->hi, chunk_cnt,
+                                                                                                      len_hist, stats, nullptr, nullptr);
+        else k_range_select<IdT, false, false><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n_all, range->lo, range->hi, chunk_cnt,
+                                                                                                len_hist, stats, nullptr, nullptr);
         k_scan_chunks<<<1, 1024, 0, stream>>>(chunk_cnt, n_chunks);
         *launches += 2;
         std::vector<uint64_t> h(size_t(v.L) + 1 + sizeof(SelStats) / 8);
@@ -635,8 +729,13 @@ cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const
     if ((e = cudaMalloc(reinterpret_cast<void**>(&i0), n * sizeof(IdT))) != cudaSuccess) return done(e);
     if ((e = cudaMalloc(reinterpret_cast<void**>(&i1), n * sizeof(IdT))) != cudaSuccess) return done(e);
     if ((e = cudaMemsetAsync(status, 0, tiles * 256 * 8, stream)) != cudaSuccess) return done(e);  // tag 0 = no pass
-    if (range) {  // second sweep: the selected ids, in id order (= shortest first, then read id), into both buffers
-        k_range_select<IdT, true><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n_all, range->lo, range->hi, chunk_cnt, nullptr, nullptr, i0, i1);
+    if (range && v.shift) {  // second sweep, ragged: the selected ids in (read, offset) order, sorted by length below
+        k_range_select<IdT, true, true><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n_all, range->lo, range->hi, chunk_cnt, nullptr, nullptr,
+                                                                                        i0, nullptr);
+        *launches += 1;
+    } else if (range) {  // second sweep, equal lengths: the selected ids in id order (= shortest first, then read id), into both buffers
+        k_range_select<IdT, true, false><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n_all, range->lo, range->hi, chunk_cnt, nullptr, nullptr,
+                                                                                         i0, i1);
         *launches += 1;
     } else if (v.shift) {
         k_init_ids_ragged<IdT><<<blocks_for(v.R * 32, 256), 256, 0, stream>>>(v, i0);
@@ -677,6 +776,7 @@ cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const
         }
         const uint64_t first = first_of[places - 1];  // the widest range: what the word's keys are made for
         const uint64_t m = n - first;
+        if (m == 0) return;  // (a key range whose suffixes are all too short for the word)
         PlaceSkip skip;
         for (uint32_t j = 0; j < MAX_PLACES; ++j) skip.n[j] = j < places ? first_of[j] - first : 0;
         const uint64_t hist_blocks_want = (m + 255) / 256;
@@ -688,6 +788,7 @@ cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const
         for (uint32_t j = 0; j < places; ++j, ++seq) {
             const uint32_t sh = begin_bit + 8 * j;
             const uint64_t f = first_of[j], mj = n - f;
+            if (mj == 0) continue;  // nothing long enough for this place: no pass, the current buffers stay current
             const unsigned tiles_j = unsigned((mj + RS_TILE - 1) / RS_TILE);
             const bool wk = j + 1 < places;  // the keys of a word are not looked at again after its last place
             if (rs_threads == 512) {
@@ -718,6 +819,13 @@ cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const
     return done(cudaSuccess);
 }
 
+// ragged ids (r << shift) | p: the bits of p in [0, L]
+inline uint32_t ragged_shift(uint32_t L) {
+    uint32_t bits = 1;
+    while ((L >> bits) != 0) ++bits;
+    return bits;
+}
+
 }  // namespace
 
 // d_off == nullptr: R reads of L bases each; else R + 1 DEVICE offsets (h_off = the same on the host), L = the longest read,
@@ -736,10 +844,8 @@ cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint
     bool wide;
     if (d_off) {
         if (L >= 65536 || !h_off) return cudaErrorInvalidConfiguration;
-        uint32_t bits = 1;
-        while ((L >> bits) != 0) ++bits;  // p in [0, L]
-        v.shift = bits;
-        wide = R > (uint64_t(1) << (32 - bits));
+        v.shift = ragged_shift(L);
+        wide = R > (uint64_t(1) << (32 - v.shift));
         std::vector<uint64_t> at_least(size_t(L) + 2, 0);  // reads of t bases or more
         for (uint64_t r = 0; r < R; ++r) ++at_least[size_t(h_off[r + 1] - h_off[r])];
         for (uint32_t t = L; t-- > 0;) at_least[t] += at_least[t + 1];
@@ -754,27 +860,34 @@ cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint
                 : build_typed<uint32_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, stream, launches);
 }
 
-// One key range of the index of R reads of L bases each: the records of the suffixes whose first key word (32 symbols at 2 bits,
-// A=0 C=1 G=2 T=3, most significant first, zero padded) lies in [key_lo, key_hi) (key_hi == 0: no upper bound) -- a contiguous range
-// of the index, *first_out = the index position of its first record, *n_out = how many there are (also set when they exceed
-// `cap`: cudaErrorInvalidPitchValue, nothing written).  before = the record that precedes the range (text << 32 | suff) for
-// lcp[0], ~0 = none / not known (lcp[0] = 0).  Scratch: 24.5 / 32.5 bytes per suffix OF THE RANGE + 8 bytes per 4096 suffixes.
-cudaError_t build_egsa_range(const uint8_t* d_reads, uint64_t R, uint32_t L, uint64_t key_lo, uint64_t key_hi, uint64_t before, uint64_t cap,
-                             uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, uint64_t* n_out, uint64_t* first_out,
-                             cudaStream_t stream, uint64_t* launches) {
+// One key range of the index: the records of the suffixes whose first key word (32 symbols at 2 bits, A=0 C=1 G=2 T=3, most
+// significant first, zero padded) lies in [key_lo, key_hi) (key_hi == 0: no upper bound) -- a contiguous range of the index,
+// *first_out = the index position of its first record, *n_out = how many there are (also set when they exceed `cap`:
+// cudaErrorInvalidPitchValue, nothing written).  before = the record that precedes the range (text << 32 | suff) for lcp[0], ~0 =
+// none / not known (lcp[0] = 0).  d_off == nullptr: R reads of L bases each; else R + 1 DEVICE offsets, L = the longest read,
+// total_bases = off[R].  The id width is the whole collection's, as in build_egsa.  Scratch: 24.5 / 32.5 bytes per suffix OF THE
+// RANGE + 8 bytes per 4096 suffixes of the collection.
+cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint64_t key_lo,
+                             uint64_t key_hi, uint64_t before, uint64_t cap, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt,
+                             uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches) {
     ReadsView v;
     v.bases = d_reads;
-    v.off = nullptr;
+    v.off = d_off;
     v.R = R;
     v.L = L;
     v.shift = 0;
-    const uint64_t n = R * (uint64_t(L) + 1);
-    std::vector<uint64_t> n_le(size_t(L) + 1, 0);
-    for (uint32_t t = 0; t <= L; ++t) n_le[t] = R * (uint64_t(t) + 1);
+    const uint64_t n = total_bases + R;
+    bool wide = n > 0xffffffffull;
+    if (d_off) {
+        if (L >= 65536) return cudaErrorInvalidConfiguration;
+        v.shift = ragged_shift(L);
+        wide = R > (uint64_t(1) << (32 - v.shift));
+    }
+    if (getenv("E2S_BUILD_IDS64")) wide = true;
     KeyRange range{key_lo, key_hi, cap, before, 0, 0};
-    const bool wide = n > 0xffffffffull || getenv("E2S_BUILD_IDS64");
-    const cudaError_t e = wide ? build_typed<uint64_t>(v, n, R * uint64_t(L), n_le.data(), &range, d_lcp, d_text, d_suff, d_bwt, stream, launches)
-                               : build_typed<uint32_t>(v, n, R * uint64_t(L), n_le.data(), &range, d_lcp, d_text, d_suff, d_bwt, stream, launches);
+    // (the suffix lengths of a range come from its selection sweep: no whole-collection n_le)
+    const cudaError_t e = wide ? build_typed<uint64_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, stream, launches)
+                               : build_typed<uint32_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, stream, launches);
     *n_out = range.n_out;
     *first_out = range.first_out;
     return e;

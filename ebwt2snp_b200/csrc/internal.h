@@ -224,10 +224,11 @@ cudaError_t launch_fill_phantom(uint32_t* lcp, uint32_t* text, uint32_t* suff, u
 cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint64_t* h_off, uint64_t R, uint32_t L, uint64_t total_bases,
                        uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches);
 
-// one key range of the index of R reads of L bases (see build_egsa.cu); cudaErrorInvalidPitchValue = more than `cap` records (*n_out says how many)
-cudaError_t build_egsa_range(const uint8_t* d_reads, uint64_t R, uint32_t L, uint64_t key_lo, uint64_t key_hi, uint64_t before, uint64_t cap,
-                             uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, uint64_t* n_out, uint64_t* first_out,
-                             cudaStream_t stream, uint64_t* launches);
+// one key range of the index (see build_egsa.cu); reads as for build_egsa (d_off == nullptr: R reads of L bases), no host offsets needed;
+// cudaErrorInvalidPitchValue = more than `cap` records (*n_out says how many)
+cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint64_t key_lo,
+                             uint64_t key_hi, uint64_t before, uint64_t cap, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt,
+                             uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches);
 
 // ---- phase 2 -----------------------------------------------------------------------------------
 struct SnpDev {  // device counters of one e2s_find_events

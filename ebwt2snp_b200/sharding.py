@@ -38,37 +38,57 @@ def shard_cuts(n, parts):
 
 def first_key_words(reads, rows, cols):
     """the 64-bit first key word (32 symbols at 2 bits, A=0 C=1 G=2 T=3, first symbol most significant, zero padded) of the suffixes
-    (rows[i], cols[i]) of the (R, L) read matrix: what e2s_build_egsa_range_dev compares with its key range"""
-    reads = np.asarray(reads)
-    L = reads.shape[1]
+    (rows[i], cols[i]) = (read, offset): what e2s_build_egsa_range_dev / e2s_build_egsa_ragged_range_dev compare with their key range.
+    `reads` = the (R, L) read matrix, or a ragged collection (bases, off): all reads back to back + R + 1 offsets."""
     code = np.zeros(256, dtype=np.uint64)
     for c, v in ((b"C", 1), (b"c", 1), (b"G", 2), (b"g", 2), (b"T", 3), (b"t", 3)):
         code[c[0]] = v
     rows = np.asarray(rows, dtype=np.int64)
     cols = np.asarray(cols, dtype=np.int64)
+    if isinstance(reads, tuple):
+        bases = np.asarray(reads[0], dtype=np.uint8).reshape(-1)
+        off = np.asarray(reads[1], dtype=np.int64)
+        start, end = off[rows] + cols, off[rows + 1]
+        last = max(len(bases) - 1, 0)
+        fetch = lambda at: code[bases[np.minimum(at, last)]] if len(bases) else np.zeros(len(at), dtype=np.uint64)  # noqa: E731
+    else:
+        reads = np.asarray(reads)
+        L = reads.shape[1]
+        start, end = cols, np.full(len(rows), L, dtype=np.int64)
+        fetch = lambda at: code[reads[rows, np.minimum(at, L - 1)]]  # noqa: E731
     key = np.zeros(len(rows), dtype=np.uint64)
     for j in range(32):
-        at = cols + j
-        inside = at < L
-        sym = np.where(inside, code[reads[rows, np.minimum(at, L - 1)]], np.uint64(0))
+        at = start + j
+        sym = np.where(at < end, fetch(at), np.uint64(0))
         key = (key << np.uint64(2)) | sym
     return key
 
 
 def key_range_cuts(parts, reads=None, sample=1 << 16, seed=0):
     """`parts` key ranges [(lo, hi), ...] that tile the 64-bit key space (hi = 0 on the last one: no upper bound) -- one per rank (or
-    per pass) for e2s_build_egsa_range_dev.  Without reads: equal slices of the key space.  With the (R, L) read matrix: the cuts are
-    quantiles of the first key words of `sample` random suffixes, so the ranges hold about the same number of records whatever the
-    base composition (the terminator suffixes, 4/3 R records under key 0, stay in the first range)."""
+    per pass) for e2s_build_egsa_range_dev / e2s_build_egsa_ragged_range_dev.  Without reads: equal slices of the key space.  With the
+    (R, L) read matrix or a ragged collection (bases, off): the cuts are quantiles of the first key words of `sample` suffixes drawn
+    uniformly over all suffix slots, terminator suffixes included, so the ranges hold about the same number of records whatever the
+    base composition (the terminator suffixes, and every suffix with an all-A first word, share key 0 and stay in the first range)."""
     parts = max(1, int(parts))
     if reads is None:
         cuts = [(i << 64) // parts for i in range(parts)]
     else:
-        reads = np.asarray(reads)
-        R, L = reads.shape
         rng = np.random.default_rng(seed)
-        m = int(min(sample, R * (L + 1)))
-        keys = np.sort(first_key_words(reads, rng.integers(0, R, size=m), rng.integers(0, L + 1, size=m)))
+        if isinstance(reads, tuple):
+            off = np.asarray(reads[1], dtype=np.int64)
+            R = len(off) - 1
+            slot0 = off + np.arange(R + 1)  # slot of (r, 0); read r owns slots [slot0[r], slot0[r + 1])
+            m = int(min(sample, slot0[R]))
+            slots = rng.integers(0, slot0[R], size=m)
+            rows = np.searchsorted(slot0, slots, side="right") - 1
+            cols = slots - slot0[rows]
+        else:
+            reads = np.asarray(reads)
+            R, L = reads.shape
+            m = int(min(sample, R * (L + 1)))
+            rows, cols = rng.integers(0, R, size=m), rng.integers(0, L + 1, size=m)
+        keys = np.sort(first_key_words(reads, rows, cols))
         cuts = [0] + [int(keys[(i * m) // parts]) for i in range(1, parts)]
         for i in range(1, parts):  # strictly increasing (a heavy key value cannot be cut: the ranges after it start past it)
             cuts[i] = max(cuts[i], cuts[i - 1] + 1)

@@ -126,7 +126,7 @@ int e2s_build_egsa_ragged_dev(e2s_ctx *ctx, const uint8_t *d_bases, const uint64
 int e2s_build_egsa_ragged(e2s_ctx *ctx, const uint8_t *bases, const uint64_t *off, uint64_t n_reads, uint32_t *lcp,
                           uint32_t *text, uint32_t *suff, uint8_t *bwt);
 
-/* ONE KEY RANGE of the index of n_reads equal-length reads: the suffixes whose first 32 symbols -- as a 64-bit word at 2 bits per
+/* ONE KEY RANGE of the index of n_reads equal-length reads (any lengths: e2s_build_egsa_ragged_range_dev below): the suffixes whose first 32 symbols -- as a 64-bit word at 2 bits per
  * base (A=0 C=1 G=2 T=3, first symbol most significant, zero padded past the end of the read) -- lie in [key_lo, key_hi)
  * (key_hi = 0: no upper bound) are a contiguous range of the index.  Writes their records to the DEVICE arrays (capacity
  * records each), *n_records = how many, *first_position = the index position of the first one.  What a collection too large for one
@@ -137,6 +137,15 @@ int e2s_build_egsa_ragged(e2s_ctx *ctx, const uint8_t *bases, const uint64_t *of
 int e2s_build_egsa_range_dev(e2s_ctx *ctx, const uint8_t *d_reads, uint64_t n_reads, uint32_t read_len, uint64_t key_lo,
                              uint64_t key_hi, uint32_t before_text, uint32_t before_suff, uint64_t capacity, uint32_t *d_lcp,
                              uint32_t *d_text, uint32_t *d_suff, uint8_t *d_bwt, uint64_t *n_records, uint64_t *first_position);
+
+/* The same for reads of ANY lengths: d_bases / off as for e2s_build_egsa_ragged_dev (off = n_reads + 1 HOST offsets, checked the
+ * same way).  The suffix ids follow the whole collection (64-bit when n_reads << bits(longest read + 1) exceeds 2^32), so the ranges of
+ * one collection concatenate to exactly the index e2s_build_egsa_ragged_dev writes.  Capacity, before and errors as above; a base
+ * outside ACGT or a read of 65536 bases or more: E2S_ERR_UNSUPPORTED.  e2s_build_egsa_ragged switches to these ranges by itself when
+ * the whole index does not fit the device. */
+int e2s_build_egsa_ragged_range_dev(e2s_ctx *ctx, const uint8_t *d_bases, const uint64_t *off, uint64_t n_reads, uint64_t key_lo,
+                                    uint64_t key_hi, uint32_t before_text, uint32_t before_suff, uint64_t capacity, uint32_t *d_lcp,
+                                    uint32_t *d_text, uint32_t *d_suff, uint8_t *d_bwt, uint64_t *n_records, uint64_t *first_position);
 
 /* Layout of the index files the shard was loaded from: byte widths of lcp (x), text (y), suff (z) and whether it
  * was the BCR triple.  Only the reference's post-EOF phantom record depends on it (DESIGN.md section 5).
