@@ -10,9 +10,11 @@ n_analysed / n_candidates / n_events and the .snp text.
 (B) three fused shards of one index (cut through clusters: adopted records) rerun three times.
 (C) one resident shard reloaded with another index of the same n through every loader, whole and in pieces; the seal
     verdict (an LCP value above 127) follows the data.
-(D) e2s_pipeline_host / e2s_pipeline_host_soa in sequence on one context (its cached shard).
+(D) e2s_pipeline_host / e2s_pipeline_host_soa in sequence on one context (its cached shard); a fresh context whose first
+    streamed call is the lean one, then .gesa loads.
 (E) one chunked shard over several passes with e2s_chunked_reset: scan passes, an abandoned pass, a clust2snp pass, lean.
-(F) a one-rank NCCL communicator: e2s_pipeline_sharded and e2s_chunked_exchange repeated.
+(F) a one-rank NCCL communicator: e2s_pipeline_sharded and e2s_chunked_exchange repeated; e2s_pipeline_host_sharded under
+    two chunk sizes.
 (G) reads restaged between steps: bigger, smaller, with non-ACGT bytes, ragged.
 """
 import os
@@ -494,6 +496,25 @@ def test_cached_shard_sequence(ctx, monkeypatch):
     host_call(ctx, B)
 
 
+def test_fresh_context_lean_first(built, gesa_file):
+    """A context whose first streamed call is the lean pipeline: the .gesa loads after it (e2s_pipeline_host's chunks, a
+    resident shard loaded from a file descriptor) use the copy stream it made and the events they share with it."""
+    d = data(1)
+    c = api.Context(0)
+    try:
+        host_call(c, d, soa=True)
+        host_call(c, d)
+        sh = c.shard(d.n)
+        try:
+            load(sh, d, "gesa_fd", (4, 4, 4), 0, d.n, gesa_file)
+            sh.seal()
+            step(sh, d, what="resident from a file descriptor after the streamed calls")
+        finally:
+            sh.close()
+    finally:
+        c.close()
+
+
 # ---------------------------------------------------------------------------------------------------------------------------
 # (E) one chunked shard over several passes (the C4 loop)
 # ---------------------------------------------------------------------------------------------------------------------------
@@ -661,7 +682,7 @@ def comm(ctx):
     cm.close()
 
 
-def test_one_rank_sharded_steps(ctx, comm):
+def test_one_rank_sharded_steps(ctx, comm, monkeypatch):
     A, B = data(1, tail=True), data(2)
     ctx.stage_reads(A.reads, A.off)
     sh = resident(ctx, A)
@@ -700,6 +721,21 @@ def test_one_rank_sharded_steps(ctx, comm):
             assert api.events_format(sh.events(), params(d)) == w.text, what
     finally:
         sh.close()
+    # e2s_pipeline_host_sharded twice on the context's cached shard, the second time with another chunk size
+    rec = synth.gesa_records(A.eg()).view(np.uint8).reshape(-1)
+    w, p = want(A), params(A)
+    for chunk in (str(T), "100003"):
+        monkeypatch.setenv("E2S_CHUNK_POSITIONS", chunk)
+        rec10 = np.empty((len(w.es) + 16) * 10, dtype=np.uint8)
+        evbuf = (api.Event * (w.res.n_candidates + 16))()
+        res, mg, st, m = api.pipeline_host_sharded(ctx, comm, rec, 0, 0, A.n, A.n, A.reads.reshape(-1), A.off, p, 16, 2, rec10=rec10,
+                                                   events=evbuf)
+        what = ("host_sharded", chunk)
+        assert m == len(w.es) and rec10[:m * 10].tobytes() == w.clusters, what
+        assert (res.n_written, res.n_clust_out, res.max_clust_length) == (len(w.es), w.enc, w.mcl), what
+        assert (mg.total_written, st.max_clust_length) == (len(w.es), w.mcl), what
+        check_counts(res.snp, w, what)
+        assert api.events_format(list(evbuf)[:res.snp.n_variants], p) == w.text, what
 
 
 # ---------------------------------------------------------------------------------------------------------------------------
