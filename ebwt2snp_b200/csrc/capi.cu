@@ -244,10 +244,19 @@ int e2s_ctx_create(int device, e2s_ctx** out) {
     CU(nullptr, cudaGetDeviceProperties(&prop, device));
     if (prop.major < 10)
         return fail(nullptr, E2S_ERR_CUDA, "device is not sm_100 class: the kernels are built for sm_100a only");
+    int sm_count = prop.multiProcessorCount;
+    if (const char* e = getenv("E2S_SM_COUNT")) {  // test hook: size every grid for fewer SMs, so CTAs loop at small inputs
+        char* end = nullptr;
+        const long v = strtol(e, &end, 10);
+        if (end == e || *end || v < 1 || v > prop.multiProcessorCount)
+            return fail(nullptr, E2S_ERR_ARG, std::string("E2S_SM_COUNT=") + e + ": expected 1.." +
+                                                  std::to_string(prop.multiProcessorCount) + " (the device's SM count)");
+        sm_count = int(v);
+    }
     CU(nullptr, cudaSetDevice(device));
     e2s_ctx* c = new e2s_ctx();
     c->device = device;
-    c->sm_count = prop.multiProcessorCount;
+    c->sm_count = sm_count;
     e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         delete c;
@@ -605,7 +614,7 @@ int e2s_shard_load_gesa(e2s_shard* s, const void* records, uint64_t first, uint6
         CU(c, cudaEventRecord(c->ev_copied[buf], c->copy_stream));
         CU(c, cudaStreamWaitEvent(c->stream, c->ev_copied[buf], 0));
         const int64_t l = int64_t(p) - int64_t(s->global_off);  // local index, may be -2 / -1
-        CU(c, launch_unpack_gesa(c->d_raw[buf], cnt, x, y, z, s->lcp + l, s->text + l, s->suff + l, s->bwt + l, c->stream));
+        CU(c, launch_unpack_gesa(c->d_raw[buf], cnt, x, y, z, s->lcp + l, s->text + l, s->suff + l, s->bwt + l, c->stream, c->sm_count));
         CU(c, cudaEventRecord(c->ev_unpacked[buf], c->stream));
         CU(c, derive_loaded(s, l, cnt, true, true));
         c->launches += 2;
@@ -703,7 +712,7 @@ int e2s_shard_load_gesa_fd(e2s_shard* s, int fd, uint64_t first, uint64_t count,
         recorded.store(int64_t(p), std::memory_order_release);
         if (ce == cudaSuccess) ce = cudaStreamWaitEvent(c->stream, c->ev_copied[buf], 0);
         const int64_t l = int64_t(p0) - int64_t(s->global_off);  // local index, may be negative (left context)
-        if (ce == cudaSuccess) ce = launch_unpack_gesa(c->d_raw[buf], cnt, x, y, z, s->lcp + l, s->text + l, s->suff + l, s->bwt + l, c->stream);
+        if (ce == cudaSuccess) ce = launch_unpack_gesa(c->d_raw[buf], cnt, x, y, z, s->lcp + l, s->text + l, s->suff + l, s->bwt + l, c->stream, c->sm_count);
         if (ce == cudaSuccess) ce = cudaEventRecord(c->ev_unpacked[buf], c->stream);
         if (ce == cudaSuccess) ce = derive_loaded(s, l, cnt, true, true);
         c->launches += 2;

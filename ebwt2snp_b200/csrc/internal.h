@@ -206,7 +206,7 @@ cudaError_t launch_pack_records(const uint64_t* d_start, const uint16_t* d_len, 
 // AoS records -> SoA.  d_rec: `count` records of (y+z+x+1) bytes; outputs are pointers to the element
 // that receives record 0 (any may be null).
 cudaError_t launch_unpack_gesa(const uint8_t* d_rec, uint64_t count, int x, int y, int z, uint32_t* lcp, uint32_t* text,
-                               uint32_t* suff, uint8_t* bwt, cudaStream_t stream);
+                               uint32_t* suff, uint8_t* bwt, cudaStream_t stream, int sm_count);
 // narrow resident copies of the local positions [a, b) just loaded (byte LCP + base-code bit planes); *flag |= 1 when an
 // LCP value in [chk_lo, chk_hi) does not fit the byte copy
 cudaError_t launch_derive(const uint32_t* lcp, const uint8_t* bwt, uint8_t* lcpt, uint4* planes, int64_t a, int64_t b,

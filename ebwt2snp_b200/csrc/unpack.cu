@@ -47,14 +47,15 @@ __global__ void __launch_bounds__(UP_THREADS) k_unpack_gesa(const uint8_t* __res
 }
 
 cudaError_t launch_unpack_gesa(const uint8_t* d_rec, uint64_t count, int x, int y, int z, uint32_t* lcp, uint32_t* text,
-                               uint32_t* suff, uint8_t* bwt, cudaStream_t stream) {
+                               uint32_t* suff, uint8_t* bwt, cudaStream_t stream, int sm_count) {
     if (count == 0) return cudaSuccess;
     const int rs = x + y + z + 1;
     const size_t smem = size_t(UP_RECS) * rs + 16;
     cudaError_t e = cudaFuncSetAttribute(k_unpack_gesa, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return e;
     uint64_t n_tiles = (count + UP_RECS - 1) / UP_RECS;
-    unsigned grid = unsigned(n_tiles < 148 * 8 ? n_tiles : 148 * 8);
+    const uint64_t cap = uint64_t(sm_count) * 8;
+    const unsigned grid = unsigned(n_tiles < cap ? n_tiles : cap);
     k_unpack_gesa<<<grid, UP_THREADS, smem, stream>>>(d_rec, count, x, y, z, lcp, text, suff, bwt);
     return cudaGetLastError();
 }

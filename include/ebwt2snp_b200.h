@@ -53,6 +53,8 @@ typedef struct e2s_comm e2s_comm; /* one process per GPU: wraps an NCCL communic
  * context
  * ------------------------------------------------------------------------------------- */
 int e2s_version(void);
+/* E2S_SM_COUNT=s in the environment (a test hook, 1 <= s <= the device's SM count, else E2S_ERR_ARG) sizes every grid of
+ * the context for s SMs, so that CTAs loop over many tiles and grid-stride rounds at small inputs. */
 int e2s_ctx_create(int device, e2s_ctx **out);
 void e2s_ctx_destroy(e2s_ctx *ctx);
 /* last error message of the context (or of the calling thread when ctx == NULL) */

@@ -205,6 +205,12 @@ def shifted(case):
 
 @pytest.mark.parametrize("lean", [False, True])
 def test_pipeline_host_chunk_inside_cluster(ctx, sub, lean, monkeypatch):
+    monkeypatch.setenv("E2S_CHUNK_POSITIONS", str(CHUNK))
+    pipeline_host_chunked(ctx, sub, lean)
+
+
+def pipeline_host_chunked(ctx, sub, lean):
+    """e2s_pipeline_host (lean: _soa) with a chunk boundary inside a designed cluster; E2S_CHUNK_POSITIONS set by the caller"""
     case, want = sub
     case, pad = shifted(case)
     if pad:
@@ -212,7 +218,6 @@ def test_pipeline_host_chunk_inside_cluster(ctx, sub, lean, monkeypatch):
     otext, ores, es, el = want
     p = params(case)
     n = case.n
-    monkeypatch.setenv("E2S_CHUNK_POSITIONS", str(CHUNK))
     rec10 = np.empty((len(es) + 16) * 10, dtype=np.uint8)
     evbuf = (api.Event * (ores.n_candidates + 16))()
     if lean:
@@ -230,6 +235,11 @@ def test_pipeline_host_chunk_inside_cluster(ctx, sub, lean, monkeypatch):
 
 @pytest.mark.parametrize("lean", [False, True])
 def test_chunked_clust2snp(ctx, sub, lean):
+    chunked_clust2snp(ctx, sub, lean)
+
+
+def chunked_clust2snp(ctx, sub, lean):
+    """clust2snp on a chunked shard of CHUNK positions (lean: text / suff from the host's pairSA)"""
     case, want = sub
     case, pad = shifted(case)
     if pad:
