@@ -20,7 +20,7 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 CUFLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-cudart", "static"] + ARCH
 
-CU_SOURCES = ["capi.cu", "cluster.cu", "scan.cu", "merge.cu", "snp.cu", "unpack.cu", "build_egsa.cu"]
+CU_SOURCES = ["ctx.cu", "shard.cu", "build_host.cu", "phase1.cu", "phase2.cu", "pipeline.cu", "cluster.cu", "scan.cu", "merge.cu", "snp.cu", "unpack.cu", "build_egsa.cu"]
 CLI_SOURCES = {"ebwt2clust": ["ebwt2clust_main.cpp"], "clust2snp": ["clust2snp_main.cpp"], "build_gesa": ["build_gesa_main.cpp"]}
 # text post-processors of the .snp format (no GPU work, no library): SURVEY.md 8(f) rank 3
 TEXT_TOOLS = {"filter_snp": ["filter_snp_main.cpp"], "snp2fastq": ["snp2fastq_main.cpp"], "snp_vs_vcf": ["snp_vs_vcf_main.cpp"]}

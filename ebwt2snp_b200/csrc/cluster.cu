@@ -862,8 +862,8 @@ uint64_t flags_words_needed(uint64_t n_local) {
 
 uint64_t emit_num_tiles(uint64_t n_local) { return flags_words_needed(n_local) / EM_TILE_WORDS; }
 
-template <int STAGES>
-static cudaError_t launch_flags_t(const FlagParams& p0, uint64_t rows_alloc32, int sm_count, cudaStream_t stream) {
+cudaError_t launch_flags(const FlagParams& p0, uint64_t rows_alloc32, int sm_count, cudaStream_t stream) {
+    constexpr int STAGES = 3;  // LCP tiles in flight per CTA
     PFN_encodeTiled enc = get_encode_fn();
     if (!enc) return cudaErrorNotSupported;
     FlagParams p = p0;
@@ -896,14 +896,6 @@ static cudaError_t launch_flags_t(const FlagParams& p0, uint64_t rows_alloc32, i
     if (grid > p.num_tiles) grid = p.num_tiles;
     kern<<<dim3(unsigned(grid)), dim3(FL_THREADS), smem, stream>>>(tmap, p);
     return cudaGetLastError();
-}
-
-cudaError_t launch_flags(const FlagParams& p, uint64_t rows_alloc32, int sm_count, cudaStream_t stream, int variant) {
-    switch (variant) {
-        case 1: return launch_flags_t<2>(p, rows_alloc32, sm_count, stream);
-        case 2: return launch_flags_t<4>(p, rows_alloc32, sm_count, stream);
-        default: return launch_flags_t<3>(p, rows_alloc32, sm_count, stream);
-    }
 }
 
 uint64_t emit_desc_words() { return uint64_t(EM_MAX_CHUNKS) * EM_DESC_WORDS; }

@@ -194,7 +194,7 @@ cudaError_t launch_export_records(const ChunkSeg* segs, uint32_t n_chunks, uint6
 uint64_t flags_words_needed(uint64_t n_local);
 uint64_t emit_num_tiles(uint64_t n_local);
 uint64_t emit_desc_words();
-cudaError_t launch_flags(const FlagParams& p, uint64_t rows_alloc32, int sm_count, cudaStream_t stream, int variant);
+cudaError_t launch_flags(const FlagParams& p, uint64_t rows_alloc32, int sm_count, cudaStream_t stream);
 cudaError_t launch_emit(const EmitParams& p, int sm_count, cudaStream_t stream);
 // small helpers: append up to 3 records to the device list / pack the list into 10-byte file records
 cudaError_t launch_put_records(uint64_t* d_start, uint16_t* d_len, uint64_t at, const uint64_t* st, const uint64_t* ln,

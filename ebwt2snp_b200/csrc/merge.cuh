@@ -1,7 +1,7 @@
 // The integer logic between the two phases, written once for host and device: chaining the shards' open-cluster states,
 // the tail + post-EOF phantom rule of cluster_lm (ref:ebwt2clust.cpp:90-135; SURVEY.md 8(a) A3) and the pval loop of
 // statistics() (ref:clust2snp.cpp:889-946).  The C ABI entry points (e2s_cluster_merge, e2s_statistics_finish,
-// e2s_exchange_finish: capi.cu) wrap these on the host; k_merge_stats runs the same code in one thread on the device, so
+// e2s_exchange_finish: phase1.cu, phase2.cu) wrap these on the host; k_merge_stats runs the same code in one thread on the device, so
 // that a resident step never leaves the stream between the scan and phase 2.
 #pragma once
 

@@ -31,10 +31,9 @@ def run_cluster(ctx, lcp, bwt, k, m):
     return s, l, nc
 
 
-@pytest.mark.parametrize("variant", [0, 1, 2])
-def test_cluster_fuzz(ctx, variant, monkeypatch):
-    monkeypatch.setenv("E2S_CLUSTER_VARIANT", str(variant))
-    rng = np.random.default_rng(100 + variant)
+@pytest.mark.parametrize("case", [0, 1, 2])
+def test_cluster_fuzz(ctx, case):
+    rng = np.random.default_rng(100 + case)
     sizes = [2, 3, 4, 5, 17, 255, 256, 257, 4095, 4096, 4097, 8191, 8192, 8193, 12289, 40000, 70001, 300000]
     for it, n in enumerate(sizes * 2):
         k = int(rng.choice([1, 2, 3, 5, 16, 70]))

@@ -9,7 +9,7 @@ each feature lands on a chunk's first, second and later tiles.
 
 (A) the one-pass scan on planted tile boundaries at 1, 2, 3, 7 SMs and the device's own: records, n_clust_out, statistics;
     a segment that overflows in a chunk's later tile (the scan reruns on grown segments).
-(B) the same inputs through K1 + K2 (E2S_SCAN_LEGACY, every stage ring of E2S_CLUSTER_VARIANT), and -k > 127 over LCP values
+(B) the same inputs through K1 + K2 (E2S_SCAN_LEGACY), and -k > 127 over LCP values
     above 127, which takes that path by itself.
 (C) shards cut anywhere and chunked shards at one SM: summaries against helpers.emulate_shard, the assembled .clusters.
 (D) phase 2 on the designed cases of tests/phase2_cases.py at 1 and 3 SMs, the volume case over 183 tiles included.
@@ -251,19 +251,18 @@ def test_segment_overflow_in_later_tile(ctxs, sm):
 # ---------------------------------------------------------------------------------------------------------------------------
 # (B) K1 + K2
 # ---------------------------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("variant", [0, 1, 2])
-def test_k1_k2_tile_boundaries(ctxs, variant, monkeypatch):
-    """E2S_SCAN_LEGACY=1 with K1's stage rings of 3, 2 and 4 (E2S_CLUSTER_VARIANT 0 / 1 / 2) at every SM count"""
+@pytest.mark.parametrize("case", [0, 1, 2])
+def test_k1_k2_tile_boundaries(ctxs, case, monkeypatch):
+    """E2S_SCAN_LEGACY=1 at every SM count, three sets of (k, -m) pairs and planted patterns"""
     monkeypatch.setenv("E2S_SCAN_LEGACY", "1")
-    monkeypatch.setenv("E2S_CLUSTER_VARIANT", str(variant))
     ns = sizes(tiles=(3, 13, 40), deltas=(-1, 2))
     for si, sm in enumerate(SMS):
         ctx = ctxs(sm)
-        kms = km_pairs(si + 3 * variant, len(ns))
+        kms = km_pairs(si + 3 * case, len(ns))
         for i, n in enumerate(ns):
             k, m = kms[i]
-            lcp, bwt = planted(n, k, (i + variant) % 5, seed=5000 + 100 * variant + 10 * si + i, rot=i + variant)
-            check_scan(ctx, lcp, bwt, k, m, (variant, sm, n, k, m))
+            lcp, bwt = planted(n, k, (i + case) % 5, seed=5000 + 100 * case + 10 * si + i, rot=i + case)
+            check_scan(ctx, lcp, bwt, k, m, (case, sm, n, k, m))
 
 
 @pytest.mark.parametrize("sm", SMS, ids=SM_IDS)
