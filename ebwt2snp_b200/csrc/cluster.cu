@@ -258,11 +258,6 @@ struct EmitShared {
 constexpr int NO_POS = 0x7fffffff;
 constexpr uint64_t NO_TILE = ~0ull;
 
-__device__ __forceinline__ uint64_t global_ns() {
-    uint64_t t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
 __device__ __forceinline__ bool has_zero_byte(uint32_t x) { return ((x - 0x01010101u) & ~x & 0x80808080u) != 0; }
 
 __global__ void __launch_bounds__(EM_THREADS, 4) k_cluster_emit(EmitParams p) {
@@ -285,7 +280,6 @@ __global__ void __launch_bounds__(EM_THREADS, 4) k_cluster_emit(EmitParams p) {
     if (tid == 0) s_chunk = atomicAdd(&p.res->ticket, 1ull);
     __syncthreads();
     const uint64_t c = s_chunk, n_chunks = gridDim.x;
-    if (p.dbg && tid == 0) p.dbg[c * 4 + 0] = global_ns();
     const uint64_t tpc = (p.num_tiles + n_chunks - 1) / n_chunks;  // tiles per chunk
     const uint64_t t_lo = c * tpc < p.num_tiles ? c * tpc : p.num_tiles;
     const uint64_t t_hi = t_lo + tpc < p.num_tiles ? t_lo + tpc : p.num_tiles;
@@ -699,7 +693,6 @@ __global__ void __launch_bounds__(EM_THREADS, 4) k_cluster_emit(EmitParams p) {
     }
 
     // ================= exchange =================
-    if (p.dbg && tid == 0) p.dbg[c * 4 + 1] = global_ns();
     if (warp == 0) {
         if (lane == 0) {
             my_desc[CD_FIRST_E] = first_e;
@@ -765,7 +758,6 @@ __global__ void __launch_bounds__(EM_THREADS, 4) k_cluster_emit(EmitParams p) {
     __syncthreads();
 
     // ================= pass 2 =================
-    if (p.dbg && tid == 0) p.dbg[c * 4 + 2] = global_ns();
     {
         uint64_t X = sh.x_in, obase = sh.prefix;
         const uint64_t chunk_end = sh.prefix + sh.red[0], carried_pos = sh.carried_pos;
@@ -781,7 +773,6 @@ __global__ void __launch_bounds__(EM_THREADS, 4) k_cluster_emit(EmitParams p) {
     __syncthreads();
     for (int i = tid; i < E2S_HIST_BINS; i += EM_THREADS)
         if (sh.hist[i]) atomicAdd(&p.res->hist[i], (unsigned long long)sh.hist[i]);
-    if (p.dbg && tid == 0) p.dbg[c * 4 + 3] = global_ns();
     if (c == 0 && tid == 0 && p.tail_lcp) {
         p.res->tail_lcp_nm2 = p.tail_lcp[0];
         p.res->tail_lcp_nm1 = p.tail_lcp[1];

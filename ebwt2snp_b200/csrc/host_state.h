@@ -6,6 +6,7 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <functional>
 #include <initializer_list>
 #include <string>
 #include <vector>
@@ -190,8 +191,8 @@ struct e2s_shard {
     uint8_t* d_packed = nullptr;
     uint64_t packed_cap = 0;
     unsigned long long* d_hist = nullptr;
-    // fused prefilter (pipeline mode): armed by e2s_pipeline_resident with clust2snp's -m before the scan
-    uint32_t pf_arm = 0;             // mcov to use in the next e2s_cluster_run, 0 = plain scan
+    // fused prefilter: clust2snp's -m for the next e2s_cluster_run (e2s_cluster_prefilter), 0 = plain scan
+    uint32_t pf_arm = 0;
     e2s::SurvEntry* d_pf_list = nullptr;
     uint64_t pf_cap = 0;
     uint4* d_planes = nullptr;       // resident base-code bit planes of the BWT (planes.cuh), written by the loads
@@ -261,13 +262,16 @@ int load_lcp_bwt(e2s_shard* s, const void* lcp, int x, const uint8_t* bwt, uint6
 
 // phase1.cu
 void put_rec10(uint8_t* o, uint64_t start, uint64_t len);
-int ensure_records(e2s_shard* s, uint64_t cap);
 int ensure_contiguous(e2s_shard* s);
-int grow_segments(e2s_shard* s);
 SnpArrays shard_arrays(const e2s_shard* s);
 uint64_t analysed_count(const ClusterDev& h, const e2s_cluster_merged& mg, int mcov_out, int max_clust_length);
-int scan_enqueue(e2s_shard* s, uint32_t k, int32_t min_len);
-int cluster_run_impl(e2s_shard* s, uint32_t k, int32_t min_len, e2s_cluster_summary* sum, e2s_comm* cm);
+// The scan of the shard, with the fused prefilter of clust2snp's -m `mcov` (0: none), run until its buffers held everything.
+// Each attempt enqueues the scan, then `behind` (the caller's work that must follow it; may be empty), then the copy of the
+// accumulators to *s->h_pin, and synchronises once.  A full record buffer is grown and the scan rerun; so is a full survivor
+// list when retry_survivors.  cm != NULL: `behind` copied every rank's exchange row to cm->h_recv, and an overflow on any
+// rank reruns the scan on all of them.  At most two resizes.
+int run_scan(e2s_shard* s, uint32_t k, int32_t min_len, uint32_t mcov, bool retry_survivors, const e2s_comm* cm,
+             const std::function<int()>& behind);
 const char* merge_message(int rc);
 int merge_status(int rc);
 

@@ -122,7 +122,6 @@ struct EmitParams {  // K2
     uint32_t pf_mcov;
     SurvEntry* pf_list;             // out: clusters that need the exact test, unordered
     uint64_t pf_cap;
-    uint64_t* dbg;       // optional: 4 globaltimer stamps per chunk (start, pass 1 done, exchange done, end); null = off
     ClusterDev* res;
     const uint32_t* tail_lcp;  // &lcp[n_global-2] when this is the last shard, else null
     const uint8_t* tail_bwt;   // &bwt[n_global-1]

@@ -28,7 +28,7 @@ static bool one_pass_ok(const e2s_shard* s, uint32_t k, int32_t min_len) {
     return s->sealed && s->lcpt_ok && (!s->lcpt_sat || k <= 127u) && min_len <= 33;
 }
 
-int ensure_records(e2s_shard* s, uint64_t cap) {
+static int ensure_records(e2s_shard* s, uint64_t cap) {
     if (cap <= s->rec_cap && s->d_start) return E2S_OK;
     cudaFree(s->d_start);
     cudaFree(s->d_len);
@@ -93,7 +93,7 @@ static void make_summary(const ClusterDev& h, uint64_t n_local, uint64_t global_
 
 // a record segment of the one-pass scan overflowed: grow the segments to the fullest one (the chunks keep counting past their
 // capacity)
-int grow_segments(e2s_shard* s) {
+static int grow_segments(e2s_shard* s) {
     std::vector<ChunkRec> hc(s->n_chunks);
     CU(s->ctx, cudaMemcpy(hc.data(), s->d_chunks, hc.size() * sizeof(ChunkRec), cudaMemcpyDeviceToHost));
     uint64_t mx = 0;
@@ -128,70 +128,73 @@ uint64_t analysed_count(const ClusterDev& h, const e2s_cluster_merged& mg, int m
     return na;
 }
 
-// K1 + K2.  cm == NULL: this shard's accumulators come back with one device-to-host copy.  cm != NULL (one process per
-// GPU): the rows of ALL shards come back instead -- packed on the device, all-gathered by NCCL on the same stream, one
-// copy, one synchronisation -- and are left in cm->h_recv for the caller (e2s_pipeline_sharded).
-// Everything the scan launches, enqueued on the context's stream without a synchronisation: accumulators zeroed, K1 + K2
-// (k_lcp_flags + k_cluster_emit) or the one-pass k_cluster_scan + k_chunk_resolve.  s->last_one_pass says which.
-int scan_enqueue(e2s_shard* s, uint32_t k, int32_t min_len) {
-    e2s_ctx* c = s->ctx;
-    // One pass over the byte LCP (k_cluster_scan) whenever the shard has it and min_len allows the bit-parallel length
-    // test; else the two-kernel path on the 4-byte LCP (k_lcp_flags + k_cluster_emit).  E2S_SCAN_LEGACY=1 forces the latter.
-    const bool one_pass = s->last_one_pass = one_pass_ok(s, k, min_len) && !getenv("E2S_SCAN_LEGACY");
-    const uint64_t num_tiles = emit_num_tiles(s->n_local);
-    if (one_pass) {
-        if (!s->d_chunks) {
-            if (cudaMalloc(reinterpret_cast<void**>(&s->d_chunks), SCAN_MAX_CHUNKS * sizeof(ChunkRec)) != cudaSuccess ||
-                cudaMalloc(reinterpret_cast<void**>(&s->d_segs), SCAN_MAX_CHUNKS * sizeof(ChunkSeg)) != cudaSuccess)
-                return fail(c, E2S_ERR_NOMEM, "chunk tables");
-        }
-        CU(c, scan_plan(s->n_local, c->sm_count, &s->n_chunks, &s->tiles_per_chunk));  // (n_local changes from chunk to chunk of a chunked shard)
-        {
-            const uint64_t want = (s->n_local / 8 + 4096) / s->n_chunks + 64;
-            int rc = ensure_segments(s, want > s->seg_cap ? want : s->seg_cap);
-            if (rc) return rc;
-        }
-    } else {
-        if (!s->d_desc) {
-            if (cudaMalloc(reinterpret_cast<void**>(&s->d_desc), emit_desc_words() * 8) != cudaSuccess)
-                return fail(c, E2S_ERR_NOMEM, "chunk descriptors");
-            s->desc_cap = emit_desc_words();
-        }
-        if (!s->d_flags) {
-            s->flag_words = flags_words_needed(s->n_local);
-            if (cudaMalloc(reinterpret_cast<void**>(&s->d_flags), s->flag_words * 2 * 4) != cudaSuccess)
-                return fail(c, E2S_ERR_NOMEM, "flag masks");
-            // K1 overwrites the words of its tiles; the tail up to K2's tile size stays zero
-            CU(c, cudaMemsetAsync(s->d_flags, 0, s->flag_words * 2 * 4, c->stream));
+// The fused prefilter's survivor list for a scan whose records fill at most `records` slots (mcov == 0: none): what the scan
+// kernels get in *list / *cap.
+static int arm_survivors(e2s_shard* s, uint32_t mcov, uint64_t records, SurvEntry** list, uint64_t* cap) {
+    *list = nullptr;
+    *cap = 0;
+    if (!mcov) return E2S_OK;
+    uint64_t want = records / 16 + 4096;
+    if (const char* dbg = getenv("E2S_PF_CAPACITY")) {  // test hook: a tiny list forces the overflow -> two-phase fallback
+        const uint64_t v = strtoull(dbg, nullptr, 10);
+        if (v) {
+            want = v;
+            if (s->pf_cap > v && !s->pf_want) s->pf_cap = v;  // also shrink the advertised capacity of an existing buffer
         }
     }
-    if (!one_pass && !s->d_start) {
+    if (s->pf_want > want) want = s->pf_want;  // (an overflow of the last attempt asked for more)
+    if (want > s->pf_cap) {
+        cudaFree(s->d_pf_list);
+        s->d_pf_list = nullptr;
+        s->pf_cap = 0;
+        if (cudaMalloc(reinterpret_cast<void**>(&s->d_pf_list), (want + 8) * sizeof(SurvEntry)) != cudaSuccess)
+            return fail(s->ctx, E2S_ERR_NOMEM, "prefilter survivor list");
+        s->pf_cap = want;
+    }
+    *list = s->d_pf_list;
+    *cap = s->pf_cap > 4 ? s->pf_cap - 4 : 0;  // (room for the records k_merge_stats adopts)
+    return E2S_OK;
+}
+
+// K1 + K2 (k_lcp_flags + k_cluster_emit) on the 4-byte LCP, accumulators zeroed first: the records go to d_start / d_len.
+static int enqueue_k1_k2(e2s_shard* s, uint32_t k, int32_t min_len, uint32_t mcov) {
+    e2s_ctx* c = s->ctx;
+    if (!s->d_desc) {
+        if (cudaMalloc(reinterpret_cast<void**>(&s->d_desc), emit_desc_words() * 8) != cudaSuccess)
+            return fail(c, E2S_ERR_NOMEM, "chunk descriptors");
+        s->desc_cap = emit_desc_words();
+    }
+    if (!s->d_flags) {
+        s->flag_words = flags_words_needed(s->n_local);
+        if (cudaMalloc(reinterpret_cast<void**>(&s->d_flags), s->flag_words * 2 * 4) != cudaSuccess)
+            return fail(c, E2S_ERR_NOMEM, "flag masks");
+        // K1 overwrites the words of its tiles; the tail up to K2's tile size stays zero
+        CU(c, cudaMemsetAsync(s->d_flags, 0, s->flag_words * 2 * 4, c->stream));
+    }
+    if (!s->d_start) {
         int rc = ensure_records(s, s->n_local / 8 + 4096);
         if (rc) return rc;
     }
-    // K1: LCP -> START/END masks (two-kernel path only)
-    if (!one_pass) {
-        FlagParams fp;
-        fp.lcp = s->lcp;
-        fp.n_local = s->n_local;
-        fp.global_off = s->global_off;
-        fp.n_global = s->n_global;
-        fp.k = k;
-        fp.num_tiles = 0;
-        fp.s_words = s->d_flags;
-        fp.e_words = s->d_flags + s->flag_words;
-        c->timer.begin(E2S_KERNEL_FLAGS, c->stream);
-        cudaError_t le = launch_flags(fp, s->alloc_r / 32, c->sm_count, c->stream);
-        c->timer.end(c->stream);
-        CU(c, le);
-        ++c->launches;
-    }
+    FlagParams fp;
+    fp.lcp = s->lcp;
+    fp.n_local = s->n_local;
+    fp.global_off = s->global_off;
+    fp.n_global = s->n_global;
+    fp.k = k;
+    fp.num_tiles = 0;
+    fp.s_words = s->d_flags;
+    fp.e_words = s->d_flags + s->flag_words;
+    c->timer.begin(E2S_KERNEL_FLAGS, c->stream);
+    cudaError_t le = launch_flags(fp, s->alloc_r / 32, c->sm_count, c->stream);
+    c->timer.end(c->stream);
+    CU(c, le);
+    ++c->launches;
     CU(c, cudaMemsetAsync(s->d_res, 0, sizeof(ClusterDev), c->stream));
-    if (!one_pass) CU(c, cudaMemsetAsync(s->d_desc, 0, s->desc_cap * 8, c->stream));
+    CU(c, cudaMemsetAsync(s->d_desc, 0, s->desc_cap * 8, c->stream));
     EmitParams p;
     p.s_words = s->d_flags;
     p.e_words = s->d_flags + s->flag_words;
-    p.num_tiles = num_tiles;
+    p.num_tiles = emit_num_tiles(s->n_local);
     p.global_off = s->global_off;
     p.n_global = s->n_global;
     p.min_len = min_len;
@@ -200,134 +203,112 @@ int scan_enqueue(e2s_shard* s, uint32_t k, int32_t min_len) {
     p.cap = s->rec_cap - 4;  // room for adopted records
     p.desc = s->d_desc;
     p.planes = s->d_planes;
-    p.pf_mcov = (s->pf_arm && s->sealed) ? s->pf_arm : 0;
-    p.pf_list = nullptr;
-    p.pf_cap = 0;
-    if (p.pf_mcov) {
-        uint64_t want = (one_pass ? s->seg_cap * s->n_chunks : s->rec_cap) / 16 + 4096;
-        if (const char* dbg = getenv("E2S_PF_CAPACITY")) {  // test hook: a tiny list forces the overflow -> two-phase fallback
-            const uint64_t v = strtoull(dbg, nullptr, 10);
-            if (v) {
-                want = v;
-                if (s->pf_cap > v && !s->pf_want) s->pf_cap = v;  // also shrink the advertised capacity of an existing buffer
-            }
-        }
-        if (s->pf_want > want) want = s->pf_want;  // (an overflow of the last attempt asked for more)
-        if (want > s->pf_cap) {
-            cudaFree(s->d_pf_list);
-            s->d_pf_list = nullptr;
-            s->pf_cap = 0;
-            if (cudaMalloc(reinterpret_cast<void**>(&s->d_pf_list), (want + 8) * sizeof(SurvEntry)) != cudaSuccess)
-                return fail(c, E2S_ERR_NOMEM, "prefilter survivor list");
-            s->pf_cap = want;
-        }
-        p.pf_list = s->d_pf_list;
-        p.pf_cap = s->pf_cap > 4 ? s->pf_cap - 4 : 0;  // (room for the records k_merge_stats adopts)
-    }
-    p.dbg = nullptr;
+    p.pf_mcov = mcov;
+    if (int rc = arm_survivors(s, mcov, s->rec_cap, &p.pf_list, &p.pf_cap)) return rc;
     p.res = s->d_res;
     const bool is_last = s->global_off + s->n_local == s->n_global;
     p.tail_lcp = is_last ? s->lcp + s->n_local - 2 : nullptr;
     p.tail_bwt = is_last ? s->bwt + s->n_local - 1 : nullptr;
-    if (one_pass) {
-        CU(c, cudaMemsetAsync(s->d_chunks, 0, size_t(s->n_chunks) * sizeof(ChunkRec), c->stream));
-        Scan8Params sp;
-        sp.lcpt = s->lcpt;
-        sp.planes = s->d_planes;
-        sp.n_local = s->n_local;
-        sp.global_off = s->global_off;
-        sp.n_global = s->n_global;
-        sp.k = k;
-        sp.min_len = min_len;
-        sp.num_tiles = 0;
-        sp.n_chunks = s->n_chunks;
-        sp.tiles_per_chunk = s->tiles_per_chunk;
-        sp.seg_start = s->d_seg_start;
-        sp.seg_len = s->d_seg_len;
-        sp.seg_cap = s->seg_cap;
-        sp.chunks = s->d_chunks;
-        sp.pf_mcov = p.pf_mcov;
-        sp.pf_list = p.pf_list;
-        sp.pf_cap = p.pf_cap;
-        sp.res = s->d_res;
-        sp.tail_lcp = p.tail_lcp;
-        sp.tail_bwt = p.tail_bwt;
-        c->timer.begin(E2S_KERNEL_SCAN1, c->stream);
-        cudaError_t le = launch_scan(sp, s->alloc_r, c->stream);
-        c->timer.end(c->stream);
-        CU(c, le);
-        ResolveParams rp;
-        rp.chunks = s->d_chunks;
-        rp.segs = s->d_segs;
-        rp.n_chunks = s->n_chunks;
-        rp.min_len = min_len;
-        rp.global_off = s->global_off;
-        rp.n_global = s->n_global;
-        rp.init_state = s->chunked ? s->carry_state : (s->global_off == 0 ? 0 : 1);
-        rp.planes = s->d_planes;
-        rp.pf_mcov = p.pf_mcov;
-        rp.pf_list = p.pf_list;
-        rp.pf_cap = p.pf_cap;
-        rp.res = s->d_res;
-        c->timer.begin(E2S_KERNEL_RESOLVE, c->stream);
-        cudaError_t re = launch_chunk_resolve(rp, c->stream);
-        c->timer.end(c->stream);
-        CU(c, re);
-        ++c->launches;
-    } else {
-        c->timer.begin(E2S_KERNEL_EMIT, c->stream);
-        cudaError_t le = launch_emit(p, c->sm_count, c->stream);
-        c->timer.end(c->stream);
-        CU(c, le);
-    }
+    c->timer.begin(E2S_KERNEL_EMIT, c->stream);
+    le = launch_emit(p, c->sm_count, c->stream);
+    c->timer.end(c->stream);
+    CU(c, le);
     ++c->launches;
     return E2S_OK;
 }
 
-int cluster_run_impl(e2s_shard* s, uint32_t k, int32_t min_len, e2s_cluster_summary* sum, e2s_comm* cm) {
-    if (!s || !sum) return fail(s ? s->ctx : nullptr, E2S_ERR_ARG, "e2s_cluster_run: NULL argument");
+// k_cluster_scan + k_chunk_resolve, one pass over the bit-sliced LCP, accumulators zeroed first: the records go to the
+// per-chunk segments.  A chunked shard starts from the open-cluster state its earlier chunks left.
+static int enqueue_one_pass(e2s_shard* s, uint32_t k, int32_t min_len, uint32_t mcov) {
     e2s_ctx* c = s->ctx;
-    if (s->chunked) return fail(c, E2S_ERR_STATE, "chunked shard: use e2s_chunk_begin / e2s_chunk_scan / e2s_chunked_finish");
-    if (k == 0) return fail(c, E2S_ERR_ARG, "k must be >= 1 (the CLI maps 0 to the default 16)");
-    CU(c, cudaSetDevice(c->device));
+    if (!s->d_chunks) {
+        if (cudaMalloc(reinterpret_cast<void**>(&s->d_chunks), SCAN_MAX_CHUNKS * sizeof(ChunkRec)) != cudaSuccess ||
+            cudaMalloc(reinterpret_cast<void**>(&s->d_segs), SCAN_MAX_CHUNKS * sizeof(ChunkSeg)) != cudaSuccess)
+            return fail(c, E2S_ERR_NOMEM, "chunk tables");
+    }
+    CU(c, scan_plan(s->n_local, c->sm_count, &s->n_chunks, &s->tiles_per_chunk));  // (n_local changes from chunk to chunk of a chunked shard)
+    {
+        const uint64_t want = (s->n_local / 8 + 4096) / s->n_chunks + 64;
+        int rc = ensure_segments(s, want > s->seg_cap ? want : s->seg_cap);
+        if (rc) return rc;
+    }
+    CU(c, cudaMemsetAsync(s->d_res, 0, sizeof(ClusterDev), c->stream));
+    Scan8Params sp;
+    sp.lcpt = s->lcpt;
+    sp.planes = s->d_planes;
+    sp.n_local = s->n_local;
+    sp.global_off = s->global_off;
+    sp.n_global = s->n_global;
+    sp.k = k;
+    sp.min_len = min_len;
+    sp.num_tiles = 0;
+    sp.n_chunks = s->n_chunks;
+    sp.tiles_per_chunk = s->tiles_per_chunk;
+    sp.seg_start = s->d_seg_start;
+    sp.seg_len = s->d_seg_len;
+    sp.seg_cap = s->seg_cap;
+    sp.chunks = s->d_chunks;
+    sp.pf_mcov = mcov;
+    if (int rc = arm_survivors(s, mcov, s->seg_cap * s->n_chunks, &sp.pf_list, &sp.pf_cap)) return rc;
+    sp.res = s->d_res;
+    const bool is_last = s->global_off + s->n_local == s->n_global;
+    sp.tail_lcp = is_last ? s->lcp + s->n_local - 2 : nullptr;
+    sp.tail_bwt = is_last ? s->bwt + s->n_local - 1 : nullptr;
+    CU(c, cudaMemsetAsync(s->d_chunks, 0, size_t(s->n_chunks) * sizeof(ChunkRec), c->stream));
+    c->timer.begin(E2S_KERNEL_SCAN1, c->stream);
+    cudaError_t le = launch_scan(sp, s->alloc_r, c->stream);
+    c->timer.end(c->stream);
+    CU(c, le);
+    ++c->launches;
+    ResolveParams rp;
+    rp.chunks = s->d_chunks;
+    rp.segs = s->d_segs;
+    rp.n_chunks = s->n_chunks;
+    rp.min_len = min_len;
+    rp.global_off = s->global_off;
+    rp.n_global = s->n_global;
+    rp.init_state = s->chunked ? s->carry_state : (s->global_off == 0 ? 0 : 1);
+    rp.planes = s->d_planes;
+    rp.pf_mcov = mcov;
+    rp.pf_list = sp.pf_list;
+    rp.pf_cap = sp.pf_cap;
+    rp.res = s->d_res;
+    c->timer.begin(E2S_KERNEL_RESOLVE, c->stream);
+    le = launch_chunk_resolve(rp, c->stream);
+    c->timer.end(c->stream);
+    CU(c, le);
+    ++c->launches;
+    return E2S_OK;
+}
+
+int run_scan(e2s_shard* s, uint32_t k, int32_t min_len, uint32_t mcov, bool retry_survivors, const e2s_comm* cm,
+             const std::function<int()>& behind) {
+    e2s_ctx* c = s->ctx;
+    // One pass over the byte LCP (k_cluster_scan) whenever the shard has it and min_len allows the bit-parallel length test;
+    // else the two-kernel path on the 4-byte LCP.  E2S_SCAN_LEGACY=1 forces the latter on a resident shard: a chunked shard
+    // has the one-pass scan only.
+    const bool one_pass = s->last_one_pass = one_pass_ok(s, k, min_len) && (s->chunked || !getenv("E2S_SCAN_LEGACY"));
     if (!s->h_pin) CU(c, cudaHostAlloc(reinterpret_cast<void**>(&s->h_pin), sizeof(ClusterDev), cudaHostAllocDefault));
     ClusterDev& h = *s->h_pin;
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        int erc = scan_enqueue(s, k, min_len);
-        if (erc) return erc;
-        const bool one_pass = s->last_one_pass;
-        bool any_overflow = false;
-        uint64_t max_written = 0;
-        if (cm) {
-            CU(c, launch_pack_exchange(s->d_res, s->n_local, s->global_off, uint64_t(s->lay_x), cm->d_send, c->stream));
-            ++c->launches;
-            if (int rc = all_gather_rows(c, cm)) return rc;
-            CU(c, cudaMemcpyAsync(cm->h_recv, cm->d_recv, size_t(cm->world) * XR_WORDS * 8, cudaMemcpyDeviceToHost, c->stream));
-            CU(c, cudaStreamSynchronize(c->stream));
-            memcpy(&h, cm->h_recv + size_t(cm->rank) * XR_WORDS, sizeof h);
-            for (int g = 0; g < cm->world; ++g) {  // every rank sees every overflow flag: all of them repeat the round together
-                const ClusterDev& hg = *reinterpret_cast<const ClusterDev*>(cm->h_recv + size_t(g) * XR_WORDS);
-                any_overflow |= (hg.overflow & 1) != 0;  // (bit 1 = survivor list: not fatal here, find_events then runs its own prefilter)
-                if (hg.n_written > max_written) max_written = hg.n_written;
-            }
-        } else {
-            CU(c, cudaMemcpyAsync(&h, s->d_res, sizeof h, cudaMemcpyDeviceToHost, c->stream));
-            CU(c, cudaStreamSynchronize(c->stream));
-            any_overflow = (h.overflow & 1) != 0;
-            max_written = h.n_written;
-        }
-        if (!any_overflow) break;
-        if (attempt == 1) return fail(c, E2S_ERR_STATE, "record buffer overflow after resize");
-        if ((h.overflow & 1) || !cm) {
-            const int rc = one_pass ? grow_segments(s) : ensure_records(s, (cm ? h.n_written : max_written) + 4096);
-            if (rc) return rc;
-        }
+    for (int attempt = 0;; ++attempt) {
+        int rc = one_pass ? enqueue_one_pass(s, k, min_len, mcov) : enqueue_k1_k2(s, k, min_len, mcov);
+        if (!rc && behind) rc = behind();
+        if (rc) return rc;
+        CU(c, cudaMemcpyAsync(&h, s->d_res, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaStreamSynchronize(c->stream));
+        // bit 0: a record buffer was full; bit 1 (or more entries than the list holds once k_merge_stats appended the
+        // adopted records): the survivor list was
+        const bool records_full = h.overflow & 1;
+        const bool survivors_full = retry_survivors && ((h.overflow & 2) || h.n_pf > s->pf_cap);
+        bool again = records_full || survivors_full;
+        if (cm)  // every rank sees every rank's row: all of them repeat the round together
+            for (int g = 0; g < cm->world; ++g)
+                again |= (reinterpret_cast<const ClusterDev*>(cm->h_recv + size_t(g) * XR_WORDS)->overflow & (retry_survivors ? 3 : 1)) != 0;
+        if (!again) return E2S_OK;
+        if (attempt == 2) return fail(c, E2S_ERR_STATE, "record / survivor buffers still too small after two resizes");
+        if (records_full && (rc = one_pass ? grow_segments(s) : ensure_records(s, h.n_written + 4096))) return rc;
+        if (survivors_full) s->pf_want = h.n_pf + h.n_pf / 8 + 4096;
     }
-    make_summary(h, s->n_local, s->global_off, s->n_global, k, min_len, uint64_t(s->lay_x), sum);
-    const uint32_t mcov = (s->pf_arm && s->sealed) ? s->pf_arm : 0;
-    s->rl.scanned(h, mcov, !s->last_one_pass);
-    s->rl.survivors(h.n_pf, mcov != 0 && !(h.overflow & 2) && h.n_pf + 4 <= s->pf_cap, false);
-    return E2S_OK;
 }
 
 // capacity of the payload / survivor list of a chunked shard (grown between chunks, contents kept)
@@ -497,28 +478,8 @@ int e2s_chunk_scan(e2s_shard* s, uint32_t k, int32_t min_len, int mcov_out, uint
         return fail(c, E2S_ERR_UNSUPPORTED,
                     "chunked shards need the one-pass scan: -m <= 33, and -k <= 127 when an LCP value exceeds 127; "
                     "use a resident shard for this input");
-    if (!s->h_pin) CU(c, cudaHostAlloc(reinterpret_cast<void**>(&s->h_pin), sizeof(ClusterDev), cudaHostAllocDefault));
-    ClusterDev& h = *s->h_pin;
-    const uint32_t arm_before = s->pf_arm;
-    s->pf_arm = uint32_t(mcov_out);
-    for (int attempt = 0;; ++attempt) {
-        if ((rc = scan_enqueue(s, k, min_len))) break;
-        cudaError_t e = cudaMemcpyAsync(&h, s->d_res, sizeof h, cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        if (e != cudaSuccess) {
-            rc = cuda_fail(c, e, "chunk scan");
-            break;
-        }
-        if (!h.overflow) break;
-        if (attempt >= 2) {
-            rc = fail(c, E2S_ERR_STATE, "record / survivor buffers still too small after two resizes");
-            break;
-        }
-        if ((h.overflow & 1) && (rc = grow_segments(s))) break;
-        if (h.overflow & 2) s->pf_want = h.n_pf + h.n_pf / 8 + 4096;
-    }
-    s->pf_arm = arm_before;
-    if (rc) return rc;
+    if ((rc = run_scan(s, k, min_len, uint32_t(mcov_out), true, nullptr, nullptr))) return rc;
+    const ClusterDev& h = *s->h_pin;
     if (mcov_out && h.n_pf && (rc = capture_survivors(s, h.n_pf))) return rc;
     // the range's accumulators; the state the next chunk starts from
     ClusterDev& a = s->acc;
@@ -539,7 +500,7 @@ int e2s_chunk_scan(e2s_shard* s, uint32_t k, int32_t min_len, int mcov_out, uint
     a.ticket++;  // chunks scanned
     if (a.any_event) s->carry_state = h.open_start ? h.open_start - 1 + 2 : 0;
     s->chunk_open = false;
-    s->rl.scanned(h, uint32_t(mcov_out), false);
+    s->rl.scanned(h, uint32_t(mcov_out), !s->last_one_pass);
     if (n_records) *n_records = h.n_written;
     return E2S_OK;
 }
@@ -625,7 +586,20 @@ int e2s_chunked_finish(e2s_shard* s, uint32_t k, int32_t min_len, e2s_cluster_su
 }
 
 int e2s_cluster_run(e2s_shard* s, uint32_t k, int32_t min_len, e2s_cluster_summary* sum) {
-    return cluster_run_impl(s, k, min_len, sum, nullptr);
+    if (!s || !sum) return fail(s ? s->ctx : nullptr, E2S_ERR_ARG, "e2s_cluster_run: NULL argument");
+    e2s_ctx* c = s->ctx;
+    if (s->chunked) return fail(c, E2S_ERR_STATE, "chunked shard: use e2s_chunk_begin / e2s_chunk_scan / e2s_chunked_finish");
+    if (k == 0) return fail(c, E2S_ERR_ARG, "k must be >= 1 (the CLI maps 0 to the default 16)");
+    CU(c, cudaSetDevice(c->device));
+    // a full survivor list is not retried: find_events then runs its own prefilter (K3a)
+    const uint32_t mcov = s->sealed ? s->pf_arm : 0;
+    int rc = run_scan(s, k, min_len, mcov, false, nullptr, nullptr);
+    if (rc) return rc;
+    const ClusterDev& h = *s->h_pin;
+    make_summary(h, s->n_local, s->global_off, s->n_global, k, min_len, uint64_t(s->lay_x), sum);
+    s->rl.scanned(h, mcov, !s->last_one_pass);
+    s->rl.survivors(h.n_pf, mcov != 0 && !(h.overflow & 2) && h.n_pf + 4 <= s->pf_cap, false);
+    return E2S_OK;
 }
 
 int e2s_cluster_merge(const e2s_cluster_summary* all, int n_shards, int my, e2s_cluster_merged* out) {

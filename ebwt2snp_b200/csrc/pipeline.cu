@@ -11,7 +11,7 @@ using namespace e2s;
 namespace e2s {
 
 // may both phases run in one pass, the scan running clust2snp's BWT prefilter?  Needs a valid -m; E2S_NO_FUSED_PREFILTER
-// keeps the two phases apart as the CLIs have to.
+// keeps the two phases apart as the CLIs have to (e2s_pipeline_sharded always runs them in one pass).
 static bool fused_prefilter(const e2s_snp_params* p) {
     return !(getenv("E2S_NO_FUSED_PREFILTER") || p->mcov_out < 1 || 2 * p->mcov_out > E2S_MAX_C_LEN);
 }
@@ -36,35 +36,27 @@ static int pipeline_step(e2s_shard* s, e2s_comm* cm, uint32_t k, int32_t min_len
         CU(c, cudaHostAlloc(reinterpret_cast<void**>(&s->h_mout), sizeof(MergeOut), cudaHostAllocDefault));
         CU(c, cudaMalloc(reinterpret_cast<void**>(&s->d_row), XR_WORDS * 8));
     }
-    if (!s->h_pin) CU(c, cudaHostAlloc(reinterpret_cast<void**>(&s->h_pin), sizeof(ClusterDev), cudaHostAllocDefault));
-    ClusterDev& h = *s->h_pin;
     MergeOut& mo = *s->h_mout;
-    const uint32_t arm_before = s->pf_arm;
-    s->pf_arm = uint32_t(p->mcov_out);
     s->rl.events_present(false);
     s->events.clear();
     const SnpArrays a = shard_arrays(s);  // (phase 2 starts from the survivor list: the record list is not walked)
     const char* err = "";
-    int rc = E2S_OK;
-    for (int attempt = 0;; ++attempt) {
-        if ((rc = scan_enqueue(s, k, min_len))) break;
+    e2s_snp_counts counts;
+    // behind the scan on the stream: the exchange row (all-gathered when there is a communicator), k_merge_stats, phase 2 from the
+    // survivor list -- its length and max_clust_length read on the device -- and the copies of the results
+    auto merge_and_phase2 = [&]() -> int {
         uint64_t* send = cm ? cm->d_send : s->d_row;
-        const uint64_t* rows = send;
         c->timer.begin(E2S_KERNEL_MERGE, c->stream);
-        if ((rc = launch_pack_exchange(s->d_res, s->n_local, s->global_off, uint64_t(s->lay_x), send, c->stream) == cudaSuccess ? 0 : 1)) {
+        if (launch_pack_exchange(s->d_res, s->n_local, s->global_off, uint64_t(s->lay_x), send, c->stream) != cudaSuccess) {
             c->timer.end(c->stream);
-            rc = fail(c, E2S_ERR_CUDA, "k_pack_exchange");
-            break;
+            return fail(c, E2S_ERR_CUDA, "k_pack_exchange");
         }
-        if (cm) {
-            if ((rc = all_gather_rows(c, cm))) {
-                c->timer.end(c->stream);
-                break;
-            }
-            rows = cm->d_recv;
+        if (int rc = cm ? all_gather_rows(c, cm) : E2S_OK) {
+            c->timer.end(c->stream);
+            return rc;
         }
         MergeParams mp;
-        mp.rows = reinterpret_cast<const unsigned long long*>(rows);
+        mp.rows = reinterpret_cast<const unsigned long long*>(cm ? cm->d_recv : send);
         mp.world = world;
         mp.my = my;
         mp.n_global = s->n_global;
@@ -81,16 +73,10 @@ static int pipeline_step(e2s_shard* s, e2s_comm* cm, uint32_t k, int32_t min_len
         cudaError_t e = launch_merge_stats(mp, c->stream);
         c->timer.end(c->stream);
         c->launches += 2;
-        // phase 2 from the survivor list, its length and max_clust_length read on the device
-        e2s_snp_counts counts;
         if (e == cudaSuccess) {
             where = "phase 2 kernels";
             e = snp_run(s->work, a, *p, E2S_MAX_C_LEN, c->d_bases, c->d_off, c->n_reads, c->sm_count, c->stream, &counts, &c->launches, &err,
                         &c->timer, s->d_pf_list, s->pf_cap, &s->d_res->n_pf, &s->d_mout->total.max_clust_length, false);
-        }
-        if (e == cudaSuccess) {
-            where = "copy of the scan accumulators";
-            e = cudaMemcpyAsync(&h, s->d_res, sizeof h, cudaMemcpyDeviceToHost, c->stream);
         }
         if (e == cudaSuccess) {
             where = "copy of the merge result";
@@ -100,52 +86,24 @@ static int pipeline_step(e2s_shard* s, e2s_comm* cm, uint32_t k, int32_t min_len
             where = "copy of the exchange rows";
             e = cudaMemcpyAsync(cm->h_recv, cm->d_recv, size_t(world) * XR_WORDS * 8, cudaMemcpyDeviceToHost, c->stream);
         }
-        if (e == cudaSuccess) {
-            where = "synchronisation of the step";
-            e = cudaStreamSynchronize(c->stream);  // the only synchronisation of the step
-        }
-        if (e != cudaSuccess) {
-            rc = cuda_fail(c, e, err && err[0] ? err : where);
-            break;
-        }
-        // a full record segment (on any rank: every rank sees every row) or a full survivor list: more room, once more
-        bool any_overflow = h.overflow != 0;
-        if (cm)
-            for (int g = 0; g < world; ++g) any_overflow |= reinterpret_cast<const ClusterDev*>(cm->h_recv + size_t(g) * XR_WORDS)->overflow != 0;
-        const bool pf_overflow = h.n_pf > s->pf_cap || (h.overflow & 2);
-        if (any_overflow || pf_overflow) {
-            if (attempt >= 2) {
-                rc = fail(c, E2S_ERR_STATE, "record / survivor buffers still too small after two resizes");
-                break;
-            }
-            if ((h.overflow & 1) && (rc = s->last_one_pass ? grow_segments(s) : ensure_records(s, h.n_written + 4096))) break;
-            if (pf_overflow) s->pf_want = h.n_pf + h.n_pf / 8 + 4096;
-            continue;
-        }
-        if (mo.status != MERGE_OK) {
-            rc = fail(c, merge_status(mo.status), mo.status == MERGE_EMPTY ? "no clusters (the reference divides by zero here)" : merge_message(mo.status));
-            break;
-        }
-        cudaError_t src = cudaSuccess;
-        if (!snp_collect(s->work, &counts, &err, &src)) {
-            if (src == cudaSuccess)  // a capacity guess of phase 2 was too small: the lists it starts from are still on the device
-                src = snp_run(s->work, a, *p, mo.total.max_clust_length, c->d_bases, c->d_off, c->n_reads, c->sm_count, c->stream, &counts,
-                              &c->launches, &err, &c->timer, s->d_pf_list, s->pf_cap, &s->d_res->n_pf, nullptr, true);
-            if (src == cudaErrorInvalidValue && err && strstr(err, "outside the staged reads")) {
-                rc = fail(c, E2S_ERR_UNSUPPORTED, err);
-                break;
-            }
-            if (src != cudaSuccess) {
-                rc = cuda_fail(c, src, err);
-                break;
-            }
-        }
-        counts.n_analysed = analysed_count(h, mo.mine, p->mcov_out, mo.total.max_clust_length);
-        *cnt_out = counts;
-        break;
-    }
-    s->pf_arm = arm_before;
+        return e == cudaSuccess ? E2S_OK : cuda_fail(c, e, err && err[0] ? err : where);
+    };
+    // the scan's own synchronisation is the only one of the step
+    int rc = run_scan(s, k, min_len, uint32_t(p->mcov_out), true, cm, merge_and_phase2);
     if (rc) return rc;
+    const ClusterDev& h = *s->h_pin;
+    if (mo.status != MERGE_OK)
+        return fail(c, merge_status(mo.status), mo.status == MERGE_EMPTY ? "no clusters (the reference divides by zero here)" : merge_message(mo.status));
+    cudaError_t src = cudaSuccess;
+    if (!snp_collect(s->work, &counts, &err, &src)) {
+        if (src == cudaSuccess)  // a capacity guess of phase 2 was too small: the lists it starts from are still on the device
+            src = snp_run(s->work, a, *p, mo.total.max_clust_length, c->d_bases, c->d_off, c->n_reads, c->sm_count, c->stream, &counts,
+                          &c->launches, &err, &c->timer, s->d_pf_list, s->pf_cap, &s->d_res->n_pf, nullptr, true);
+        if (src == cudaErrorInvalidValue && err && strstr(err, "outside the staged reads")) return fail(c, E2S_ERR_UNSUPPORTED, err);
+        if (src != cudaSuccess) return cuda_fail(c, src, err);
+    }
+    counts.n_analysed = analysed_count(h, mo.mine, p->mcov_out, mo.total.max_clust_length);
+    *cnt_out = counts;
     // the shard's state, as e2s_cluster_run + e2s_cluster_finalize + e2s_find_events leave it
     s->rl.scanned(h, uint32_t(p->mcov_out), !s->last_one_pass);
     s->rl.survivors(h.n_pf, true, true);
@@ -358,25 +316,13 @@ int e2s_pipeline_resident(e2s_shard* s, uint32_t k, int32_t min_len, const e2s_s
     return phase2_to_caller(s, p, nullptr, 0, res);
 }
 
-// The sharded step in one call: K1, K2, ONE all-gather of the scan accumulators (summary + own length histogram) on
-// the stream, host merge of all shards + statistics, K3/K4 on local data.  Two host synchronisations, like the
-// single-shard e2s_pipeline_resident.
+// The sharded step in one call: the resident step of one shard (pipeline_step), the shards' exchange rows all-gathered by
+// NCCL on the stream and merged on the device by every rank.  One host synchronisation.
 int e2s_pipeline_sharded(e2s_shard* s, e2s_comm* cm, uint32_t k, int32_t min_len, const e2s_snp_params* p, e2s_cluster_merged* mg,
                          e2s_stats* st, e2s_snp_counts* cnt) {
     if (!s || !cm || !p || !mg || !st || !cnt) return fail(s ? s->ctx : nullptr, E2S_ERR_ARG, "e2s_pipeline_sharded: NULL argument");
-    e2s_ctx* c = s->ctx;
-    if (cm->ctx != c) return fail(c, E2S_ERR_ARG, "e2s_pipeline_sharded: communicator belongs to another context");
-    // the exchange between the phases stays on the device: ncclAllGather of the rows, k_merge_stats on every rank (pipeline_step)
-    if (fused_prefilter(p)) return pipeline_step(s, cm, k, min_len, p, mg, st, cnt);
-    e2s_cluster_summary own_sum;
-    int rc = cluster_run_impl(s, k, min_len, &own_sum, cm);
-    if (rc) return rc;
-    if ((rc = e2s_exchange_rows_finish(cm->h_recv, cm->world, cm->rank, s->n_global, k, min_len, p->mcov_out, p->pval, mg, st))) {
-        c->err = g_err;
-        return rc;
-    }
-    if ((rc = e2s_cluster_finalize(s, mg))) return rc;
-    return e2s_find_events(s, p, st->max_clust_length, cnt);
+    if (cm->ctx != s->ctx) return fail(s->ctx, E2S_ERR_ARG, "e2s_pipeline_sharded: communicator belongs to another context");
+    return pipeline_step(s, cm, k, min_len, p, mg, st, cnt);
 }
 
 // ebwt2clust + clust2snp from host buffers.  The records stream through a CHUNKED shard (a chunk is a shard in time): the

@@ -372,9 +372,10 @@ int e2s_pipeline_resident(e2s_shard *sh, uint32_t k, int32_t min_len, const e2s_
 /* One process per GPU (SURVEY.md 8(e)): the exchange between the phases inside the library.  A communicator wraps an
  * NCCL communicator created from a 128-byte unique id (made on one rank with e2s_comm_unique_id and handed to the others
  * by whatever launched the processes: torch.distributed in bench.py).  NCCL is bound at run time (libnccl.so.2).
- * e2s_pipeline_sharded = e2s_pipeline_resident for a shard of a sharded eBWT: K1 + K2, ONE ncclAllGather of every shard's
- * scan accumulators on the context's stream, e2s_exchange_finish on the host (identical on all ranks), K3/K4 on local
- * data.  Collective: every rank of the communicator must call it. */
+ * e2s_pipeline_sharded = e2s_pipeline_resident for a shard of a sharded eBWT: the scan with clust2snp's BWT prefilter, ONE
+ * ncclAllGather of every shard's scan accumulators on the context's stream, the merge and statistics() of all shards on the
+ * device (identical on all ranks), K3x/K3b/K4 on the shard's survivors, one host synchronisation.  Needs valid clust2snp
+ * parameters (E2S_ERR_UNSUPPORTED otherwise).  Collective: every rank of the communicator must call it. */
 /* Host-only (no CUDA), exposed for tests and for callers that move the rows themselves: e2s_exchange_row_words() u64 words per
  * shard = the scan's device accumulators (ClusterDev: counters, open-cluster state, tail values, length histogram of the
  * shard's own records) followed by n_local, global_off, lcp_bytes, 0.  e2s_exchange_rows_finish turns the gathered rows

@@ -12,9 +12,10 @@ n_analysed / n_candidates / n_events and the .snp text.
     verdict (an LCP value above 127) follows the data.
 (D) e2s_pipeline_host / e2s_pipeline_host_soa in sequence on one context (its cached shard); a fresh context whose first
     streamed call is the lean one, then .gesa loads.
-(E) one chunked shard over several passes with e2s_chunked_reset: scan passes, an abandoned pass, a clust2snp pass, lean.
-(F) a one-rank NCCL communicator: e2s_pipeline_sharded and e2s_chunked_exchange repeated; e2s_pipeline_host_sharded under
-    two chunk sizes.
+(E) one chunked shard over several passes with e2s_chunked_reset: scan passes, an abandoned pass, a clust2snp pass, lean;
+    E2S_SCAN_LEGACY, which a chunked shard does not follow.
+(F) a one-rank NCCL communicator: e2s_pipeline_sharded (with and without E2S_NO_FUSED_PREFILTER, which it ignores) and
+    e2s_chunked_exchange repeated; e2s_pipeline_host_sharded under two chunk sizes.
 (G) reads restaged between steps: bigger, smaller, with non-ACGT bytes, ragged.
 """
 import os
@@ -537,9 +538,10 @@ def load_chunk(sh, d, clo, cn, lean):
         sh.load_soa(d.lcp[a:b], d.text[a:b], d.suff[a:b], d.bwt[a:b], first=a)
 
 
-def scan_pass(sh, d, k=16, m=2, mcov=5, lean=False, stop_after=None):
+def scan_pass(sh, d, k=16, m=2, mcov=5, lean=False, stop_after=None, after_scan=None):
     """chunk_begin / load / chunk_scan over the range, the records fetched chunk by chunk; then finish -> merge -> finalize ->
-    statistics -> find_events, all compared with the oracle.  stop_after: abandon the pass after that many chunks"""
+    statistics -> find_events, all compared with the oracle.  stop_after: abandon the pass after that many chunks; after_scan:
+    called after each chunk's scan"""
     w = want(d, k, m, mcov, xyz=(1, 4, 1) if lean else (4, 4, 4), bcr=lean)
     p = params(d, mcov)
     keep = None
@@ -553,6 +555,8 @@ def scan_pass(sh, d, k=16, m=2, mcov=5, lean=False, stop_after=None):
         sh.chunk_begin(clo, cn)
         load_chunk(sh, d, clo, cn, lean)
         m_ = sh.chunk_scan(k, m, mcov)
+        if after_scan:
+            after_scan()
         recs.append(sh.cluster_fetch_packed())
         assert len(recs[-1]) == 10 * m_
     sm = sh.chunked_finish(k, m)
@@ -561,7 +565,8 @@ def scan_pass(sh, d, k=16, m=2, mcov=5, lean=False, stop_after=None):
     tail = O.clusters_to_bytes(np.array(mg.append_start[:mg.n_append], dtype=np.uint64), np.array(mg.append_len[:mg.n_append], dtype=np.uint16))
     what = (d.name, k, m, mcov, lean)
     assert b"".join(recs) + tail == w.clusters and mg.n_clust_out == w.enc and mg.total_written == len(w.es), what
-    st = sh.statistics(mcov, 0.99)
+    st, ost = sh.statistics(mcov, 0.99), O.statistics(w.es, w.el, mcov, 0.99)
+    assert list(st.hist) == list(ost.hist) and (st.n_clust, st.n_bases) == (ost.n_clust, ost.n_bases), what
     assert st.max_clust_length == w.mcl, what
     cnt = sh.find_events(p, st.max_clust_length)
     check_counts(cnt, w, what)
@@ -621,6 +626,27 @@ def test_chunked_reset_passes(ctx):
         run(C)
         run(A)
     finally:
+        sh.close()
+
+
+def test_chunked_scan_legacy_hook(ctx, monkeypatch):
+    """E2S_SCAN_LEGACY=1 forces K1 + K2 on resident shards only: a chunked shard keeps the one-pass scan, which writes each
+    chunk's records to its segments and starts from the open-cluster state the chunks before it left"""
+    d = data(1, tail=True)
+    monkeypatch.setenv("E2S_SCAN_LEGACY", "1")
+    sh = ctx.shard(d.n, 0, d.n, chunk_positions=CHUNK_E)
+    assert len(list(sh.chunks())) == 5
+    ctx.stage_reads(d.reads, d.off)
+    ctx.timing(True)
+    try:
+        drain(ctx)
+        for i, m in enumerate((2, 33)):
+            if i:
+                sh.chunked_reset()
+            scan_pass(sh, d, m=m, after_scan=lambda: path(ctx, True))
+    finally:
+        ctx.timing(False)
+        drain(ctx)
         sh.close()
 
 
@@ -686,17 +712,27 @@ def test_one_rank_sharded_steps(ctx, comm, monkeypatch):
     A, B = data(1, tail=True), data(2)
     ctx.stage_reads(A.reads, A.off)
     sh = resident(ctx, A)
+    ctx.timing(True)
     try:
-        for i, mcov in enumerate((5, 3, 5)):
-            w = want(A, mcov=mcov)
-            p = params(A, mcov)
-            mg, st, cnt = sh.pipeline_sharded(comm, p, 16, 2)
-            what = ("sharded", i, mcov)
-            assert (mg.total_written, mg.n_clust_out, st.max_clust_length) == (len(w.es), w.enc, w.mcl), what
-            check_counts(cnt, w, what)
-            assert sh.cluster_fetch_packed() == w.clusters and api.events_format(sh.events(), p) == w.text, what
-            step(sh, A, mcov=mcov, what="resident after sharded")
+        # E2S_NO_FUSED_PREFILTER keeps the phases of the resident step apart, not those of the sharded step
+        for no_fused in (False, True):
+            if no_fused:
+                monkeypatch.setenv("E2S_NO_FUSED_PREFILTER", "1")
+            for i, mcov in enumerate((5, 3, 5)):
+                w = want(A, mcov=mcov)
+                p = params(A, mcov)
+                drain(ctx)
+                mg, st, cnt = sh.pipeline_sharded(comm, p, 16, 2)
+                what = ("sharded", no_fused, i, mcov)
+                assert ctx.kernel_time(api.KERNEL_SCAN)[1] == 0, what  # (phase 2 starts from the scan's survivors: no k_code_scan)
+                assert (mg.total_written, mg.n_clust_out, st.max_clust_length) == (len(w.es), w.enc, w.mcl), what
+                check_counts(cnt, w, what)
+                assert sh.cluster_fetch_packed() == w.clusters and api.events_format(sh.events(), p) == w.text, what
+                step(sh, A, mcov=mcov, what="resident after sharded")
+        monkeypatch.delenv("E2S_NO_FUSED_PREFILTER")
     finally:
+        ctx.timing(False)
+        drain(ctx)
         sh.close()
     sh = ctx.shard(A.n, 0, A.n, chunk_positions=CHUNK_E)
     try:
