@@ -88,7 +88,7 @@ SYMBOLS = [
     "e2s_comm_unique_id", "e2s_comm_create", "e2s_comm_destroy", "e2s_pipeline_sharded",
     "e2s_exchange_row_words", "e2s_exchange_rows_finish",
     "e2s_pipeline_host_soa", "e2s_shard_host_gsa", "e2s_shard_load_lcp_bwt", "e2s_shard_load_bcr", "e2s_chunk_stage_clusters", "e2s_chunked_clusters_finish",
-    "e2s_pipeline_host_sharded", "e2s_shard_create_chunked", "e2s_shard_chunk_positions", "e2s_chunk_begin", "e2s_chunk_scan", "e2s_chunked_finish", "e2s_chunked_reset", "e2s_chunked_exchange",
+    "e2s_pipeline_host_sharded", "e2s_shard_build_egsa", "e2s_pipeline_reads", "e2s_shard_create_chunked", "e2s_shard_chunk_positions", "e2s_chunk_begin", "e2s_chunk_scan", "e2s_chunked_finish", "e2s_chunked_reset", "e2s_chunked_exchange",
 ]
 
 _lib = None
@@ -191,6 +191,9 @@ def load_library():
                                               C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_int32, C.POINTER(SnpParams),
                                               C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.c_void_p, C.c_uint64,
                                               C.POINTER(ClusterMerged), C.POINTER(Stats), C.POINTER(PipelineResult)]
+    lib.e2s_shard_build_egsa.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
+    lib.e2s_pipeline_reads.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_int32,
+                                       C.POINTER(SnpParams), C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(PipelineResult)]
     _lib = lib
     return lib
 
@@ -444,6 +447,22 @@ class Context:
                                             C.byref(res)))
         return res
 
+    def pipeline_reads(self, bases, off, params, k=16, min_len=2, x=1, y=4, z=1, rec10=None, events=None):
+        """ebwt2clust + clust2snp from the reads alone (e2s_pipeline_reads): `bases` = all reads back to back, `off` = R + 1
+        offsets (host).  The index is built on the device into the context's resident shard; records and events come out as
+        pipeline_host returns them for the X.gesa of layout x / y / z."""
+        bases = np.ascontiguousarray(bases, dtype=np.uint8).reshape(-1)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        if bases.size == 0:
+            bases = np.zeros(1, dtype=np.uint8)
+        res = PipelineResult()
+        cap_r = (rec10.nbytes // 10) if rec10 is not None else 0
+        cap_e = len(events) if events is not None else 0
+        self._ck(self.lib.e2s_pipeline_reads(self.h, _ptr(bases), _ptr(off), len(off) - 1, x, y, z, k, min_len, C.byref(params),
+                                             _ptr(rec10), cap_r, C.cast(events, C.c_void_p) if events is not None else None, cap_e,
+                                             C.byref(res)))
+        return res
+
     def pipeline_host_soa(self, lcp, bwt, pair_sa, n, reads_bases, reads_off, params, k=16, min_len=2, x=4, y=4, z=4,
                           rec10=None, events=None):
         """The same from the BCR triple (X.out.lcp, X.out, X.out.pairSA as byte buffers): only lcp + bwt cross PCIe in full,
@@ -601,6 +620,12 @@ class Shard:
             pair_sa = np.ascontiguousarray(pair_sa).view(np.uint8)
             self.ctx._ck(self.lib.e2s_shard_load_bcr(self.h, _ptr(lcp), x, _ptr(bwt), _ptr(pair_sa), y, z, int(first), count))
         self.ctx.synchronize()
+
+    def build_egsa(self, off, x=1, y=4, z=1):
+        """the index of the reads staged on this shard's context (Context.stage_reads; `off` = their R + 1 offsets, host) built on
+        the device straight into this resident shard, each field kept at its .gesa width (e2s_shard_build_egsa); seal() next"""
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        self.ctx._ck(self.lib.e2s_shard_build_egsa(self.h, _ptr(off), x, y, z))
 
     def set_layout(self, x=4, y=4, z=4, bcr=False):
         """byte widths / format of the index files the arrays came from (the reference's phantom record depends on it)"""

@@ -1,4 +1,4 @@
-"""Builds the CUDA library and the two CLIs in-tree with nvcc for sm_100a (cross-compiles without a GPU).
+"""Builds the CUDA library and the CLIs in-tree with nvcc for sm_100a (cross-compiles without a GPU).
 
     python -m ebwt2snp_b200.build            # library + CLIs
 """
@@ -21,7 +21,8 @@ ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 CUFLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-cudart", "static"] + ARCH
 
 CU_SOURCES = ["ctx.cu", "shard.cu", "build_host.cu", "phase1.cu", "phase2.cu", "pipeline.cu", "cluster.cu", "scan.cu", "merge.cu", "snp.cu", "unpack.cu", "build_egsa.cu"]
-CLI_SOURCES = {"ebwt2clust": ["ebwt2clust_main.cpp"], "clust2snp": ["clust2snp_main.cpp"], "build_gesa": ["build_gesa_main.cpp"]}
+CLI_SOURCES = {"ebwt2clust": ["ebwt2clust_main.cpp"], "clust2snp": ["clust2snp_main.cpp"], "build_gesa": ["build_gesa_main.cpp"],
+               "ebwt2snp": ["ebwt2snp_main.cpp"]}
 # text post-processors of the .snp format (no GPU work, no library): SURVEY.md 8(f) rank 3
 TEXT_TOOLS = {"filter_snp": ["filter_snp_main.cpp"], "snp2fastq": ["snp2fastq_main.cpp"], "snp_vs_vcf": ["snp_vs_vcf_main.cpp"]}
 

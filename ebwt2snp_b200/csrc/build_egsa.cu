@@ -36,7 +36,7 @@
 //   k_egsa_finish  decode (r, p); text, suff, bwt; lcp with the previous record = min(len_a - p_a, len_b - p_b, first
 //                  differing symbol) by clz on XORed key words.
 // Ids are 32-bit when they fit (equal lengths: n < 2^32; ragged: R << shift <= 2^32), else 64-bit.
-// Outputs go straight to device arrays (a shard's resident SoA arrays via e2s_shard_load_soa_dev, or the caller's).
+// Outputs go straight to device arrays (a resident shard's own arrays: e2s_shard_build_egsa, or the caller's).
 
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -63,7 +63,7 @@ struct ReadsView {
     __device__ __forceinline__ uint32_t len(uint64_t r) const { return off ? uint32_t(off[r + 1] - off[r]) : L; }
     __device__ __forceinline__ uint64_t row(uint64_t r, uint64_t st) const { return (st >> 5) + 2 * r; }
     template <typename IdT>
-    __device__ __forceinline__ void decode(IdT id, uint64_t& r, uint32_t& p) const {
+    __host__ __device__ __forceinline__ void decode(IdT id, uint64_t& r, uint32_t& p) const {
         if (shift) {
             r = uint64_t(id) >> shift;
             p = uint32_t(id) & ((1u << shift) - 1u);
@@ -387,9 +387,9 @@ k_radix_pass(const uint64_t* __restrict__ kin, const IdT* __restrict__ iin, uint
 template <typename IdT>
 __global__ void k_egsa_finish(ReadsView v, const uint64_t* __restrict__ packed, const IdT* __restrict__ ids, uint64_t n,
                               uint32_t* __restrict__ lcp, uint32_t* __restrict__ text, uint32_t* __restrict__ suff,
-                              uint8_t* __restrict__ bwt, uint64_t before) {
+                              uint8_t* __restrict__ bwt, uint64_t before, FieldMask mask) {
     // before: the record that precedes record 0 in the whole index, text << 32 | suff (a key range that does not start the
-    // index); ~0 = none, lcp[0] = 0
+    // index); ~0 = none, lcp[0] = 0.  mask: the field widths the values are kept at (all ones: full values)
     const uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;  // blockDim.x is a multiple of 32: whole warps leave together
     const uint32_t lane = threadIdx.x & 31;
     const bool valid = i < n;
@@ -399,8 +399,8 @@ __global__ void k_egsa_finish(ReadsView v, const uint64_t* __restrict__ packed, 
         v.decode(ids[i], r, p);
         st = v.start(r);
         len = v.len(r);
-        text[i] = uint32_t(r);
-        suff[i] = p;
+        text[i] = uint32_t(r) & mask.text;
+        suff[i] = p & mask.suff;
         bwt[i] = p ? v.bases[st + p - 1] : uint8_t('$');
     }
     const uint64_t* row = packed + v.row(r, st);
@@ -439,7 +439,7 @@ __global__ void k_egsa_finish(ReadsView v, const uint64_t* __restrict__ packed, 
             }
         }
     }
-    if (valid) lcp[i] = l;
+    if (valid) lcp[i] = l & mask.lcp;
 }
 
 // ---- one key range of the index ---------------------------------------------------------------------------------------------
@@ -647,13 +647,14 @@ struct KeyRange {              // host side: one key range of the index
     uint64_t cap;              // records the output arrays hold
     uint64_t before;           // the record before the range, text << 32 | suff; ~0 = none / not known
     uint64_t n_out, first_out; // results: records written, index position of the first one
+    uint64_t last;             // result: the last record written, text << 32 | suff at full width
 };
 
 inline unsigned blocks_for(uint64_t n, int t) { return unsigned((n + uint64_t(t) - 1) / uint64_t(t)); }
 
 template <typename IdT>
 cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const uint64_t* n_le_all, KeyRange* range, uint32_t* d_lcp,
-                        uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches) {
+                        uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, FieldMask mask, cudaStream_t stream, uint64_t* launches) {
     const uint32_t W = (v.L + 31) / 32;
     uint64_t n = n_all;                // suffixes this call sorts (a key range: known after the first sweep)
     const uint64_t* n_le = n_le_all;
@@ -812,10 +813,19 @@ cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const
         const uint32_t syms = v.L - 32 * uint32_t(w) < 32 ? v.L - 32 * uint32_t(w) : 32;
         sort_word(uint32_t(w), 64 - 2 * syms, (2 * syms + 7) / 8);
     }
-    k_egsa_finish<IdT><<<blocks_for(n, 256), 256, 0, stream>>>(v, packed, ic, n, d_lcp, d_text, d_suff, d_bwt, range ? range->before : ~uint64_t(0));
+    k_egsa_finish<IdT><<<blocks_for(n, 256), 256, 0, stream>>>(v, packed, ic, n, d_lcp, d_text, d_suff, d_bwt, range ? range->before : ~uint64_t(0),
+                                                               mask);
     *launches += 1;
     if ((e = cudaGetLastError()) != cudaSuccess) return done(e);
+    IdT last_id = 0;  // (the outputs may be masked: the next range's `before` is decoded from the id)
+    if (range && (e = cudaMemcpyAsync(&last_id, ic + n - 1, sizeof(IdT), cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return done(e);
     if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return done(e);
+    if (range) {
+        uint64_t r = 0;
+        uint32_t p = 0;
+        v.decode(last_id, r, p);
+        range->last = (r << 32) | p;
+    }
     return done(cudaSuccess);
 }
 
@@ -832,7 +842,8 @@ inline uint32_t ragged_shift(uint32_t L) {
 // total_bases = off[R].
 // scratch (freed before returning): two key buffers + two id buffers + tile status = 24.5 (32-bit ids) / 32.5 bytes per suffix
 cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint64_t* h_off, uint64_t R, uint32_t L, uint64_t total_bases,
-                       uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches) {
+                       uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches,
+                       FieldMask mask) {
     ReadsView v;
     v.bases = d_reads;
     v.off = d_off;
@@ -856,8 +867,8 @@ cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint
         for (uint32_t t = 0; t <= L; ++t) n_le[t] = R * (uint64_t(t) + 1);
     }
     if (getenv("E2S_BUILD_IDS64")) wide = true;  // test hook: the 64-bit instantiation on small inputs
-    return wide ? build_typed<uint64_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, stream, launches)
-                : build_typed<uint32_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, stream, launches);
+    return wide ? build_typed<uint64_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches)
+                : build_typed<uint32_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches);
 }
 
 // One key range of the index: the records of the suffixes whose first key word (32 symbols at 2 bits, A=0 C=1 G=2 T=3, most
@@ -869,7 +880,8 @@ cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint
 // RANGE + 8 bytes per 4096 suffixes of the collection.
 cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint64_t key_lo,
                              uint64_t key_hi, uint64_t before, uint64_t cap, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt,
-                             uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches) {
+                             uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches, FieldMask mask,
+                             uint64_t* last_out) {
     ReadsView v;
     v.bases = d_reads;
     v.off = d_off;
@@ -884,12 +896,13 @@ cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint
         wide = R > (uint64_t(1) << (32 - v.shift));
     }
     if (getenv("E2S_BUILD_IDS64")) wide = true;
-    KeyRange range{key_lo, key_hi, cap, before, 0, 0};
+    KeyRange range{key_lo, key_hi, cap, before, 0, 0, ~uint64_t(0)};
     // (the suffix lengths of a range come from its selection sweep: no whole-collection n_le)
-    const cudaError_t e = wide ? build_typed<uint64_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, stream, launches)
-                               : build_typed<uint32_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, stream, launches);
+    const cudaError_t e = wide ? build_typed<uint64_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches)
+                               : build_typed<uint32_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches);
     *n_out = range.n_out;
     *first_out = range.first_out;
+    if (last_out) *last_out = range.last;
     return e;
 }
 

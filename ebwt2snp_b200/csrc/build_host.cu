@@ -1,8 +1,9 @@
-// The index builder's entry points: whole index or key range, reads of one length or ragged, device or host buffers
-// (a host index larger than one call's device memory is built key range by key range).
+// The index builder's entry points: whole index or key range, reads of one length or ragged, device or host buffers, or
+// straight into a resident shard (an index larger than one call's device memory is built key range by key range).
 
 #include <stdlib.h>
 
+#include <functional>
 #include <utility>
 
 #include "host_state.h"
@@ -42,24 +43,11 @@ static int upload_offsets(e2s_ctx* c, const char* who, const uint64_t* off, uint
     return E2S_OK;
 }
 
-// shared by the four whole-index builder entry points.  off = nullptr: n_reads reads of read_len bases; else n_reads + 1 HOST offsets.
-static int build_egsa_common(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* off, uint64_t n_reads, uint32_t read_len,
-                             uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt) {
-    if (n_reads > 0xffffffffull) return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": more than 2^32 - 1 reads (text is a 32-bit field)");
-    uint64_t total = n_reads * uint64_t(read_len);
-    uint32_t longest = read_len;
-    uint64_t* d_off = nullptr;
-    if (off) {
-        int rc = check_offsets(c, who, off, n_reads, &longest);
-        if (rc == E2S_OK) rc = upload_offsets(c, who, off, n_reads, &d_off);
-        if (rc != E2S_OK) return rc;
-        total = off[n_reads];
-    }
-    cudaError_t e = build_egsa(d_reads, d_off, off, n_reads, longest, total, d_lcp, d_text, d_suff, d_bwt, c->stream, &c->launches);
-    if (d_off) {
-        cudaStreamSynchronize(c->stream);
-        cudaFree(d_off);
-    }
+// The whole index in one call, arguments checked.  d_off == nullptr: n_reads reads of `longest` bases; else n_reads + 1 DEVICE
+// offsets (off: the same in host memory), longest = the longest read.
+static int build_whole(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* d_off, const uint64_t* off, uint64_t n_reads,
+                       uint32_t longest, uint64_t total, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, FieldMask mask) {
+    const cudaError_t e = build_egsa(d_reads, d_off, off, n_reads, longest, total, d_lcp, d_text, d_suff, d_bwt, c->stream, &c->launches, mask);
     if (e == cudaErrorMemoryAllocation) {
         cudaGetLastError();
         return fail(c, E2S_ERR_NOMEM, std::string(who) + ": scratch buffers (24.5 bytes per suffix with 32-bit suffix ids, 32.5 with 64-bit ids)");
@@ -78,16 +66,39 @@ static int build_egsa_common(e2s_ctx* c, const char* who, const uint8_t* d_reads
     return E2S_OK;
 }
 
+// shared by the whole-index builder entry points of caller buffers.  off = nullptr: n_reads reads of read_len bases; else n_reads + 1
+// HOST offsets.
+static int build_egsa_common(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* off, uint64_t n_reads, uint32_t read_len,
+                             uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt) {
+    if (n_reads > 0xffffffffull) return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": more than 2^32 - 1 reads (text is a 32-bit field)");
+    uint64_t total = n_reads * uint64_t(read_len);
+    uint32_t longest = read_len;
+    uint64_t* d_off = nullptr;
+    if (off) {
+        int rc = check_offsets(c, who, off, n_reads, &longest);
+        if (rc == E2S_OK) rc = upload_offsets(c, who, off, n_reads, &d_off);
+        if (rc != E2S_OK) return rc;
+        total = off[n_reads];
+    }
+    const int rc = build_whole(c, who, d_reads, d_off, off, n_reads, longest, total, d_lcp, d_text, d_suff, d_bwt, FieldMask());
+    if (d_off) {
+        cudaStreamSynchronize(c->stream);
+        cudaFree(d_off);
+    }
+    return rc;
+}
+
 // one key range, both read shapes (arguments checked by the caller).  d_off == nullptr: n_reads reads of read_len bases; else n_reads + 1
 // DEVICE offsets, read_len = the longest read, total = off[n_reads].
 static int build_range_common(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* d_off, uint64_t n_reads, uint32_t read_len,
                               uint64_t total, uint64_t key_lo, uint64_t key_hi, uint32_t before_text, uint32_t before_suff, uint64_t capacity,
-                              uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, uint64_t* n_records, uint64_t* first_position) {
+                              uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, uint64_t* n_records, uint64_t* first_position,
+                              FieldMask mask = FieldMask(), uint64_t* last = nullptr) {
     const uint64_t before = before_text == 0xffffffffu ? ~uint64_t(0) : (uint64_t(before_text) << 32) | before_suff;
     *n_records = 0;
     *first_position = 0;
     cudaError_t e = build_egsa_range(d_reads, d_off, n_reads, read_len, total, key_lo, key_hi, before, capacity, d_lcp, d_text, d_suff, d_bwt,
-                                     n_records, first_position, c->stream, &c->launches);
+                                     n_records, first_position, c->stream, &c->launches, mask, last);
     if (e == cudaErrorMemoryAllocation) {
         cudaGetLastError();
         return fail(c, E2S_ERR_NOMEM, std::string(who) + ": scratch buffers (24.5 / 32.5 bytes per suffix of the range)");
@@ -140,16 +151,26 @@ struct IndexArraysDev {
     }
 };
 
-// An index that does not fit one call's device memory (outputs 13 B + scratch 24.5 / 32.5 B per suffix): the index key range by key
-// range (build_range_common), every range's records copied to their place in the host arrays.  d_off == nullptr: n_reads reads of
-// read_len bases; else DEVICE offsets (uploaded once for all ranges), read_len = the longest read.  A range that turns out to hold more
-// than `cap` records is cut in two.  E2S_BUILD_RANGE_RECORDS=<cap> forces this path (tests).
-static int build_egsa_host_ranges(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* d_off, uint64_t n_reads, uint32_t read_len,
-                                  uint64_t total, uint64_t cap, uint32_t* lcp, uint32_t* text, uint32_t* suff, uint8_t* bwt) {
+// Where the builder puts the index: host arrays (each key range is copied there from device buffers of one range), or device
+// arrays of the whole index written in place (a shard's: `written` then runs on the positions [at, at + m) just written).
+struct IndexDest {
+    uint32_t *lcp, *text, *suff;
+    uint8_t* bwt;
+    bool device;
+    FieldMask mask;
+    std::function<int(uint64_t at, uint64_t m)> written;
+};
+
+// An index that does not fit one call's device memory (scratch 24.5 / 32.5 B per suffix, + 13 B of outputs when they go to the
+// host): the index key range by key range (build_range_common), each range's records to their place in `out`.  d_off == nullptr:
+// n_reads reads of read_len bases; else DEVICE offsets (uploaded once for all ranges), read_len = the longest read.  A range that
+// turns out to hold more than `cap` records is cut in two.
+static int build_egsa_ranges(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* d_off, uint64_t n_reads, uint32_t read_len,
+                             uint64_t total, uint64_t cap, const IndexDest& out) {
     const char* range_who = d_off ? "e2s_build_egsa_ragged_range_dev" : "e2s_build_egsa_range_dev";
     const uint64_t n = total + n_reads;
     IndexArraysDev d;
-    if (d.alloc(cap) != cudaSuccess) return fail(c, E2S_ERR_NOMEM, std::string(who) + ": device buffers of one key range");
+    if (!out.device && d.alloc(cap) != cudaSuccess) return fail(c, E2S_ERR_NOMEM, std::string(who) + ": device buffers of one key range");
     // ranges as (lo, hi) with hi = 0 for "to the end of the key space", processed in key order from a stack
     uint64_t parts = (n + cap - 1) / cap;
     parts += parts / 4 + 1;
@@ -160,15 +181,18 @@ static int build_egsa_host_ranges(e2s_ctx* c, const char* who, const uint8_t* d_
         if (hi == 0 || hi > lo) todo.emplace_back(lo, hi);
     }
     uint64_t at = 0;
-    uint32_t before_text = 0xffffffffu, before_suff = 0;
+    uint64_t before = ~uint64_t(0);  // the last record so far, text << 32 | suff at full width
     int rc = E2S_OK;
     while (!todo.empty() && rc == E2S_OK) {
         const auto [lo, hi] = todo.back();
         todo.pop_back();
-        uint64_t m = 0, first = 0;
-        rc = build_range_common(c, range_who, d_reads, d_off, n_reads, read_len, total, lo, hi, before_text, before_suff, cap, d.lcp, d.text, d.suff,
-                                d.bwt, &m, &first);
-        if (rc == E2S_ERR_ARG && m > cap) {  // too many records for the buffers: two halves (a single key value cannot be cut)
+        uint64_t m = 0, first = 0, last = before;
+        // (in place: a range never writes past the end of the index)
+        const uint64_t room = out.device && n - at < cap ? n - at : cap;
+        rc = build_range_common(c, range_who, d_reads, d_off, n_reads, read_len, total, lo, hi, uint32_t(before >> 32), uint32_t(before), room,
+                                out.device ? out.lcp + at : d.lcp, out.device ? out.text + at : d.text, out.device ? out.suff + at : d.suff,
+                                out.device ? out.bwt + at : d.bwt, &m, &first, out.mask, &last);
+        if (rc == E2S_ERR_ARG && m > room) {  // too many records for the buffers: two halves (a single key value cannot be cut)
             const uint64_t width = hi - lo;  // (mod 2^64: right for hi = 0 as long as lo > 0 or the range is not the whole space)
             if (width == 1 || (lo == 0 && hi == 0)) {
                 rc = fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": one 32-symbol prefix is shared by more suffixes than fit the device");
@@ -186,19 +210,51 @@ static int build_egsa_host_ranges(e2s_ctx* c, const char* who, const uint8_t* d_
             break;
         }
         if (m) {
-            const cudaError_t e = d.to_host(lcp + at, text + at, suff + at, bwt + at, m, c->stream);
-            if (e != cudaSuccess) {
-                rc = cuda_fail(c, e, "D2H index arrays of a key range");
-                break;
+            if (out.device) {
+                rc = out.written(at, m);
+            } else {
+                const cudaError_t e = d.to_host(out.lcp + at, out.text + at, out.suff + at, out.bwt + at, m, c->stream);
+                if (e != cudaSuccess) rc = cuda_fail(c, e, "D2H index arrays of a key range");
             }
             at += m;
-            before_text = text[at - 1];
-            before_suff = suff[at - 1];
+            before = last;
         }
     }
     if (rc == E2S_OK && at != n) rc = fail(c, E2S_ERR_STATE, std::string(who) + ": key ranges do not cover the index");
     d.release();
     return rc;
+}
+
+// Does the whole index of `total` bases in n_reads reads (the longest: `longest` bases) fit one call on the device as it is now, the
+// reads already resident?  *cap = 0: build it whole; else the records per key range.  Scratch: 24.5 B per suffix with 32-bit suffix
+// ids, 32.5 with 64-bit ids (equal lengths: n < 2^32; ragged: R << shift, shift = the bits of the longest read's length + 1), plus
+// out_bytes per suffix when the outputs are device buffers of the call; packed reads and slack (half a byte per base), and for ragged
+// reads the 2 extra packed words and the device offset of every read.  0.92 of the free memory may be used.
+// E2S_BUILD_RANGE_RECORDS=<cap> forces key ranges (tests).
+static int range_records(e2s_ctx* c, const char* who, uint64_t total, uint64_t n_reads, bool ragged, uint32_t longest, uint64_t out_bytes,
+                         const char* advice, uint64_t* cap) {
+    const uint64_t n = total + n_reads;
+    bool ids64 = n > 0xffffffffull;
+    if (ragged) {
+        uint32_t bits = 1;
+        while ((longest >> bits) != 0) ++bits;
+        ids64 = n_reads > (uint64_t(1) << (32 - bits));
+    }
+    if (getenv("E2S_BUILD_IDS64")) ids64 = true;
+    *cap = 0;
+    if (const char* f = getenv("E2S_BUILD_RANGE_RECORDS")) {
+        *cap = strtoull(f, nullptr, 10);
+        return E2S_OK;
+    }
+    size_t free_b = 0, total_b = 0;
+    cudaMemGetInfo(&free_b, &total_b);
+    const uint64_t per_suffix = out_bytes + (ids64 ? 33 : 25);
+    const double fixed = double(total) / 2 + (ragged ? 24.0 * double(n_reads) : 0.0);
+    if (double(n) * double(per_suffix) + fixed <= 0.92 * double(free_b)) return E2S_OK;
+    const double room = 0.92 * double(free_b) - fixed - double(n) / 512;
+    *cap = room > 0 ? uint64_t(room / double(per_suffix)) : 0;
+    if (*cap < 4096) return fail(c, E2S_ERR_NOMEM, std::string(who) + ": not even one key range of the index fits the device" + advice);
+    return E2S_OK;
 }
 
 // host buffers in and out: device buffers allocated and released here
@@ -207,54 +263,36 @@ static int build_egsa_host(e2s_ctx* c, const char* who, const uint8_t* reads, co
     CU(c, cudaSetDevice(c->device));
     const uint64_t total = off ? off[n_reads] : n_reads * uint64_t(read_len);
     const uint64_t n = total + n_reads;
-    // suffix ids are 64-bit beyond 2^32 (equal lengths: n; ragged: R << shift, shift = the bits of the longest read's length + 1)
-    bool ids64 = n > 0xffffffffull;
     uint32_t longest = read_len;
     if (off) {
         if (n_reads > 0xffffffffull) return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": more than 2^32 - 1 reads (text is a 32-bit field)");
         const int rc = check_offsets(c, who, off, n_reads, &longest);
         if (rc != E2S_OK) return rc;
-        uint32_t bits = 1;
-        while ((longest >> bits) != 0) ++bits;
-        ids64 = n_reads > (uint64_t(1) << (32 - bits));
     }
-    if (getenv("E2S_BUILD_IDS64")) ids64 = true;
     uint8_t* d_reads = nullptr;
     cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&d_reads), total ? total : 1);
     if (e != cudaSuccess) {
         cudaGetLastError();
         return fail(c, E2S_ERR_NOMEM, std::string(who) + ": the reads on the device");
     }
-    {   // does the whole index fit one call?  13 B of outputs + up to 32.5 B of scratch per suffix, packed reads and slack (half a byte
-        // per base), and for ragged reads the 2 extra packed words and the device offset of every read; the reads are already resident
-        size_t free_b = 0, total_b = 0;
-        cudaMemGetInfo(&free_b, &total_b);
-        const uint64_t per_suffix = 13 + (ids64 ? 33 : 25);
-        const double fixed = double(total) / 2 + (off ? 24.0 * double(n_reads) : 0.0);
-        uint64_t cap = 0;
-        if (const char* f = getenv("E2S_BUILD_RANGE_RECORDS")) cap = strtoull(f, nullptr, 10);
-        else if (double(n) * double(per_suffix) + fixed > 0.92 * double(free_b)) {
-            const double room = 0.92 * double(free_b) - fixed - double(n) / 512;
-            cap = room > 0 ? uint64_t(room / double(per_suffix)) : 0;
-            if (cap < 4096) {
-                cudaFree(d_reads);
-                return fail(c, E2S_ERR_NOMEM, std::string(who) + ": not even one key range of the index fits the device");
-            }
+    uint64_t cap = 0;
+    if (int rc = range_records(c, who, total, n_reads, off != nullptr, longest, 13, "", &cap)) {
+        cudaFree(d_reads);
+        return rc;
+    }
+    if (cap) {
+        uint64_t* d_off = nullptr;
+        int rc = E2S_OK;
+        if (off) rc = upload_offsets(c, who, off, n_reads, &d_off);
+        if (rc == E2S_OK) {
+            e = cudaMemcpyAsync(d_reads, reads, total, cudaMemcpyHostToDevice, c->stream);
+            rc = e == cudaSuccess ? build_egsa_ranges(c, who, d_reads, d_off, n_reads, longest, total, cap, IndexDest{lcp, text, suff, bwt, false, FieldMask(), nullptr})
+                                  : cuda_fail(c, e, "H2D reads");
         }
-        if (cap) {
-            uint64_t* d_off = nullptr;
-            int rc = E2S_OK;
-            if (off) rc = upload_offsets(c, who, off, n_reads, &d_off);
-            if (rc == E2S_OK) {
-                e = cudaMemcpyAsync(d_reads, reads, total, cudaMemcpyHostToDevice, c->stream);
-                rc = e == cudaSuccess ? build_egsa_host_ranges(c, who, d_reads, d_off, n_reads, longest, total, cap, lcp, text, suff, bwt)
-                                      : cuda_fail(c, e, "H2D reads");
-            }
-            cudaStreamSynchronize(c->stream);
-            cudaFree(d_off);
-            cudaFree(d_reads);
-            return rc;
-        }
+        cudaStreamSynchronize(c->stream);
+        cudaFree(d_off);
+        cudaFree(d_reads);
+        return rc;
     }
     IndexArraysDev d;
     if (d.alloc(n) != cudaSuccess) {
@@ -338,6 +376,48 @@ int e2s_build_egsa_ragged(e2s_ctx* c, const uint8_t* bases, const uint64_t* off,
     if (!c || !bases || !off || !lcp || !text || !suff || !bwt) return fail(c, E2S_ERR_ARG, "e2s_build_egsa_ragged: NULL argument");
     if (n_reads == 0) return fail(c, E2S_ERR_ARG, "e2s_build_egsa_ragged: empty read collection");
     return build_egsa_host(c, "e2s_build_egsa_ragged", bases, off, n_reads, 0, lcp, text, suff, bwt);
+}
+
+// The index of the staged reads written straight into a resident shard's arrays, each field kept at its .gesa width, then the narrow
+// copies of what was written.  The staged reads (and, for ragged reads, their staged device offsets) are the builder's input.
+int e2s_shard_build_egsa(e2s_shard* s, const uint64_t* off, int x, int y, int z) {
+    const char* who = "e2s_shard_build_egsa";
+    if (!s || !off) return fail(s ? s->ctx : nullptr, E2S_ERR_ARG, std::string(who) + ": NULL argument");
+    e2s_ctx* c = s->ctx;
+    int rc;
+    if ((rc = check_field_sizes(c, {x, y, z}))) return rc;
+    if (s->chunked || s->global_off != 0 || s->n_local != s->n_global)
+        return fail(c, E2S_ERR_ARG, std::string(who) + ": needs a resident shard that holds the whole eBWT (not chunked, global_off = 0)");
+    if (!c->d_bases || !c->d_off || c->n_reads == 0) return fail(c, E2S_ERR_STATE, std::string(who) + ": stage the reads first (e2s_reads_stage)");
+    const uint64_t n_reads = c->n_reads;
+    if (off[n_reads] != c->n_bases) return fail(c, E2S_ERR_ARG, std::string(who) + ": `off` does not describe the staged reads");
+    if (n_reads > 0xffffffffull) return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": more than 2^32 - 1 reads (text is a 32-bit field)");
+    uint32_t longest = 0;
+    if ((rc = check_offsets(c, who, off, n_reads, &longest))) return rc;
+    const uint64_t total = off[n_reads], n = total + n_reads;
+    if (s->n_local != n) return fail(c, E2S_ERR_ARG, std::string(who) + ": the shard must hold off[n_reads] + n_reads positions");
+    const bool ragged = total != n_reads * uint64_t(longest);  // (every read has `longest` bases exactly when the sum says so)
+    CU(c, cudaSetDevice(c->device));
+    uint64_t cap = 0;
+    if ((rc = range_records(c, who, total, n_reads, ragged, longest, 0,
+                            " next to the shard; build the index file with build_gesa and stream it (ebwt2clust / clust2snp, "
+                            "e2s_pipeline_host) -- a chunked or multi-GPU build from reads is not supported",
+                            &cap)))
+        return rc;
+    auto mask = [](int w) { return w >= 4 ? ~0u : (1u << (8 * w)) - 1u; };
+    const FieldMask fm{mask(x), mask(y), mask(z)};
+    auto written = [&](uint64_t at, uint64_t m) -> int {
+        CU(c, derive_loaded(s, int64_t(at), m, true, true));
+        ++c->launches;
+        return E2S_OK;
+    };
+    s->sealed = false;
+    s->lay_x = x; s->lay_y = y; s->lay_z = z; s->lay_bcr = 0;
+    CU(c, cudaMemsetAsync(s->d_seal_flag, 0, 4, c->stream));  // every position is rewritten: the old verdict goes
+    const uint64_t* d_off = ragged ? c->d_off : nullptr;
+    if (cap) return build_egsa_ranges(c, who, c->d_bases, d_off, n_reads, longest, total, cap, IndexDest{s->lcp, s->text, s->suff, s->bwt, true, fm, written});
+    if ((rc = build_whole(c, who, c->d_bases, d_off, off, n_reads, longest, total, s->lcp, s->text, s->suff, s->bwt, fm))) return rc;
+    return written(0, n);
 }
 
 }  // extern "C"

@@ -259,6 +259,8 @@ uint64_t round_up(uint64_t v, uint64_t a);
 uint64_t chunk_buffer_positions(uint64_t chunk_positions, uint64_t n_local);
 int ensure_copy_stream(e2s_ctx* c);
 int load_lcp_bwt(e2s_shard* s, const void* lcp, int x, const uint8_t* bwt, uint64_t first, uint64_t count, bool dev);
+// the narrow resident copies (byte LCP, base-code bit planes) of the local positions [l, l + cnt) just written
+cudaError_t derive_loaded(e2s_shard* s, int64_t l, uint64_t cnt, bool have_lcp, bool have_bwt);
 
 // phase1.cu
 void put_rec10(uint8_t* o, uint64_t start, uint64_t len);

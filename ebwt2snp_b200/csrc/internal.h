@@ -217,17 +217,26 @@ cudaError_t launch_fill_phantom(uint32_t* lcp, uint32_t* text, uint32_t* suff, u
                                 uint64_t count, int x, int y, int z, int bcr, cudaStream_t stream);
 
 // ---- EGSA construction (build_egsa.cu) -----------------------------------------------------------
+// What the builder keeps of each output value: the field widths of a .gesa file (lcp mod 2^(8x), text mod 2^(8y), suff mod 2^(8z),
+// as its writer truncates them); all ones = the full values
+struct FieldMask {
+    uint32_t lcp = ~0u, text = ~0u, suff = ~0u;
+};
+
 // suffix sort of R reads (device pointer, no separators) -> lcp/text/suff/bwt device arrays of total_bases + R elements; synchronises.
 // d_off == nullptr: every read has L bases; else R + 1 DEVICE offsets (h_off: the same in host memory) and L = the longest read (< 65536).
 // cudaErrorInvalidValue = a base outside ACGT / acgt; cudaErrorInvalidConfiguration = a read of 65536 bases or more.
 cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint64_t* h_off, uint64_t R, uint32_t L, uint64_t total_bases,
-                       uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches);
+                       uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches,
+                       FieldMask mask = FieldMask());
 
 // one key range of the index (see build_egsa.cu); reads as for build_egsa (d_off == nullptr: R reads of L bases), no host offsets needed;
-// cudaErrorInvalidPitchValue = more than `cap` records (*n_out says how many)
+// cudaErrorInvalidPitchValue = more than `cap` records (*n_out says how many).  *last_out (when not null, and the range is not empty) =
+// the range's last record as text << 32 | suff at full width: the `before` of the next range whatever the mask
 cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint64_t key_lo,
                              uint64_t key_hi, uint64_t before, uint64_t cap, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt,
-                             uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches);
+                             uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches, FieldMask mask = FieldMask(),
+                             uint64_t* last_out = nullptr);
 
 // ---- phase 2 -----------------------------------------------------------------------------------
 struct SnpDev {  // device counters of one e2s_find_events

@@ -234,24 +234,23 @@ static int finish_range(e2s_shard* s, const char* who, uint32_t k, int32_t min_l
     return E2S_OK;
 }
 
-// the same from a resident shard (inputs the one-pass scan does not take: an LCP value above 127, -m > 33)
-static int pipeline_host_resident(e2s_ctx* c, const void* gesa, uint64_t n, int x, int y, int z, uint32_t k, int32_t min_len,
-                                  const e2s_snp_params* p, void* rec10, uint64_t cap_records, e2s_event* events, uint64_t cap_events,
-                                  e2s_pipeline_result* res) {
-    int rc;
+// the context's cached resident shard of n positions (the whole eBWT): kept when it has that size, else made anew
+static int cached_resident(e2s_ctx* c, uint64_t n, e2s_shard** out) {
     e2s_shard* s = c->cached;
     if (!s || s->chunked || s->n_local != n || s->n_global != n) {
         if (s) e2s_shard_destroy(s);
         c->cached = nullptr;
-        rc = e2s_shard_create(c, n, 0, n, &s);
-        if (rc) return rc;
+        if (int rc = e2s_shard_create(c, n, 0, n, &s)) return rc;
         c->cached = s;
     }
-    const int rs = x + y + z + 1;
-    CU(c, cudaMemsetAsync(s->d_seal_flag, 0, 4, c->stream));  // a cached shard is reloaded from its first position: forget the old verdict
-    if ((rc = e2s_shard_load_gesa(s, gesa, 0, n, x, y, z))) return rc;
-    if ((rc = e2s_shard_seal(s))) return rc;
-    res->h2d_bytes += n * uint64_t(rs);
+    *out = s;
+    return E2S_OK;
+}
+
+// e2s_pipeline_resident on a sealed resident shard, then its records into rec10 and its events to the caller
+static int resident_to_caller(e2s_shard* s, uint32_t k, int32_t min_len, const e2s_snp_params* p, void* rec10, uint64_t cap_records,
+                              e2s_event* events, uint64_t cap_events, e2s_pipeline_result* res) {
+    int rc;
     if ((rc = e2s_pipeline_resident(s, k, min_len, p, res))) return rc;
     if (rec10) {
         uint64_t m = 0;
@@ -263,6 +262,21 @@ static int pipeline_host_resident(e2s_ctx* c, const void* gesa, uint64_t n, int 
         if ((rc = e2s_events_fetch(s, events, cap_events, &nv))) return rc;
     }
     return E2S_OK;
+}
+
+// the same from a resident shard (inputs the one-pass scan does not take: an LCP value above 127, -m > 33)
+static int pipeline_host_resident(e2s_ctx* c, const void* gesa, uint64_t n, int x, int y, int z, uint32_t k, int32_t min_len,
+                                  const e2s_snp_params* p, void* rec10, uint64_t cap_records, e2s_event* events, uint64_t cap_events,
+                                  e2s_pipeline_result* res) {
+    int rc;
+    e2s_shard* s;
+    if ((rc = cached_resident(c, n, &s))) return rc;
+    const int rs = x + y + z + 1;
+    CU(c, cudaMemsetAsync(s->d_seal_flag, 0, 4, c->stream));  // a cached shard is reloaded from its first position: forget the old verdict
+    if ((rc = e2s_shard_load_gesa(s, gesa, 0, n, x, y, z))) return rc;
+    if ((rc = e2s_shard_seal(s))) return rc;
+    res->h2d_bytes += n * uint64_t(rs);
+    return resident_to_caller(s, k, min_len, p, rec10, cap_records, events, cap_events, res);
 }
 
 // All chunks of a chunked shard's range from host records (`records` = the record of global position `first`; it must reach
@@ -358,6 +372,25 @@ int e2s_pipeline_host(e2s_ctx* c, const void* gesa, uint64_t n, int x, int y, in
     if (rc) return rc;
     // (outside the fall-back: "no clusters" is E2S_ERR_UNSUPPORTED too, and returned as it is)
     return phase2_to_caller(s, p, events, cap_events, res);
+}
+
+// ebwt2clust + clust2snp from the reads alone: the reads cross PCIe once and serve both the index build (straight into the
+// context's resident shard) and phase 2.  Inputs the one-pass scan does not take go where e2s_pipeline_resident sends them.
+int e2s_pipeline_reads(e2s_ctx* c, const uint8_t* read_bases, const uint64_t* read_off, uint64_t n_reads, int x, int y, int z, uint32_t k,
+                       int32_t min_len, const e2s_snp_params* p, void* rec10, uint64_t cap_records, e2s_event* events, uint64_t cap_events,
+                       e2s_pipeline_result* res) {
+    if (!c || !read_bases || !read_off || !p || !res) return fail(c, E2S_ERR_ARG, "e2s_pipeline_reads: NULL argument");
+    memset(res, 0, sizeof *res);
+    int rc;
+    if ((rc = check_field_sizes(c, {x, y, z}))) return rc;
+    if (n_reads == 0) return fail(c, E2S_ERR_ARG, "e2s_pipeline_reads: empty read collection");
+    const uint64_t n = read_off[n_reads] + n_reads;
+    if ((rc = stage_reads(c, read_bases, read_off, n_reads, res))) return rc;
+    e2s_shard* s;
+    if ((rc = cached_resident(c, n, &s))) return rc;
+    if ((rc = e2s_shard_build_egsa(s, read_off, x, y, z))) return rc;
+    if ((rc = e2s_shard_seal(s))) return rc;
+    return resident_to_caller(s, k, min_len, p, rec10, cap_records, events, cap_events, res);
 }
 
 // ebwt2clust + clust2snp from the BCR triple in host memory, lean: only X.out.lcp (x bytes per position) and X.out (1 byte) are

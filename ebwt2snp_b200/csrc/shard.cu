@@ -132,7 +132,7 @@ int ensure_copy_stream(e2s_ctx* c) {
 static int64_t checked_hi(const e2s_shard* s) { return int64_t(s->n_local) + (s->global_off + s->n_local == s->n_global ? 0 : 1); }
 
 // every load also writes the narrow resident copies of what it loaded (k_derive): byte LCP + base-code bit planes
-static cudaError_t derive_loaded(e2s_shard* s, int64_t l, uint64_t cnt, bool have_lcp, bool have_bwt) {
+cudaError_t derive_loaded(e2s_shard* s, int64_t l, uint64_t cnt, bool have_lcp, bool have_bwt) {
     return launch_derive(s->lcp, have_bwt ? s->bwt : nullptr, have_lcp ? s->lcpt : nullptr, s->d_planes,
                          l, l + int64_t(cnt), -2, checked_hi(s), s->d_seal_flag, s->ctx->stream, s->ctx->sm_count);
 }

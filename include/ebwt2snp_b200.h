@@ -163,6 +163,16 @@ int e2s_shard_seal(e2s_shard *sh);
  * Setting E2S_LCP_WIDE=1 in the environment before the seal keeps the 4-byte stream. */
 int e2s_shard_lcp_bytes_resident(const e2s_shard *sh);
 
+/* The index of the reads staged on the shard's context (e2s_reads_stage / _dev), built on the device straight into the
+ * shard's own arrays: what e2s_shard_load_* of the X.gesa that `build_gesa -x x -y y -z z` writes would leave, without the
+ * file (each field truncated to its width as that file holds it; the layout set as e2s_shard_set_layout(x, y, z, 0) does).
+ * off = the staged collection's n_reads + 1 offsets in HOST memory (checked as the ragged builders check them).  The shard
+ * must hold the whole eBWT: n_local = n_global = off[n_reads] + n_reads, global_off = 0, not chunked.  The whole index is
+ * built in one call when its scratch fits 0.92 of the free device memory next to the shard and the reads, else key range by
+ * key range (E2S_BUILD_RANGE_RECORDS forces ranges).  A base outside ACGT, a read of 65536 bases or more: E2S_ERR_UNSUPPORTED;
+ * not even one key range fits: E2S_ERR_NOMEM.  Call e2s_shard_seal afterwards. */
+int e2s_shard_build_egsa(e2s_shard *sh, const uint64_t *off, int x, int y, int z);
+
 /* the read collection (FASTA bases), needed by e2s_find_events only: ref:clust2snp.cpp:147-212 */
 int e2s_reads_stage(e2s_ctx *ctx, const uint8_t *bases, const uint64_t *offsets /* n_reads+1 */, uint64_t n_reads);
 int e2s_reads_stage_dev(e2s_ctx *ctx, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n_reads,
@@ -397,6 +407,14 @@ int e2s_pipeline_host(e2s_ctx *ctx, const void *gesa_records, uint64_t n, int x,
                       uint32_t k, int32_t min_len, const e2s_snp_params *p,
                       void *rec10, uint64_t cap_records, e2s_event *events, uint64_t cap_events,
                       e2s_pipeline_result *res);
+
+/* ebwt2clust + clust2snp from the reads alone, on one GPU: stage the reads (the only H2D), build the index into a resident
+ * shard (e2s_shard_build_egsa), seal, e2s_pipeline_resident, then records / events out exactly as e2s_pipeline_host returns
+ * them for the X.gesa of layout x/y/z.  res->h2d_bytes = reads + offsets.  The context's resident shard is kept for the next
+ * call of the same n. */
+int e2s_pipeline_reads(e2s_ctx *ctx, const uint8_t *read_bases, const uint64_t *read_off, uint64_t n_reads, int x, int y, int z,
+                       uint32_t k, int32_t min_len, const e2s_snp_params *p, void *rec10, uint64_t cap_records,
+                       e2s_event *events, uint64_t cap_events, e2s_pipeline_result *res);
 
 /* The same from the BCR triple (ref:include.hpp:157-188: X.out.lcp = lcp(x) per position, X.out = BWT bytes, X.out.pairSA =
  * suff(z) then text(y) per position), LEAN: phase 1 and the BWT prefilter need the LCP and the BWT only, so 1 + x bytes per
