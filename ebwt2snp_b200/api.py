@@ -89,6 +89,8 @@ SYMBOLS = [
     "e2s_exchange_row_words", "e2s_exchange_rows_finish",
     "e2s_pipeline_host_soa", "e2s_shard_host_gsa", "e2s_shard_load_lcp_bwt", "e2s_shard_load_bcr", "e2s_chunk_stage_clusters", "e2s_chunked_clusters_finish",
     "e2s_pipeline_host_sharded", "e2s_shard_build_egsa", "e2s_pipeline_reads", "e2s_shard_create_chunked", "e2s_shard_chunk_positions", "e2s_chunk_begin", "e2s_chunk_scan", "e2s_chunked_finish", "e2s_chunked_reset", "e2s_chunked_exchange",
+    "e2s_reads_key_cuts", "e2s_shard_build_egsa_range", "e2s_shard_halo_row_words", "e2s_shard_halo_row", "e2s_shard_halo_apply",
+    "e2s_device_count",
 ]
 
 _lib = None
@@ -194,8 +196,27 @@ def load_library():
     lib.e2s_shard_build_egsa.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
     lib.e2s_pipeline_reads.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_int32,
                                        C.POINTER(SnpParams), C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(PipelineResult)]
+    lib.e2s_reads_key_cuts.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+    lib.e2s_shard_build_egsa_range.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_int]
+    lib.e2s_shard_halo_row_words.restype = C.c_uint64
+    lib.e2s_shard_halo_row_words.argtypes = []
+    lib.e2s_shard_halo_row.argtypes = [C.c_void_p, C.c_void_p]
+    lib.e2s_shard_halo_apply.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
+    lib.e2s_device_count.argtypes = [C.POINTER(C.c_int)]
     _lib = lib
     return lib
+
+
+def halo_row_words() -> int:
+    """u64 words of one shard's halo row (e2s_shard_halo_row_words)"""
+    return int(load_library().e2s_shard_halo_row_words())
+
+
+def __getattr__(name):
+    """HALO_ROW_WORDS: read from the library when first asked for (importing this module does not load it)"""
+    if name == "HALO_ROW_WORDS":
+        return halo_row_words()
+    raise AttributeError(name)
 
 
 def default_params(nr_reads1=0, **kw) -> SnpParams:
@@ -430,6 +451,15 @@ class Context:
         out.update(n=m, R=R, first=int(first.value))
         return out
 
+    def key_cuts(self, off, parts):
+        """cuts of the key space into `parts` shards of the index of the staged reads (e2s_reads_key_cuts; `off` = their R + 1 offsets,
+        host) -> (key_lo: `parts` uint64 with key_lo[0] = 0, position: `parts` + 1 uint64, the index position of every cut and n)"""
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        key_lo = np.zeros(int(parts), dtype=np.uint64)
+        position = np.zeros(int(parts) + 1, dtype=np.uint64)
+        self._ck(self.lib.e2s_reads_key_cuts(self.h, _ptr(off), int(parts), _ptr(key_lo), _ptr(position)))
+        return key_lo, position
+
     def shard(self, n_local, global_off=0, n_global=None, chunk_positions=None):
         """chunk_positions: a CHUNKED shard -- the device buffers hold one chunk of the range at a time (streaming)"""
         return Shard(self, n_local, global_off, n_local if n_global is None else n_global, chunk_positions)
@@ -626,6 +656,24 @@ class Shard:
         the device straight into this resident shard, each field kept at its .gesa width (e2s_shard_build_egsa); seal() next"""
         off = np.ascontiguousarray(off, dtype=np.uint64)
         self.ctx._ck(self.lib.e2s_shard_build_egsa(self.h, _ptr(off), x, y, z))
+
+    def build_egsa_range(self, off, key_lo, key_hi, x=1, y=4, z=1):
+        """build_egsa for the records of the key range [key_lo, key_hi) only (key_hi = 0: no upper bound), which must be this shard's
+        positions of the whole index (e2s_shard_build_egsa_range); halo_row / halo_apply, then seal() next"""
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        self.ctx._ck(self.lib.e2s_shard_build_egsa_range(self.h, _ptr(off), int(key_lo), int(key_hi), x, y, z))
+
+    def halo_row(self):
+        """this built shard's halo row: HALO_ROW_WORDS uint64 (e2s_shard_halo_row)"""
+        row = np.zeros(halo_row_words(), dtype=np.uint64)
+        self.ctx._ck(self.lib.e2s_shard_halo_row(self.h, _ptr(row)))
+        return row
+
+    def halo_apply(self, rows, my):
+        """every shard's halo row in shard order ((shards, HALO_ROW_WORDS) uint64) -> this shard's halos and boundary LCPs
+        (e2s_shard_halo_apply); seal() next"""
+        rows = np.ascontiguousarray(rows, dtype=np.uint64)
+        self.ctx._ck(self.lib.e2s_shard_halo_apply(self.h, _ptr(rows), int(rows.shape[0]), int(my)))
 
     def set_layout(self, x=4, y=4, z=4, bcr=False):
         """byte widths / format of the index files the arrays came from (the reference's phantom record depends on it)"""

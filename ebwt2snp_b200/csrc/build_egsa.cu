@@ -42,6 +42,7 @@
 #include <stdint.h>
 #include <stdlib.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "common.cuh"
@@ -647,14 +648,14 @@ struct KeyRange {              // host side: one key range of the index
     uint64_t cap;              // records the output arrays hold
     uint64_t before;           // the record before the range, text << 32 | suff; ~0 = none / not known
     uint64_t n_out, first_out; // results: records written, index position of the first one
-    uint64_t last;             // result: the last record written, text << 32 | suff at full width
 };
 
 inline unsigned blocks_for(uint64_t n, int t) { return unsigned((n + uint64_t(t) - 1) / uint64_t(t)); }
 
 template <typename IdT>
 cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const uint64_t* n_le_all, KeyRange* range, uint32_t* d_lcp,
-                        uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, FieldMask mask, cudaStream_t stream, uint64_t* launches) {
+                        uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, FieldMask mask, cudaStream_t stream, uint64_t* launches,
+                        uint64_t* ends) {
     const uint32_t W = (v.L + 31) / 32;
     uint64_t n = n_all;                // suffixes this call sorts (a key range: known after the first sweep)
     const uint64_t* n_le = n_le_all;
@@ -817,16 +818,128 @@ cudaError_t build_typed(ReadsView v, uint64_t n_all, uint64_t total_bases, const
                                                                mask);
     *launches += 1;
     if ((e = cudaGetLastError()) != cudaSuccess) return done(e);
-    IdT last_id = 0;  // (the outputs may be masked: the next range's `before` is decoded from the id)
-    if (range && (e = cudaMemcpyAsync(&last_id, ic + n - 1, sizeof(IdT), cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return done(e);
+    IdT end_id[2] = {0, 0};  // (the outputs may be masked: the first and last records at full width are decoded from the ids)
+    if (ends && (e = cudaMemcpyAsync(&end_id[0], ic, sizeof(IdT), cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return done(e);
+    if (ends && (e = cudaMemcpyAsync(&end_id[1], ic + n - 1, sizeof(IdT), cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return done(e);
     if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return done(e);
-    if (range) {
+    for (int j = 0; ends && j < 2; ++j) {
         uint64_t r = 0;
         uint32_t p = 0;
-        v.decode(last_id, r, p);
-        range->last = (r << 32) | p;
+        v.decode(end_id[j], r, p);
+        ends[j] = (r << 32) | p;
     }
     return done(cudaSuccess);
+}
+
+// ---- cuts of the key space for several shards --------------------------------------------------------------------------------
+// k_key_sample takes the first key word of m suffix slots at a fixed stride (slot k n / m), k_cut_count puts every suffix of the
+// collection into the range its first key word falls in (a binary search over the cuts in shared memory) and counts them per
+// range: warp-aggregated shared-memory counters, one global atomic per CTA and range.  Slots map to suffixes as in k_range_select.
+constexpr uint32_t CUT_MAX = 1024;  // ranges one k_cut_count handles
+
+template <bool RAGGED>
+__device__ __forceinline__ uint64_t slot_key(const ReadsView& v, const uint64_t* __restrict__ packed, uint64_t i) {
+    uint64_t r, st;
+    uint32_t p, len;
+    if (RAGGED) {
+        r = read_of_slot(v.off, v.R, i);
+        st = v.off[r];
+        p = uint32_t(i - st - r);
+        len = uint32_t(v.off[r + 1] - st);
+    } else {
+        v.decode(uint64_t(i), r, p);
+        st = v.start(r);
+        len = v.L;
+    }
+    return suffix_word(packed + v.row(r, st), len, p, 0);
+}
+
+template <bool RAGGED>
+__global__ void __launch_bounds__(256) k_key_sample(ReadsView v, const uint64_t* __restrict__ packed, uint64_t n, uint64_t m,
+                                                    uint64_t* __restrict__ keys) {
+    const uint64_t k = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (k < m) keys[k] = slot_key<RAGGED>(v, packed, k * n / m);  // (k < 2^16, n < 2^47: no overflow)
+}
+
+template <bool RAGGED>
+__global__ void __launch_bounds__(SEL_THREADS) k_cut_count(ReadsView v, const uint64_t* __restrict__ packed, uint64_t n,
+                                                           const uint64_t* __restrict__ cuts, uint32_t parts,
+                                                           unsigned long long* __restrict__ counts) {
+    __shared__ uint64_t s_cut[CUT_MAX];
+    __shared__ unsigned long long s_cnt[CUT_MAX];
+    const uint32_t tid = threadIdx.x, lane = tid & 31;
+    for (uint32_t b = tid; b < parts; b += SEL_THREADS) {
+        s_cut[b] = cuts[b];
+        s_cnt[b] = 0;
+    }
+    __syncthreads();
+    const uint64_t base = (uint64_t(blockIdx.x) * SEL_THREADS + tid) * SEL_IPT;
+    // the thread's slots [base, base + SEL_IPT): ragged, the first one's read by a binary search, then a walk along the reads
+    uint64_t r = 0, st = 0;
+    uint32_t p = 0, len = 0;
+    if (RAGGED && base < n) {
+        r = read_of_slot(v.off, v.R, base);
+        st = v.off[r];
+        p = uint32_t(base - st - r);
+        len = uint32_t(v.off[r + 1] - st);
+    }
+    for (int j = 0; j < SEL_IPT; ++j) {
+        const uint64_t i = base + j;
+        uint32_t bin = CUT_MAX + lane;  // (no slot: a bin of its own, never counted)
+        if (i < n) {
+            uint64_t key;
+            if (RAGGED) {
+                if (p > len) {  // past read r's terminator: the next read
+                    ++r;
+                    st = v.off[r];
+                    p = 0;
+                    len = uint32_t(v.off[r + 1] - st);
+                }
+                key = suffix_word(packed + v.row(r, st), len, p++, 0);
+            } else {
+                key = slot_key<false>(v, packed, i);
+            }
+            uint32_t a = 0, z = parts;  // s_cut[a] <= key < s_cut[z] (s_cut[0] = 0)
+            while (z - a > 1) {
+                const uint32_t mid = (a + z) >> 1;
+                if (s_cut[mid] <= key) a = mid;
+                else z = mid;
+            }
+            bin = a;
+        }
+        const uint32_t same = __match_any_sync(0xffffffffu, bin);
+        if (bin < CUT_MAX && lane == uint32_t(__ffs(int(same)) - 1)) atomicAdd(&s_cnt[bin], (unsigned long long)__popc(same));
+    }
+    __syncthreads();
+    for (uint32_t b = tid; b < parts; b += SEL_THREADS)
+        if (s_cnt[b]) atomicAdd(counts + b, s_cnt[b]);
+}
+
+// one warp per pair of suffixes: 32 symbols per round, the first differing one by a ballot
+__global__ void __launch_bounds__(256) k_pair_lcp(const uint8_t* __restrict__ bases, const uint64_t* __restrict__ off,
+                                                  const uint64_t* __restrict__ pairs, uint32_t n_pairs, uint32_t lcp_mask,
+                                                  uint32_t* __restrict__ lcp) {
+    const uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (j >= n_pairs) return;  // (the whole warp)
+    uint64_t at[2];
+    uint32_t rest[2];
+    for (int q = 0; q < 2; ++q) {
+        const uint64_t id = pairs[2 * j + q], r = id >> 32, st = off[r];
+        const uint32_t p = uint32_t(id), len = uint32_t(off[r + 1] - st);
+        at[q] = st + p;
+        rest[q] = p <= len ? len - p : 0;  // symbols before the terminator
+    }
+    uint32_t l = rest[0] < rest[1] ? rest[0] : rest[1];
+    for (uint32_t s = 0; s < l; s += 32) {
+        const uint32_t q = s + lane;
+        const bool diff = q < l && code2(bases[at[0] + q]) != code2(bases[at[1] + q]);
+        const uint32_t b = __ballot_sync(0xffffffffu, diff);
+        if (b) {
+            l = s + uint32_t(__ffs(int(b))) - 1;
+            break;
+        }
+    }
+    if (lane == 0) lcp[j] = l & lcp_mask;
 }
 
 // ragged ids (r << shift) | p: the bits of p in [0, L]
@@ -843,7 +956,7 @@ inline uint32_t ragged_shift(uint32_t L) {
 // scratch (freed before returning): two key buffers + two id buffers + tile status = 24.5 (32-bit ids) / 32.5 bytes per suffix
 cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint64_t* h_off, uint64_t R, uint32_t L, uint64_t total_bases,
                        uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches,
-                       FieldMask mask) {
+                       FieldMask mask, uint64_t* ends) {
     ReadsView v;
     v.bases = d_reads;
     v.off = d_off;
@@ -867,8 +980,8 @@ cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint
         for (uint32_t t = 0; t <= L; ++t) n_le[t] = R * (uint64_t(t) + 1);
     }
     if (getenv("E2S_BUILD_IDS64")) wide = true;  // test hook: the 64-bit instantiation on small inputs
-    return wide ? build_typed<uint64_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches)
-                : build_typed<uint32_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches);
+    return wide ? build_typed<uint64_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches, ends)
+                : build_typed<uint32_t>(v, n, total_bases, n_le.data(), nullptr, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches, ends);
 }
 
 // One key range of the index: the records of the suffixes whose first key word (32 symbols at 2 bits, A=0 C=1 G=2 T=3, most
@@ -881,7 +994,7 @@ cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint
 cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint64_t key_lo,
                              uint64_t key_hi, uint64_t before, uint64_t cap, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt,
                              uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches, FieldMask mask,
-                             uint64_t* last_out) {
+                             uint64_t* ends_out) {
     ReadsView v;
     v.bases = d_reads;
     v.off = d_off;
@@ -896,14 +1009,77 @@ cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint
         wide = R > (uint64_t(1) << (32 - v.shift));
     }
     if (getenv("E2S_BUILD_IDS64")) wide = true;
-    KeyRange range{key_lo, key_hi, cap, before, 0, 0, ~uint64_t(0)};
+    KeyRange range{key_lo, key_hi, cap, before, 0, 0};
     // (the suffix lengths of a range come from its selection sweep: no whole-collection n_le)
-    const cudaError_t e = wide ? build_typed<uint64_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches)
-                               : build_typed<uint32_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches);
+    const cudaError_t e = wide ? build_typed<uint64_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches, ends_out)
+                               : build_typed<uint32_t>(v, n, total_bases, nullptr, &range, d_lcp, d_text, d_suff, d_bwt, mask, stream, launches, ends_out);
     *n_out = range.n_out;
     *first_out = range.first_out;
-    if (last_out) *last_out = range.last;
     return e;
+}
+
+// Cuts of the key space for `parts` shards (the declaration in internal.h).  The sample is sorted on the host; cut i is its
+// (i / parts) quantile, bumped to one above cut i - 1 when it is not above it (a heavy key value cannot be cut: the ranges after
+// it start past it).  Then one sweep over all suffixes counts each range exactly.  cudaErrorInvalidConfiguration: the cuts
+// cannot be made strictly increasing, or parts is 0 or above CUT_MAX.
+cudaError_t key_cuts(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint32_t parts,
+                     uint64_t* key_lo, uint64_t* position, cudaStream_t stream, uint64_t* launches) {
+    if (parts == 0 || parts > CUT_MAX || (d_off && L >= 65536)) return cudaErrorInvalidConfiguration;
+    ReadsView v;
+    v.bases = d_reads;
+    v.off = d_off;
+    v.R = R;
+    v.L = L;
+    v.shift = d_off ? ragged_shift(L) : 0;
+    const uint64_t n = total_bases + R, n_chunks = (n + SEL_CHUNK - 1) / SEL_CHUNK;
+    if (n_chunks >= (uint64_t(1) << 31)) return cudaErrorInvalidConfiguration;
+    const uint64_t m = n < (uint64_t(1) << 16) ? n : (uint64_t(1) << 16);
+    const uint64_t packed_words = (total_bases >> 5) + 2 * R + 2;
+    uint64_t *packed = nullptr, *scratch = nullptr;  // scratch: the bad flag, the sample, the cuts, the counts
+    auto done = [&](cudaError_t rc) {
+        cudaFree(packed);
+        cudaFree(scratch);
+        return rc;
+    };
+    const size_t scratch_words = 1 + m + 2 * size_t(parts);
+    cudaError_t e;
+    if ((e = cudaMalloc(reinterpret_cast<void**>(&packed), packed_words * 8)) != cudaSuccess) return done(e);
+    if ((e = cudaMalloc(reinterpret_cast<void**>(&scratch), scratch_words * 8)) != cudaSuccess) return done(e);
+    if ((e = cudaMemsetAsync(scratch, 0, scratch_words * 8, stream)) != cudaSuccess) return done(e);
+    uint64_t *d_sample = scratch + 1, *d_cuts = d_sample + m;
+    unsigned long long* d_counts = reinterpret_cast<unsigned long long*>(d_cuts + parts);
+    k_pack_reads<<<blocks_for(R * 32, 256), 256, 0, stream>>>(v, packed, reinterpret_cast<uint32_t*>(scratch));
+    if (d_off) k_key_sample<true><<<blocks_for(m, 256), 256, 0, stream>>>(v, packed, n, m, d_sample);
+    else k_key_sample<false><<<blocks_for(m, 256), 256, 0, stream>>>(v, packed, n, m, d_sample);
+    *launches += 2;
+    std::vector<uint64_t> h(size_t(1 + m));
+    if ((e = cudaMemcpyAsync(h.data(), scratch, h.size() * 8, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return done(e);
+    if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return done(e);
+    if (uint32_t(h[0])) return done(cudaErrorInvalidValue);
+    std::sort(h.begin() + 1, h.end());
+    key_lo[0] = 0;
+    for (uint32_t i = 1; i < parts; ++i) {
+        const uint64_t q = h[size_t(1 + uint64_t(i) * m / parts)];
+        if (key_lo[i - 1] == ~uint64_t(0)) return done(cudaErrorInvalidConfiguration);
+        key_lo[i] = q > key_lo[i - 1] ? q : key_lo[i - 1] + 1;
+    }
+    if ((e = cudaMemcpyAsync(d_cuts, key_lo, size_t(parts) * 8, cudaMemcpyHostToDevice, stream)) != cudaSuccess) return done(e);
+    if (d_off) k_cut_count<true><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n, d_cuts, parts, d_counts);
+    else k_cut_count<false><<<unsigned(n_chunks), SEL_THREADS, 0, stream>>>(v, packed, n, d_cuts, parts, d_counts);
+    *launches += 1;
+    std::vector<uint64_t> cnt(parts);
+    if ((e = cudaMemcpyAsync(cnt.data(), d_counts, size_t(parts) * 8, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return done(e);
+    if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return done(e);
+    position[0] = 0;
+    for (uint32_t i = 0; i < parts; ++i) position[i + 1] = position[i] + cnt[i];
+    return done(position[parts] == n ? cudaSuccess : cudaErrorUnknown);
+}
+
+cudaError_t launch_pair_lcp(const uint8_t* bases, const uint64_t* off, const uint64_t* pairs, uint32_t n_pairs, uint32_t lcp_mask,
+                            uint32_t* lcp, cudaStream_t stream) {
+    if (n_pairs == 0) return cudaSuccess;
+    k_pair_lcp<<<blocks_for(uint64_t(n_pairs) * 32, 256), 256, 0, stream>>>(bases, off, pairs, n_pairs, lcp_mask, lcp);
+    return cudaGetLastError();
 }
 
 }  // namespace e2s

@@ -46,8 +46,9 @@ static int upload_offsets(e2s_ctx* c, const char* who, const uint64_t* off, uint
 // The whole index in one call, arguments checked.  d_off == nullptr: n_reads reads of `longest` bases; else n_reads + 1 DEVICE
 // offsets (off: the same in host memory), longest = the longest read.
 static int build_whole(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* d_off, const uint64_t* off, uint64_t n_reads,
-                       uint32_t longest, uint64_t total, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, FieldMask mask) {
-    const cudaError_t e = build_egsa(d_reads, d_off, off, n_reads, longest, total, d_lcp, d_text, d_suff, d_bwt, c->stream, &c->launches, mask);
+                       uint32_t longest, uint64_t total, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, FieldMask mask,
+                       uint64_t* ends = nullptr) {
+    const cudaError_t e = build_egsa(d_reads, d_off, off, n_reads, longest, total, d_lcp, d_text, d_suff, d_bwt, c->stream, &c->launches, mask, ends);
     if (e == cudaErrorMemoryAllocation) {
         cudaGetLastError();
         return fail(c, E2S_ERR_NOMEM, std::string(who) + ": scratch buffers (24.5 bytes per suffix with 32-bit suffix ids, 32.5 with 64-bit ids)");
@@ -93,12 +94,12 @@ static int build_egsa_common(e2s_ctx* c, const char* who, const uint8_t* d_reads
 static int build_range_common(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* d_off, uint64_t n_reads, uint32_t read_len,
                               uint64_t total, uint64_t key_lo, uint64_t key_hi, uint32_t before_text, uint32_t before_suff, uint64_t capacity,
                               uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, uint64_t* n_records, uint64_t* first_position,
-                              FieldMask mask = FieldMask(), uint64_t* last = nullptr) {
+                              FieldMask mask = FieldMask(), uint64_t* ends = nullptr) {
     const uint64_t before = before_text == 0xffffffffu ? ~uint64_t(0) : (uint64_t(before_text) << 32) | before_suff;
     *n_records = 0;
     *first_position = 0;
     cudaError_t e = build_egsa_range(d_reads, d_off, n_reads, read_len, total, key_lo, key_hi, before, capacity, d_lcp, d_text, d_suff, d_bwt,
-                                     n_records, first_position, c->stream, &c->launches, mask, last);
+                                     n_records, first_position, c->stream, &c->launches, mask, ends);
     if (e == cudaErrorMemoryAllocation) {
         cudaGetLastError();
         return fail(c, E2S_ERR_NOMEM, std::string(who) + ": scratch buffers (24.5 / 32.5 bytes per suffix of the range)");
@@ -152,87 +153,107 @@ struct IndexArraysDev {
 };
 
 // Where the builder puts the index: host arrays (each key range is copied there from device buffers of one range), or device
-// arrays of the whole index written in place (a shard's: `written` then runs on the positions [at, at + m) just written).
+// arrays written in place (a shard's: `written` then runs on the local positions [l, l + m) just written).  Either way the arrays
+// start at the index position of the first record the build writes.
 struct IndexDest {
     uint32_t *lcp, *text, *suff;
     uint8_t* bwt;
     bool device;
     FieldMask mask;
-    std::function<int(uint64_t at, uint64_t m)> written;
+    std::function<int(uint64_t l, uint64_t m)> written;
 };
 
-// An index that does not fit one call's device memory (scratch 24.5 / 32.5 B per suffix, + 13 B of outputs when they go to the
-// host): the index key range by key range (build_range_common), each range's records to their place in `out`.  d_off == nullptr:
-// n_reads reads of read_len bases; else DEVICE offsets (uploaded once for all ranges), read_len = the longest read.  A range that
-// turns out to hold more than `cap` records is cut in two.
+// The records of the key interval [lo, hi) (hi = 0: to the end of the key space) that do not fit one call's device memory (scratch
+// 24.5 / 32.5 B per suffix, + 13 B of outputs when they go to the host): sub-range by sub-range (build_range_common), each one's
+// records to their place in `out`.  They must be the n_range positions of the index from position at0.  d_off == nullptr: n_reads
+// reads of read_len bases; else DEVICE offsets, read_len = the longest read.  A sub-range that turns out to hold more than `cap`
+// records is cut in two.  ends (not null): the first and last record at full width.  E2S_ERR_ARG: the interval's records are not
+// those positions.
 static int build_egsa_ranges(e2s_ctx* c, const char* who, const uint8_t* d_reads, const uint64_t* d_off, uint64_t n_reads, uint32_t read_len,
-                             uint64_t total, uint64_t cap, const IndexDest& out) {
+                             uint64_t total, uint64_t lo0, uint64_t hi0, uint64_t at0, uint64_t n_range, uint64_t cap, const IndexDest& out,
+                             uint64_t* ends) {
     const char* range_who = d_off ? "e2s_build_egsa_ragged_range_dev" : "e2s_build_egsa_range_dev";
-    const uint64_t n = total + n_reads;
+    const uint64_t end = at0 + n_range;
     IndexArraysDev d;
     if (!out.device && d.alloc(cap) != cudaSuccess) return fail(c, E2S_ERR_NOMEM, std::string(who) + ": device buffers of one key range");
-    // ranges as (lo, hi) with hi = 0 for "to the end of the key space", processed in key order from a stack
-    uint64_t parts = (n + cap - 1) / cap;
-    parts += parts / 4 + 1;
+    // sub-ranges as (lo, hi) with hi = 0 for "to the end of the key space", processed in key order from a stack
+    uint64_t parts = 1;
+    if (n_range > cap) {
+        parts = (n_range + cap - 1) / cap;
+        parts += parts / 4 + 1;
+    }
+    using u128 = unsigned __int128;
+    const u128 width0 = (hi0 == 0 ? u128(1) << 64 : u128(hi0)) - lo0;
     std::vector<std::pair<uint64_t, uint64_t>> todo;
     for (uint64_t i = parts; i-- > 0;) {
-        const uint64_t lo = uint64_t((static_cast<unsigned __int128>(i) << 64) / parts);
-        const uint64_t hi = i + 1 == parts ? 0 : uint64_t((static_cast<unsigned __int128>(i + 1) << 64) / parts);
-        if (hi == 0 || hi > lo) todo.emplace_back(lo, hi);
+        const uint64_t lo = lo0 + uint64_t(width0 * i / parts);
+        const uint64_t hi = i + 1 == parts ? hi0 : lo0 + uint64_t(width0 * (i + 1) / parts);
+        if (i + 1 == parts || hi != lo) todo.emplace_back(lo, hi);
     }
-    uint64_t at = 0;
+    uint64_t at = at0;
     uint64_t before = ~uint64_t(0);  // the last record so far, text << 32 | suff at full width
     int rc = E2S_OK;
+    auto mismatch = [&]() {
+        return fail(c, E2S_ERR_ARG, std::string(who) + ": the key range's records are not index positions [" + std::to_string(at0) + ", " +
+                                        std::to_string(end) + ")");
+    };
     while (!todo.empty() && rc == E2S_OK) {
         const auto [lo, hi] = todo.back();
         todo.pop_back();
-        uint64_t m = 0, first = 0, last = before;
-        // (in place: a range never writes past the end of the index)
-        const uint64_t room = out.device && n - at < cap ? n - at : cap;
+        uint64_t m = 0, first = 0, got[2] = {before, before};
+        // (in place: a range never writes past the end of the arrays)
+        const uint64_t room = out.device && end - at < cap ? end - at : cap;
+        const uint64_t l = at - at0;
         rc = build_range_common(c, range_who, d_reads, d_off, n_reads, read_len, total, lo, hi, uint32_t(before >> 32), uint32_t(before), room,
-                                out.device ? out.lcp + at : d.lcp, out.device ? out.text + at : d.text, out.device ? out.suff + at : d.suff,
-                                out.device ? out.bwt + at : d.bwt, &m, &first, out.mask, &last);
+                                out.device ? out.lcp + l : d.lcp, out.device ? out.text + l : d.text, out.device ? out.suff + l : d.suff,
+                                out.device ? out.bwt + l : d.bwt, &m, &first, out.mask, got);
         if (rc == E2S_ERR_ARG && m > room) {  // too many records for the buffers: two halves (a single key value cannot be cut)
-            const uint64_t width = hi - lo;  // (mod 2^64: right for hi = 0 as long as lo > 0 or the range is not the whole space)
-            if (width == 1 || (lo == 0 && hi == 0)) {
+            if (m > end - at) {
+                rc = mismatch();
+                break;
+            }
+            const u128 width = (hi == 0 ? u128(1) << 64 : u128(hi)) - lo;
+            if (width == 1) {
                 rc = fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": one 32-symbol prefix is shared by more suffixes than fit the device");
                 break;
             }
-            const uint64_t mid = lo + (width >> 1);
+            const uint64_t mid = lo + uint64_t(width >> 1);
             todo.emplace_back(mid, hi);
             todo.emplace_back(lo, mid);
             rc = E2S_OK;
             continue;
         }
         if (rc != E2S_OK) break;
-        if (first != at || at + m > n) {
-            rc = fail(c, E2S_ERR_STATE, std::string(who) + ": key ranges do not tile the index");
+        if (first != at || m > end - at) {
+            rc = mismatch();
             break;
         }
         if (m) {
             if (out.device) {
-                rc = out.written(at, m);
+                rc = out.written(l, m);
             } else {
-                const cudaError_t e = d.to_host(out.lcp + at, out.text + at, out.suff + at, out.bwt + at, m, c->stream);
+                const cudaError_t e = d.to_host(out.lcp + l, out.text + l, out.suff + l, out.bwt + l, m, c->stream);
                 if (e != cudaSuccess) rc = cuda_fail(c, e, "D2H index arrays of a key range");
             }
+            if (ends && at == at0) ends[0] = got[0];
             at += m;
-            before = last;
+            before = got[1];
         }
     }
-    if (rc == E2S_OK && at != n) rc = fail(c, E2S_ERR_STATE, std::string(who) + ": key ranges do not cover the index");
+    if (rc == E2S_OK && at != end) rc = mismatch();
+    if (rc == E2S_OK && ends) ends[1] = before;
     d.release();
     return rc;
 }
 
-// Does the whole index of `total` bases in n_reads reads (the longest: `longest` bases) fit one call on the device as it is now, the
-// reads already resident?  *cap = 0: build it whole; else the records per key range.  Scratch: 24.5 B per suffix with 32-bit suffix
-// ids, 32.5 with 64-bit ids (equal lengths: n < 2^32; ragged: R << shift, shift = the bits of the longest read's length + 1), plus
-// out_bytes per suffix when the outputs are device buffers of the call; packed reads and slack (half a byte per base), and for ragged
-// reads the 2 extra packed words and the device offset of every read.  0.92 of the free memory may be used.
-// E2S_BUILD_RANGE_RECORDS=<cap> forces key ranges (tests).
-static int range_records(e2s_ctx* c, const char* who, uint64_t total, uint64_t n_reads, bool ragged, uint32_t longest, uint64_t out_bytes,
-                         const char* advice, uint64_t* cap) {
+// Do the n_sort suffixes of the index of `total` bases in n_reads reads (the longest: `longest` bases) -- all of them, or one shard's
+// key range -- fit one call on the device as it is now, the reads already resident?  *cap = 0: build them in one call; else the
+// records per key range.  Scratch: 24.5 B per suffix sorted with 32-bit suffix ids, 32.5 with 64-bit ids (equal lengths: n < 2^32;
+// ragged: R << shift, shift = the bits of the longest read's length + 1), plus out_bytes per suffix when the outputs are device buffers
+// of the call; packed reads and slack (half a byte per base), and for ragged reads the 2 extra packed words and the device offset of
+// every read.  0.92 of the free memory may be used.  E2S_BUILD_RANGE_RECORDS=<cap> forces key ranges (tests).
+static int range_records(e2s_ctx* c, const char* who, uint64_t total, uint64_t n_reads, uint64_t n_sort, bool ragged, uint32_t longest,
+                         uint64_t out_bytes, const char* advice, uint64_t* cap) {
     const uint64_t n = total + n_reads;
     bool ids64 = n > 0xffffffffull;
     if (ragged) {
@@ -250,7 +271,7 @@ static int range_records(e2s_ctx* c, const char* who, uint64_t total, uint64_t n
     cudaMemGetInfo(&free_b, &total_b);
     const uint64_t per_suffix = out_bytes + (ids64 ? 33 : 25);
     const double fixed = double(total) / 2 + (ragged ? 24.0 * double(n_reads) : 0.0);
-    if (double(n) * double(per_suffix) + fixed <= 0.92 * double(free_b)) return E2S_OK;
+    if (double(n_sort) * double(per_suffix) + fixed <= 0.92 * double(free_b)) return E2S_OK;
     const double room = 0.92 * double(free_b) - fixed - double(n) / 512;
     *cap = room > 0 ? uint64_t(room / double(per_suffix)) : 0;
     if (*cap < 4096) return fail(c, E2S_ERR_NOMEM, std::string(who) + ": not even one key range of the index fits the device" + advice);
@@ -276,7 +297,7 @@ static int build_egsa_host(e2s_ctx* c, const char* who, const uint8_t* reads, co
         return fail(c, E2S_ERR_NOMEM, std::string(who) + ": the reads on the device");
     }
     uint64_t cap = 0;
-    if (int rc = range_records(c, who, total, n_reads, off != nullptr, longest, 13, "", &cap)) {
+    if (int rc = range_records(c, who, total, n_reads, n, off != nullptr, longest, 13, "", &cap)) {
         cudaFree(d_reads);
         return rc;
     }
@@ -286,7 +307,8 @@ static int build_egsa_host(e2s_ctx* c, const char* who, const uint8_t* reads, co
         if (off) rc = upload_offsets(c, who, off, n_reads, &d_off);
         if (rc == E2S_OK) {
             e = cudaMemcpyAsync(d_reads, reads, total, cudaMemcpyHostToDevice, c->stream);
-            rc = e == cudaSuccess ? build_egsa_ranges(c, who, d_reads, d_off, n_reads, longest, total, cap, IndexDest{lcp, text, suff, bwt, false, FieldMask(), nullptr})
+            rc = e == cudaSuccess ? build_egsa_ranges(c, who, d_reads, d_off, n_reads, longest, total, 0, 0, 0, n, cap,
+                                                      IndexDest{lcp, text, suff, bwt, false, FieldMask(), nullptr}, nullptr)
                                   : cuda_fail(c, e, "H2D reads");
         }
         cudaStreamSynchronize(c->stream);
@@ -378,16 +400,17 @@ int e2s_build_egsa_ragged(e2s_ctx* c, const uint8_t* bases, const uint64_t* off,
     return build_egsa_host(c, "e2s_build_egsa_ragged", bases, off, n_reads, 0, lcp, text, suff, bwt);
 }
 
-// The index of the staged reads written straight into a resident shard's arrays, each field kept at its .gesa width, then the narrow
-// copies of what was written.  The staged reads (and, for ragged reads, their staged device offsets) are the builder's input.
-int e2s_shard_build_egsa(e2s_shard* s, const uint64_t* off, int x, int y, int z) {
+// The records of the key range [key_lo, key_hi) of the staged reads' index written straight into a resident shard's arrays, each field
+// kept at its .gesa width, then the narrow copies of what was written.  The staged reads (and, for ragged reads, their staged device
+// offsets) are the builder's input.  The whole key space (0, 0) on a shard of the whole index is one build when its scratch fits.
+int e2s_shard_build_egsa_range(e2s_shard* s, const uint64_t* off, uint64_t key_lo, uint64_t key_hi, int x, int y, int z) {
     const char* who = "e2s_shard_build_egsa";
     if (!s || !off) return fail(s ? s->ctx : nullptr, E2S_ERR_ARG, std::string(who) + ": NULL argument");
     e2s_ctx* c = s->ctx;
     int rc;
     if ((rc = check_field_sizes(c, {x, y, z}))) return rc;
-    if (s->chunked || s->global_off != 0 || s->n_local != s->n_global)
-        return fail(c, E2S_ERR_ARG, std::string(who) + ": needs a resident shard that holds the whole eBWT (not chunked, global_off = 0)");
+    if (s->chunked) return fail(c, E2S_ERR_ARG, std::string(who) + ": needs a resident shard (not chunked)");
+    if (key_hi != 0 && key_hi <= key_lo) return fail(c, E2S_ERR_ARG, std::string(who) + ": empty key range");
     if (!c->d_bases || !c->d_off || c->n_reads == 0) return fail(c, E2S_ERR_STATE, std::string(who) + ": stage the reads first (e2s_reads_stage)");
     const uint64_t n_reads = c->n_reads;
     if (off[n_reads] != c->n_bases) return fail(c, E2S_ERR_ARG, std::string(who) + ": `off` does not describe the staged reads");
@@ -395,29 +418,82 @@ int e2s_shard_build_egsa(e2s_shard* s, const uint64_t* off, int x, int y, int z)
     uint32_t longest = 0;
     if ((rc = check_offsets(c, who, off, n_reads, &longest))) return rc;
     const uint64_t total = off[n_reads], n = total + n_reads;
-    if (s->n_local != n) return fail(c, E2S_ERR_ARG, std::string(who) + ": the shard must hold off[n_reads] + n_reads positions");
+    if (s->n_global != n) return fail(c, E2S_ERR_ARG, std::string(who) + ": the shard's n_global must be off[n_reads] + n_reads");
+    const bool whole = key_lo == 0 && key_hi == 0;
+    if (whole && s->n_local != n) return fail(c, E2S_ERR_ARG, std::string(who) + ": the whole key space needs a shard of the whole eBWT");
     const bool ragged = total != n_reads * uint64_t(longest);  // (every read has `longest` bases exactly when the sum says so)
     CU(c, cudaSetDevice(c->device));
     uint64_t cap = 0;
-    if ((rc = range_records(c, who, total, n_reads, ragged, longest, 0,
-                            " next to the shard; build the index file with build_gesa and stream it (ebwt2clust / clust2snp, "
-                            "e2s_pipeline_host) -- a chunked or multi-GPU build from reads is not supported",
+    if ((rc = range_records(c, who, total, n_reads, s->n_local, ragged, longest, 0,
+                            " next to the shard; split the index over more shards, or build the index file with build_gesa and stream "
+                            "it (ebwt2clust / clust2snp, e2s_pipeline_host)",
                             &cap)))
         return rc;
     auto mask = [](int w) { return w >= 4 ? ~0u : (1u << (8 * w)) - 1u; };
     const FieldMask fm{mask(x), mask(y), mask(z)};
-    auto written = [&](uint64_t at, uint64_t m) -> int {
-        CU(c, derive_loaded(s, int64_t(at), m, true, true));
+    auto written = [&](uint64_t l, uint64_t m) -> int {
+        CU(c, derive_loaded(s, int64_t(l), m, true, true));
         ++c->launches;
         return E2S_OK;
     };
     s->sealed = false;
+    s->ends_known = false;
     s->lay_x = x; s->lay_y = y; s->lay_z = z; s->lay_bcr = 0;
     CU(c, cudaMemsetAsync(s->d_seal_flag, 0, 4, c->stream));  // every position is rewritten: the old verdict goes
     const uint64_t* d_off = ragged ? c->d_off : nullptr;
-    if (cap) return build_egsa_ranges(c, who, c->d_bases, d_off, n_reads, longest, total, cap, IndexDest{s->lcp, s->text, s->suff, s->bwt, true, fm, written});
-    if ((rc = build_whole(c, who, c->d_bases, d_off, off, n_reads, longest, total, s->lcp, s->text, s->suff, s->bwt, fm))) return rc;
-    return written(0, n);
+    if (whole && !cap) {
+        if ((rc = build_whole(c, who, c->d_bases, d_off, off, n_reads, longest, total, s->lcp, s->text, s->suff, s->bwt, fm, s->ends))) return rc;
+        rc = written(0, n);
+    } else {
+        rc = build_egsa_ranges(c, who, c->d_bases, d_off, n_reads, longest, total, key_lo, key_hi, s->global_off, s->n_local, cap ? cap : s->n_local,
+                               IndexDest{s->lcp, s->text, s->suff, s->bwt, true, fm, written}, s->ends);
+    }
+    s->ends_known = rc == E2S_OK;
+    return rc;
+}
+
+int e2s_shard_build_egsa(e2s_shard* s, const uint64_t* off, int x, int y, int z) { return e2s_shard_build_egsa_range(s, off, 0, 0, x, y, z); }
+
+// Cuts of the key space into `parts` shards of the staged reads' index (the builder's key words and slot map, a fixed-stride sample).
+int e2s_reads_key_cuts(e2s_ctx* c, const uint64_t* off, int parts, uint64_t* key_lo, uint64_t* position) {
+    const char* who = "e2s_reads_key_cuts";
+    if (!c || !off || !key_lo || !position) return fail(c, E2S_ERR_ARG, std::string(who) + ": NULL argument");
+    if (parts < 1) return fail(c, E2S_ERR_ARG, std::string(who) + ": parts must be at least 1");
+    if (!c->d_bases || !c->d_off || c->n_reads == 0) return fail(c, E2S_ERR_STATE, std::string(who) + ": stage the reads first (e2s_reads_stage)");
+    const uint64_t n_reads = c->n_reads;
+    if (off[n_reads] != c->n_bases) return fail(c, E2S_ERR_ARG, std::string(who) + ": `off` does not describe the staged reads");
+    uint32_t longest = 0;
+    int rc;
+    if ((rc = check_offsets(c, who, off, n_reads, &longest))) return rc;
+    const uint64_t total = off[n_reads], n = total + n_reads;
+    if (uint64_t(parts) * 2 > n) return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": too many shards for this collection (each needs 2 positions)");
+    if (parts > 1024) return fail(c, E2S_ERR_ARG, std::string(who) + ": at most 1024 parts");
+    if (parts == 1) {  // the whole key space: nothing to sample or count
+        key_lo[0] = 0;
+        position[0] = 0;
+        position[1] = n;
+        return E2S_OK;
+    }
+    const bool ragged = total != n_reads * uint64_t(longest);
+    CU(c, cudaSetDevice(c->device));
+    const cudaError_t e = key_cuts(c->d_bases, ragged ? c->d_off : nullptr, n_reads, longest, total, uint32_t(parts), key_lo, position, c->stream,
+                                   &c->launches);
+    if (e == cudaErrorMemoryAllocation) {
+        cudaGetLastError();
+        return fail(c, E2S_ERR_NOMEM, std::string(who) + ": the packed reads (a quarter byte per base)");
+    }
+    if (e == cudaErrorInvalidValue) {
+        cudaGetLastError();
+        return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": a read holds a base outside ACGT/acgt");
+    }
+    if (e != cudaErrorInvalidConfiguration && e != cudaSuccess) return cuda_fail(c, e, "key_cuts");
+    for (int i = 0; i < parts && e == cudaSuccess; ++i)
+        if (position[i + 1] - position[i] < 2) {
+            return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": too many shards for this collection (a key range holds fewer than 2 "
+                                                                   "positions; one key value cannot be split)");
+        }
+    if (e != cudaSuccess) return fail(c, E2S_ERR_UNSUPPORTED, std::string(who) + ": too many shards for this collection (the cuts cannot increase)");
+    return E2S_OK;
 }
 
 }  // extern "C"

@@ -189,6 +189,14 @@ int e2s_ctx_kernel_time(e2s_ctx* c, int kernel, double* total_ms, uint64_t* laun
     return E2S_OK;
 }
 
+int e2s_device_count(int* count) {
+    if (!count) return fail(nullptr, E2S_ERR_ARG, "count == NULL");
+    *count = 0;
+    const cudaError_t e = cudaGetDeviceCount(count);
+    if (e != cudaSuccess) return cuda_fail(nullptr, e, "cudaGetDeviceCount");
+    return E2S_OK;
+}
+
 int e2s_ctx_mem_info(e2s_ctx* c, uint64_t* free_bytes, uint64_t* total_bytes) {
     if (!c) return fail(nullptr, E2S_ERR_ARG, "ctx == NULL");
     CU(c, cudaSetDevice(c->device));

@@ -163,6 +163,10 @@ struct e2s_shard {
                                  // the 4-byte stream then
     bool sealed = false;
     int lay_x = 4, lay_y = 4, lay_z = 4, lay_bcr = 0;  // layout of the index files (phantom record only)
+    // built from the reads (e2s_shard_build_egsa_range): its first and last record as text << 32 | suff at full width (the stored
+    // fields may be truncated), for the halo row
+    uint64_t ends[2] = {0, 0};
+    bool ends_known = false;
     // record list
     uint64_t* d_start = nullptr;
     uint16_t* d_len = nullptr;

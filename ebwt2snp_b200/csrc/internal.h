@@ -228,15 +228,27 @@ struct FieldMask {
 // cudaErrorInvalidValue = a base outside ACGT / acgt; cudaErrorInvalidConfiguration = a read of 65536 bases or more.
 cudaError_t build_egsa(const uint8_t* d_reads, const uint64_t* d_off, const uint64_t* h_off, uint64_t R, uint32_t L, uint64_t total_bases,
                        uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt, cudaStream_t stream, uint64_t* launches,
-                       FieldMask mask = FieldMask());
+                       FieldMask mask = FieldMask(), uint64_t* ends = nullptr);
 
 // one key range of the index (see build_egsa.cu); reads as for build_egsa (d_off == nullptr: R reads of L bases), no host offsets needed;
-// cudaErrorInvalidPitchValue = more than `cap` records (*n_out says how many).  *last_out (when not null, and the range is not empty) =
-// the range's last record as text << 32 | suff at full width: the `before` of the next range whatever the mask
+// cudaErrorInvalidPitchValue = more than `cap` records (*n_out says how many).  ends (of both builders; when not null, and the range is
+// not empty) = the first and the last record written as text << 32 | suff at full width, whatever the mask: the `before` of the next
+// range, and the ends a shard's halo row carries
 cudaError_t build_egsa_range(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint64_t key_lo,
                              uint64_t key_hi, uint64_t before, uint64_t cap, uint32_t* d_lcp, uint32_t* d_text, uint32_t* d_suff, uint8_t* d_bwt,
                              uint64_t* n_out, uint64_t* first_out, cudaStream_t stream, uint64_t* launches, FieldMask mask = FieldMask(),
-                             uint64_t* last_out = nullptr);
+                             uint64_t* ends = nullptr);
+
+// Cuts of the key space into `parts` ranges of about equal size (see build_egsa.cu): key_lo[0] = 0 < key_lo[1] < ... (the first key
+// words, as for build_egsa_range), position[i] = the index position of cut i, position[parts] = total_bases + R.  Deterministic: a
+// fixed-stride sample of the suffix slots, no RNG.  Reads as for build_egsa_range.  cudaErrorInvalidValue = a base outside ACGT / acgt.
+cudaError_t key_cuts(const uint8_t* d_reads, const uint64_t* d_off, uint64_t R, uint32_t L, uint64_t total_bases, uint32_t parts,
+                     uint64_t* key_lo, uint64_t* position, cudaStream_t stream, uint64_t* launches);
+
+// lcp[j] = the builder's LCP (capped at the shorter suffix, never across a terminator) of the suffixes pairs[2 j] and pairs[2 j + 1]
+// (text << 32 | suff, device memory) of the reads `bases` / R + 1 DEVICE offsets `off`, masked with lcp_mask; one launch, no sync
+cudaError_t launch_pair_lcp(const uint8_t* bases, const uint64_t* off, const uint64_t* pairs, uint32_t n_pairs, uint32_t lcp_mask,
+                            uint32_t* lcp, cudaStream_t stream);
 
 // ---- phase 2 -----------------------------------------------------------------------------------
 struct SnpDev {  // device counters of one e2s_find_events

@@ -570,6 +570,125 @@ int e2s_shard_seal(e2s_shard* s) {
     return E2S_OK;
 }
 
+// ---- halos of shards built from the reads --------------------------------------------------------------------------------
+// A halo row: n_local, global_off, the first and the last record's ids (text << 32 | suff at full width), then HALO_ROW_RECS records
+// of 2 words (lcp | text << 32, suff | bwt << 32) as stored: the shard's last HALO_LAST records, then its first min(HALO_FIRST,
+// n_local) (zeros past n_local).
+constexpr uint64_t HALO_LAST = 2, HALO_FIRST = MAX_C_LEN + 1, HALO_HEAD = 4;
+constexpr uint64_t HALO_ROW_WORDS = HALO_HEAD + 2 * (HALO_LAST + HALO_FIRST);
+
+uint64_t e2s_shard_halo_row_words(void) { return HALO_ROW_WORDS; }
+
+int e2s_shard_halo_row(e2s_shard* s, uint64_t* row) {
+    if (!s || !row) return fail(s ? s->ctx : nullptr, E2S_ERR_ARG, "e2s_shard_halo_row: NULL argument");
+    e2s_ctx* c = s->ctx;
+    if (s->chunked || !s->ends_known) return fail(c, E2S_ERR_STATE, "e2s_shard_halo_row: build the shard from the reads first (e2s_shard_build_egsa_range)");
+    CU(c, cudaSetDevice(c->device));
+    const uint64_t nf = s->n_local < HALO_FIRST ? s->n_local : HALO_FIRST, nr = HALO_LAST + HALO_FIRST;
+    std::vector<uint32_t> lcp(nr, 0), text(nr, 0), suff(nr, 0);
+    std::vector<uint8_t> bwt(nr, 0);
+    const int64_t at[2] = {int64_t(s->n_local - HALO_LAST), 0};
+    const uint64_t cnt[2] = {HALO_LAST, nf}, to[2] = {0, HALO_LAST};
+    for (int q = 0; q < 2; ++q) {
+        CU(c, cudaMemcpyAsync(lcp.data() + to[q], s->lcp + at[q], cnt[q] * 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaMemcpyAsync(text.data() + to[q], s->text + at[q], cnt[q] * 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaMemcpyAsync(suff.data() + to[q], s->suff + at[q], cnt[q] * 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaMemcpyAsync(bwt.data() + to[q], s->bwt + at[q], cnt[q], cudaMemcpyDeviceToHost, c->stream));
+    }
+    CU(c, cudaStreamSynchronize(c->stream));
+    row[0] = s->n_local;
+    row[1] = s->global_off;
+    row[2] = s->ends[0];
+    row[3] = s->ends[1];
+    for (uint64_t i = 0; i < nr; ++i) {
+        row[HALO_HEAD + 2 * i] = uint64_t(lcp[i]) | (uint64_t(text[i]) << 32);
+        row[HALO_HEAD + 2 * i + 1] = uint64_t(suff[i]) | (uint64_t(bwt[i]) << 32);
+    }
+    return E2S_OK;
+}
+
+// Every shard's halo row in shard order -> this shard's left halo (the previous shard's last 2 records), right halo (the first
+// records of the shards after it, up to 151 or the end of the eBWT) and own position 0, with every record that starts a shard
+// given its boundary LCP: LCP(last suffix of shard g - 1, first suffix of shard g), the builder's rule on the staged reads (one
+// k_pair_lcp launch), masked to the lcp width.  Written through the SoA load, which re-derives the narrow copies.
+int e2s_shard_halo_apply(e2s_shard* s, const uint64_t* rows, int n_shards, int my) {
+    const char* who = "e2s_shard_halo_apply";
+    if (!s || !rows) return fail(s ? s->ctx : nullptr, E2S_ERR_ARG, std::string(who) + ": NULL argument");
+    e2s_ctx* c = s->ctx;
+    if (n_shards < 1 || my < 0 || my >= n_shards) return fail(c, E2S_ERR_ARG, std::string(who) + ": need 0 <= my < n_shards");
+    if (s->chunked || !s->ends_known) return fail(c, E2S_ERR_STATE, std::string(who) + ": build the shard from the reads first (e2s_shard_build_egsa_range)");
+    if (!c->d_bases || !c->d_off || c->n_reads == 0) return fail(c, E2S_ERR_STATE, std::string(who) + ": stage the reads first (e2s_reads_stage)");
+    auto row = [&](int g) { return rows + size_t(g) * HALO_ROW_WORDS; };
+    uint64_t at = 0;
+    for (int g = 0; g < n_shards; ++g) {
+        const uint64_t* r = row(g);
+        if (r[1] != at || r[0] < 2 || r[0] > s->n_global - at)
+            return fail(c, E2S_ERR_ARG, std::string(who) + ": the rows do not tile the eBWT (shard " + std::to_string(g) + ")");
+        if ((r[2] >> 32) >= c->n_reads || (r[3] >> 32) >= c->n_reads)
+            return fail(c, E2S_ERR_ARG, std::string(who) + ": a row names a read that is not staged (shard " + std::to_string(g) + ")");
+        at += r[0];
+    }
+    if (at != s->n_global) return fail(c, E2S_ERR_ARG, std::string(who) + ": the rows do not cover the eBWT");
+    const uint64_t* mine = row(my);
+    if (mine[0] != s->n_local || mine[1] != s->global_off || mine[2] != s->ends[0] || mine[3] != s->ends[1])
+        return fail(c, E2S_ERR_ARG, std::string(who) + ": row `my` is not this shard's");
+    CU(c, cudaSetDevice(c->device));
+    // the boundary LCPs: blcp[g - 1] for the first record of shard g >= 1
+    const uint32_t nb = uint32_t(n_shards - 1);
+    std::vector<uint32_t> blcp(nb);
+    if (nb) {
+        std::vector<uint64_t> pairs(2 * size_t(nb));
+        for (uint32_t g = 1; g <= nb; ++g) {
+            pairs[2 * (g - 1)] = row(int(g) - 1)[3];
+            pairs[2 * (g - 1) + 1] = row(int(g))[2];
+        }
+        uint64_t* d = nullptr;  // the pairs, then the LCPs
+        if (cudaMalloc(reinterpret_cast<void**>(&d), size_t(nb) * 20) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(c, E2S_ERR_NOMEM, std::string(who) + ": boundary pairs");
+        }
+        uint32_t* d_lcp = reinterpret_cast<uint32_t*>(d + 2 * size_t(nb));
+        const uint32_t mask = s->lay_x >= 4 ? ~0u : (1u << (8 * s->lay_x)) - 1u;
+        cudaError_t e = cudaMemcpyAsync(d, pairs.data(), size_t(nb) * 16, cudaMemcpyHostToDevice, c->stream);
+        if (e == cudaSuccess) e = launch_pair_lcp(c->d_bases, c->d_off, d, nb, mask, d_lcp, c->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(blcp.data(), d_lcp, size_t(nb) * 4, cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        cudaFree(d);
+        ++c->launches;
+        if (e != cudaSuccess) return cuda_fail(c, e, "boundary LCPs");
+    }
+    // the records to write, in global order: [global_off - 2, global_off + 1) when my > 0, then the right halo
+    std::vector<uint32_t> lcp, text, suff;
+    std::vector<uint8_t> bwt;
+    auto put = [&](int g, uint64_t i) {  // record slot i of row g, its boundary LCP when it starts shard g >= 1
+        const uint64_t* r = row(g);
+        const uint64_t w0 = r[HALO_HEAD + 2 * i], w1 = r[HALO_HEAD + 2 * i + 1];
+        const bool starts = g > 0 && (i == HALO_LAST || (i == 0 && r[0] == HALO_LAST));
+        lcp.push_back(starts ? blcp[size_t(g) - 1] : uint32_t(w0));
+        text.push_back(uint32_t(w0 >> 32));
+        suff.push_back(uint32_t(w1));
+        bwt.push_back(uint8_t(w1 >> 32));
+    };
+    if (my > 0) {
+        for (uint64_t i = 0; i < HALO_LAST; ++i) put(my - 1, i);
+        put(my, HALO_LAST);
+        if (int rc = load_soa(s, lcp.data(), text.data(), suff.data(), bwt.data(), s->global_off - HALO_LAST, lcp.size(), cudaMemcpyHostToDevice))
+            return rc;
+        CU(c, cudaStreamSynchronize(c->stream));  // (the vectors are reused)
+    }
+    lcp.clear(); text.clear(); suff.clear(); bwt.clear();
+    for (int g = my + 1; g < n_shards && lcp.size() < HALO_FIRST; ++g) {
+        const uint64_t nf = row(g)[0] < HALO_FIRST ? row(g)[0] : HALO_FIRST;
+        for (uint64_t i = 0; i < nf && lcp.size() < HALO_FIRST; ++i) put(g, HALO_LAST + i);
+    }
+    if (!lcp.empty()) {
+        if (int rc = load_soa(s, lcp.data(), text.data(), suff.data(), bwt.data(), s->global_off + s->n_local, lcp.size(), cudaMemcpyHostToDevice))
+            return rc;
+        CU(c, cudaStreamSynchronize(c->stream));
+    }
+    return E2S_OK;
+}
+
 int e2s_shard_lcp_bytes_resident(const e2s_shard* s) { return s ? (s->sealed && s->lcpt_ok ? 1 : 4) : 0; }
 
 int e2s_reads_stage(e2s_ctx* c, const uint8_t* bases, const uint64_t* off, uint64_t n_reads) {

@@ -230,6 +230,24 @@ def exchange_halo(lcp, text, suff, bwt, device, group=None):
     return left, right
 
 
+def shard_from_reads(ctx: "api.Context", bases, off, x, y, z, device, group=None) -> "api.Shard":
+    """This rank's resident shard of ONE index built from all the reads (one process per rank, every rank passes the same reads):
+    the reads are staged, the key cuts computed locally (the same on every rank, no collective), this rank's key range built into
+    its shard, the halo rows exchanged with one all-gather and applied, and the shard sealed.  hot_path_step runs on it next."""
+    rank, world = _world(group)
+    bases = np.ascontiguousarray(bases, dtype=np.uint8).reshape(-1)
+    off = np.ascontiguousarray(off, dtype=np.uint64)
+    ctx.stage_reads(bases if bases.size else np.zeros(1, dtype=np.uint8), off)
+    key_lo, position = ctx.key_cuts(off, world)
+    lo, hi = int(position[rank]), int(position[rank + 1])
+    sh = ctx.shard(hi - lo, lo, int(position[world]))
+    sh.build_egsa_range(off, int(key_lo[rank]), int(key_lo[rank + 1]) if rank + 1 < world else 0, x, y, z)
+    rows = all_gather_words(sh.halo_row(), device, group)
+    sh.halo_apply(rows, rank)
+    sh.seal()
+    return sh
+
+
 def exchange_and_merge(summary: api.ClusterSummary, own: api.Stats, mcov_out, pval, device, group=None):
     """ONE collective between the phases: every rank contributes its scan summary and the length histogram of its OWN
     records; every rank then runs the (host, integer) merge for all shards, adds the records the merge creates at shard

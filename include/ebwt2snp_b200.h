@@ -64,6 +64,8 @@ int e2s_ctx_set_stream(e2s_ctx *ctx, void *cuda_stream);
 int e2s_ctx_synchronize(e2s_ctx *ctx);
 /* free / total device memory of the context's GPU right now (the CLIs choose between a resident and a chunked shard with it) */
 int e2s_ctx_mem_info(e2s_ctx *ctx, uint64_t *free_bytes, uint64_t *total_bytes);
+/* the CUDA devices this process sees */
+int e2s_device_count(int *count);
 /* number of kernel launches issued through this context so far (bench.py's gpu_launches) */
 uint64_t e2s_ctx_launch_count(const e2s_ctx *ctx);
 /* Per-kernel device time, measured with CUDA events recorded on the context's stream around the
@@ -172,6 +174,41 @@ int e2s_shard_lcp_bytes_resident(const e2s_shard *sh);
  * key range (E2S_BUILD_RANGE_RECORDS forces ranges).  A base outside ACGT, a read of 65536 bases or more: E2S_ERR_UNSUPPORTED;
  * not even one key range fits: E2S_ERR_NOMEM.  Call e2s_shard_seal afterwards. */
 int e2s_shard_build_egsa(e2s_shard *sh, const uint64_t *off, int x, int y, int z);
+
+/* ---- one index over several shards, each built from the reads for its own key range -------------------------------------
+ * Every shard (one per GPU, or several on one) stages all the reads, and
+ *   1. e2s_reads_key_cuts      the same cuts on every shard (deterministic, no collective);
+ *   2. e2s_shard_create        shard i: n_local = position[i+1] - position[i], global_off = position[i], n_global = position[parts];
+ *   3. e2s_shard_build_egsa_range  shard i's key range [key_lo[i], key_lo[i+1]) (key_hi = 0 on the last shard);
+ *   4. e2s_shard_halo_row      this shard's row, moved to every shard by the caller (host memory, torch.distributed, ...);
+ *   5. e2s_shard_halo_apply    all rows in shard order, then e2s_shard_seal;
+ * then the shards are what e2s_shard_load_* of the X.gesa of `build_gesa -x -y -z` with 2 positions of left and 151 of right halo
+ * would leave, and the multi-shard sequence (e2s_cluster_run, e2s_exchange_finish / e2s_pipeline_sharded, ...) runs on them. */
+
+/* Cuts of the key space (the builder's first key word: 32 symbols at 2 bits, A=0 C=1 G=2 T=3, first symbol most significant, zero
+ * padded) into `parts` (1..1024) ranges of about equal size for the reads staged on ctx (off = their n_reads + 1 HOST offsets).
+ * key_lo[0] = 0 < key_lo[1] < ... < key_lo[parts-1]; range i is [key_lo[i], key_lo[i+1]) (no upper bound for the last); position[i]
+ * = the exact index position of cut i, position[parts] = off[n_reads] + n_reads.  Cuts are quantiles of the first key words of a
+ * fixed-stride sample of the suffixes (no RNG: the same reads give the same cuts everywhere).  All suffixes of one key value stay in
+ * one range, so a heavy value (e.g. the terminators, key 0) makes its range larger.  A range of fewer than 2 positions:
+ * E2S_ERR_UNSUPPORTED (too many shards for this collection). */
+int e2s_reads_key_cuts(e2s_ctx *ctx, const uint64_t *off, int parts, uint64_t *key_lo, uint64_t *position);
+/* e2s_shard_build_egsa for the records of the key range [key_lo, key_hi) (key_hi = 0: no upper bound) only, written at the shard's
+ * local positions: they must be its global positions [global_off, global_off + n_local) of an eBWT of n_global = off[n_reads] +
+ * n_reads positions (E2S_ERR_ARG otherwise).  Resident shards only.  The range is built in one call when its scratch fits 0.92 of the
+ * free device memory, else sub-range by sub-range.  lcp of the shard's position 0 is left at 0 when global_off > 0: the halo step
+ * sets it.  e2s_shard_build_egsa is this call with key_lo = key_hi = 0 on a shard of the whole eBWT. */
+int e2s_shard_build_egsa_range(e2s_shard *sh, const uint64_t *off, uint64_t key_lo, uint64_t key_hi, int x, int y, int z);
+/* u64 words of one halo row: n_local, global_off, the ids (text << 32 | suff at full width) of the shard's first and last suffix,
+ * then its last 2 and its first min(151, n_local) records as stored */
+uint64_t e2s_shard_halo_row_words(void);
+/* this built shard's halo row (row: e2s_shard_halo_row_words() words) */
+int e2s_shard_halo_row(e2s_shard *sh, uint64_t *row);
+/* rows = every shard's halo row in shard order (they must tile the eBWT; row `my` is this shard's).  Writes the left halo (the
+ * previous shard's last 2 records), the right halo (the first records of the shards after this one, up to 151 or the end of the
+ * eBWT) and this shard's lcp[0], every record that starts a shard carrying the LCP of the last suffix of the shard before it and its
+ * own first suffix (the builder's rule on the staged reads, masked to the lcp width).  Call e2s_shard_seal afterwards. */
+int e2s_shard_halo_apply(e2s_shard *sh, const uint64_t *rows, int n_shards, int my);
 
 /* the read collection (FASTA bases), needed by e2s_find_events only: ref:clust2snp.cpp:147-212 */
 int e2s_reads_stage(e2s_ctx *ctx, const uint8_t *bases, const uint64_t *offsets /* n_reads+1 */, uint64_t n_reads);
