@@ -76,6 +76,9 @@ class PipelineResult(C.Structure):
                 ("reserved", C.c_int32), ("snp", SnpCounts), ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64)]
 
 
+# e2s_gather_fn: (user, rank, world, send, recv, words) -> 0 when recv holds every rank's row
+GATHER_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_uint64)
+
 # every symbol include/ebwt2snp_b200.h declares (tests/test_abi.py checks the list against the header)
 SYMBOLS = [
     "e2s_version", "e2s_ctx_create", "e2s_ctx_destroy", "e2s_last_error", "e2s_ctx_set_stream",
@@ -85,7 +88,7 @@ SYMBOLS = [
     "e2s_cluster_fetch", "e2s_cluster_fetch_packed", "e2s_clusters_stage_packed", "e2s_clusters_stage",
     "e2s_statistics", "e2s_statistics_finish", "e2s_exchange_finish", "e2s_snp_default_params", "e2s_find_events", "e2s_events_fetch",
     "e2s_events_format", "e2s_free", "e2s_pipeline_resident", "e2s_pipeline_host",
-    "e2s_comm_unique_id", "e2s_comm_create", "e2s_comm_destroy", "e2s_pipeline_sharded",
+    "e2s_comm_unique_id", "e2s_comm_create", "e2s_comm_create_gather", "e2s_comm_destroy", "e2s_pipeline_sharded",
     "e2s_exchange_row_words", "e2s_exchange_rows_finish",
     "e2s_pipeline_host_soa", "e2s_shard_host_gsa", "e2s_shard_load_lcp_bwt", "e2s_shard_load_bcr", "e2s_chunk_stage_clusters", "e2s_chunked_clusters_finish",
     "e2s_pipeline_host_sharded", "e2s_shard_build_egsa", "e2s_pipeline_reads", "e2s_shard_create_chunked", "e2s_shard_chunk_positions", "e2s_chunk_begin", "e2s_chunk_scan", "e2s_chunked_finish", "e2s_chunked_reset", "e2s_chunked_exchange",
@@ -166,6 +169,7 @@ def load_library():
     lib.e2s_exchange_rows_finish.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_int32, C.c_int, C.c_double,
                                              C.POINTER(ClusterMerged), C.POINTER(Stats)]
     lib.e2s_comm_create.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+    lib.e2s_comm_create_gather.argtypes = [C.c_void_p, C.c_int, C.c_int, GATHER_FN, C.c_void_p, C.POINTER(C.c_void_p)]
     lib.e2s_comm_destroy.argtypes = [C.c_void_p]
     lib.e2s_comm_destroy.restype = None
     lib.e2s_pipeline_sharded.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_int32, C.POINTER(SnpParams),
@@ -538,6 +542,27 @@ class Comm:
         h = C.c_void_p()
         ctx._ck(self.lib.e2s_comm_create(ctx.h, idb, rank, world, C.byref(h)))
         self.h, self.rank, self.world = h, rank, world
+
+    @classmethod
+    def gather(cls, ctx: Context, rank: int, world: int, fn):
+        """A communicator whose all-gather the caller performs (e2s_comm_create_gather): fn(rank, send, recv) gets this rank's
+        row (uint64 numpy view) and must fill recv ((world, row words) uint64 view) with every rank's row in rank order, on every
+        rank, and return True; anything else (or an exception) fails the library call.  Lets several ranks run as threads of one
+        process on one GPU."""
+        def trampoline(_user, r, w, send, recv, words):
+            try:
+                s = np.ctypeslib.as_array(send, shape=(int(words),))
+                d = np.ctypeslib.as_array(recv, shape=(int(w), int(words)))
+                return 0 if fn(int(r), s, d) else 1
+            except Exception:  # (an exception cannot cross the C frames: it fails the call instead)
+                return 1
+        self = cls.__new__(cls)
+        self.ctx, self.lib = ctx, ctx.lib
+        self._fn = GATHER_FN(trampoline)  # alive as long as the communicator
+        h = C.c_void_p()
+        ctx._ck(self.lib.e2s_comm_create_gather(ctx.h, int(rank), int(world), self._fn, None, C.byref(h)))
+        self.h, self.rank, self.world = h, int(rank), int(world)
+        return self
 
     def close(self):
         if self.h:

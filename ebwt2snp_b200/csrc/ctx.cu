@@ -1,4 +1,5 @@
-// Contexts, errors, kernel timing, and the NCCL binding behind the communicators of the one-process-per-GPU exchange.
+// Contexts, errors, kernel timing, and the communicators of the exchange between the phases: NCCL (one process per GPU) or
+// the caller's own all-gather.
 
 #include <dlfcn.h>
 #include <stdlib.h>
@@ -55,6 +56,13 @@ int cuda_fail(e2s_ctx* ctx, cudaError_t e, const char* what) {
 
 // every rank's exchange row (cm->d_send) into cm->d_recv, on the context's stream
 int all_gather_rows(e2s_ctx* c, e2s_comm* cm) {
+    if (cm->fn) {  // the caller's all-gather, on the host: the row out (the stream waits for it), the callback, the rows back in
+        CU(c, cudaMemcpyAsync(cm->h_send, cm->d_send, XR_WORDS * 8, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaStreamSynchronize(c->stream));
+        if (cm->fn(cm->user, cm->rank, cm->world, cm->h_send, cm->h_recv, XR_WORDS) != 0) return fail(c, E2S_ERR_STATE, "caller's all-gather failed");
+        CU(c, cudaMemcpyAsync(cm->d_recv, cm->h_recv, size_t(cm->world) * XR_WORDS * 8, cudaMemcpyHostToDevice, c->stream));
+        return E2S_OK;
+    }
     NcclApi* na = nccl_api();
     const int nr = na->AllGather(cm->d_send, cm->d_recv, XR_WORDS, NCCL_UINT64, cm->nccl, c->stream);
     if (nr != 0) return fail(c, E2S_ERR_CUDA, std::string("ncclAllGather: ") + (na->GetErrorString ? na->GetErrorString(nr) : "error"));
@@ -249,6 +257,28 @@ int e2s_comm_create(e2s_ctx* c, const uint8_t* id128, int rank, int world, e2s_c
     return E2S_OK;
 }
 
+int e2s_comm_create_gather(e2s_ctx* c, int rank, int world, e2s_gather_fn fn, void* user, e2s_comm** out) {
+    if (!c || !fn || !out || world < 1 || rank < 0 || rank >= world) return fail(c, E2S_ERR_ARG, "e2s_comm_create_gather: bad argument");
+    *out = nullptr;
+    CU(c, cudaSetDevice(c->device));
+    e2s_comm* cm = new e2s_comm();
+    cm->ctx = c;
+    cm->fn = fn;
+    cm->user = user;
+    cm->rank = rank;
+    cm->world = world;
+    cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&cm->d_send), XR_WORDS * 8);
+    if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&cm->d_recv), size_t(world) * XR_WORDS * 8);
+    if (e == cudaSuccess) e = cudaHostAlloc(reinterpret_cast<void**>(&cm->h_recv), size_t(world) * XR_WORDS * 8, cudaHostAllocDefault);
+    if (e == cudaSuccess) e = cudaHostAlloc(reinterpret_cast<void**>(&cm->h_send), XR_WORDS * 8, cudaHostAllocDefault);
+    if (e != cudaSuccess) {
+        e2s_comm_destroy(cm);
+        return fail(c, E2S_ERR_NOMEM, "e2s_comm_create_gather: exchange buffers");
+    }
+    *out = cm;
+    return E2S_OK;
+}
+
 void e2s_comm_destroy(e2s_comm* cm) {
     if (!cm) return;
     cudaSetDevice(cm->ctx->device);
@@ -258,6 +288,7 @@ void e2s_comm_destroy(e2s_comm* cm) {
     cudaFree(cm->d_send);
     cudaFree(cm->d_recv);
     cudaFreeHost(cm->h_recv);
+    cudaFreeHost(cm->h_send);
     delete cm;
 }
 

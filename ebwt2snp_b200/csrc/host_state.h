@@ -234,10 +234,13 @@ struct e2s_shard {
 struct e2s_comm {
     e2s_ctx* ctx = nullptr;
     void* nccl = nullptr;
+    e2s_gather_fn fn = nullptr;  // instead of nccl: the caller's all-gather, on the host (e2s_comm_create_gather)
+    void* user = nullptr;
     int rank = 0, world = 1;
     uint64_t* d_send = nullptr;  // XR_WORDS
     uint64_t* d_recv = nullptr;  // world * XR_WORDS
     uint64_t* h_recv = nullptr;  // pinned
+    uint64_t* h_send = nullptr;  // pinned, XR_WORDS (fn only)
 };
 
 namespace e2s {

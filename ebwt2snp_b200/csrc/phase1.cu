@@ -138,8 +138,10 @@ static int arm_survivors(e2s_shard* s, uint32_t mcov, uint64_t records, SurvEntr
     if (const char* dbg = getenv("E2S_PF_CAPACITY")) {  // test hook: a tiny list forces the overflow -> two-phase fallback
         const uint64_t v = strtoull(dbg, nullptr, 10);
         if (v) {
-            want = v;
-            if (s->pf_cap > v && !s->pf_want) s->pf_cap = v;  // also shrink the advertised capacity of an existing buffer
+            // at least the 4 entries the scan leaves to k_merge_stats: the <= 3 records a shard adopts always fit, so a rank
+            // never finds its list full after the exchange (it would repeat the scan alone, the other ranks not knowing)
+            want = v > 4 ? v : 4;
+            if (s->pf_cap > want && !s->pf_want) s->pf_cap = want;  // also shrink the advertised capacity of an existing buffer
         }
     }
     if (s->pf_want > want) want = s->pf_want;  // (an overflow of the last attempt asked for more)

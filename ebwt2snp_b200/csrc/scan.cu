@@ -736,15 +736,16 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+// looked up once, by the initializer of a function-local static: contexts on several host threads may launch concurrently
 static PFN_encodeTiled scan_encode_fn() {
-    static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
+    static const PFN_encodeTiled fn = [] {
         void* ptr = nullptr;
         cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_encodeTiled>(ptr);
-    }
+        return cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess &&
+                       q == cudaDriverEntryPointSuccess
+                   ? reinterpret_cast<PFN_encodeTiled>(ptr)
+                   : nullptr;
+    }();
     return fn;
 }
 

@@ -47,7 +47,8 @@ extern "C" {
 
 typedef struct e2s_ctx e2s_ctx;
 typedef struct e2s_shard e2s_shard;
-typedef struct e2s_comm e2s_comm; /* one process per GPU: wraps an NCCL communicator (e2s_comm_create) */
+typedef struct e2s_comm e2s_comm; /* one process per GPU: wraps an NCCL communicator (e2s_comm_create), or the caller's own
+                                     all-gather (e2s_comm_create_gather: several ranks on one GPU, as the tests run them) */
 
 /* ---------------------------------------------------------------------------------------
  * context
@@ -432,6 +433,14 @@ int e2s_exchange_rows_finish(const uint64_t *rows, int n_shards, int my, uint64_
                              int mcov_out, double pval, e2s_cluster_merged *mine, e2s_stats *total);
 int e2s_comm_unique_id(uint8_t *id128);
 int e2s_comm_create(e2s_ctx *ctx, const uint8_t *id128, int rank, int world, e2s_comm **out);
+/* A communicator whose all-gather the caller performs: where the library would call ncclAllGather it copies this rank's row
+ * (`words` u64) to the host, synchronises the context's stream and calls fn(user, rank, world, send, recv, words).  fn must
+ * return on every rank with recv = the `world` rows in rank order (the contract of ncclAllGather), and 0; any other value fails
+ * the call with E2S_ERR_STATE.  The rows then go back to the device on the stream.  It lets several ranks of one sharded step
+ * run in one process, on one GPU (threads and a barrier), so the multi-rank step is testable without several GPUs.  The
+ * callback runs on the thread that made the library call. */
+typedef int (*e2s_gather_fn)(void *user, int rank, int world, const uint64_t *send, uint64_t *recv, uint64_t words);
+int e2s_comm_create_gather(e2s_ctx *ctx, int rank, int world, e2s_gather_fn fn, void *user, e2s_comm **out);
 void e2s_comm_destroy(e2s_comm *comm);
 int e2s_pipeline_sharded(e2s_shard *sh, e2s_comm *comm, uint32_t k, int32_t min_len, const e2s_snp_params *p,
                          e2s_cluster_merged *merged, e2s_stats *stats, e2s_snp_counts *counts);
